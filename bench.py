@@ -81,6 +81,28 @@ def algorithmic_bytes(q):
     return 8 * (zH + zA + 3 * nV + 2 * nC) + 8 * (2 * nV + nC) + 4 * (nV + nC) + 16
 
 
+DUMP_BYTES = 60 * 1000 * 1000  # array data of --dump-outputs: the files, headers included, stay under 64 MB
+
+
+def dump_outputs(path, groups, B):
+    """What a caller of the timed path holds after its last step, per dumped QP: x [B, nV], the multipliers of the bounds
+    [B, nV] and of the constraints [B, nC] (not written when nC = 0), the objective, status and iteration count [B], written as
+    float64 `path/<dump>_<array>.npy`.  Above DUMP_BYTES in all, the same seeded sample of replicas (rows) is kept for every dumped QP."""
+    os.makedirs(path, exist_ok=True)
+    total = sum(8 * B * (2 * gr["nV"] + gr["nC"] + 3) for gr in groups)
+    rows = np.arange(B)
+    if total > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(B, B * DUMP_BYTES // total, replace=False))
+    for gr in sorted(groups, key=lambda gr: gr["q"]["name"]):
+        s = gr["s"]
+        arrays = {"x": s.get_optimal_solution(), "y_bounds": s.get_multipliers_bounds(), "y_constr": s.get_multipliers_constr(),
+                  "obj": s.get_obj_value(), "status": s.get_status(), "iters": s.get_iterations()}
+        for k, a in arrays.items():
+            if a.size == 0:  # y_constr of a dump without constraints (nC = 0): nothing to compare
+                continue
+            np.save(os.path.join(path, "%s_%s.npy" % (gr["q"]["name"], k)), np.ascontiguousarray(a[rows], dtype=np.float64))
+
+
 def perturbed_starts(nlp, B, k):
     """SURVEY.md 8d config 3: x0_i = clip(x0*(1 + 0.1 N) + 0.1 N), default_rng(71000 + problem index)."""
     x0, _ = nlp.Get_starting_point()
@@ -337,6 +359,8 @@ def run_gpu(args, rank, world, local_rank):
         sampler.start()
     use_streams(True)
     ms_res, launches, _ = timed(step_resident, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, groups, B)
     ms_e2e_serial, _, _ = timed(step_e2e, args.steps, max(3, args.warmup // 2))  # one step at a time (L2 flush + join between steps)
     ms_e2e = timed_e2e_overlapped(args.steps, max(4, args.warmup)) if (groups_b and streams) else ms_e2e_serial
     clocks = sampler.stop() if rank == 0 else None  # sampled every 20 ms across both timed regions (and their warm-ups)
@@ -751,8 +775,12 @@ def main():
     ap.add_argument("--strong", type=int, default=1000000, help="instances of the strong-scaling block (configs[4]); 0: off")
     ap.add_argument("--e2e-overlap", type=int, default=1, help="1: the end-to-end path alternates two handle sets (consecutive steps overlap); 0: one step at a time")
     ap.add_argument("--streams", type=int, default=1, help="1: one CUDA stream per dumped QP (overlapping launches), 0: default stream")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the solutions of the last one as DIR/<dump>_<array>.npy (rank 0; float64)")
     args = ap.parse_args()
-    rank = int(os.environ.get("RANK", "0"))
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's solutions; --impl reference has none to write")
+    rank =int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":

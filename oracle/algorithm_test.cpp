@@ -12,7 +12,7 @@
 // branches, which refresh both constraint sides -- the reference's own default backend is QORE, src/Options.cpp:24-25).
 //
 // model file: restartsqp_b200.nl_reader.write_model_file (sizes, bounds, start, patterns, starting points as hex floats);
-// evaluator: oracle/_gen/nlp_<name>_<hash>.so (nlp_fc, nlp_all).  Output: exitflag iter qp_iter obj x..., doubles as hex floats.
+// evaluator: the library oracle_py.SqpOracle compiled for the model (its `evaluator` path; nlp_fc, nlp_all).  Output: exitflag iter qp_iter obj x..., doubles as hex floats.
 #include <dlfcn.h>
 
 #include <cstdio>

@@ -298,16 +298,30 @@ class _SqpProblem(C.Structure):
                 [("second_order_correction", C.c_int)])
 
 
+_GEN = None
+
+
+def _gen_dir():
+    """Where SqpOracle compiles model evaluators: one temporary directory per process, removed at exit."""
+    global _GEN
+    if _GEN is None:
+        import atexit
+        import shutil
+        import tempfile
+        _GEN = tempfile.mkdtemp(prefix="sqpb200_oracle_gen_")
+        atexit.register(shutil.rmtree, _GEN, True)
+    return _GEN
+
+
 class SqpOracle:
     """CPU restatement of Algorithm::Optimize (oracle_sqp.c) for one model: `nlp` is a restartsqp_b200.nl_reader.AmplNLP (or
     anything with c_source(), the triplet patterns, bounds and start); its evaluator is generated as C and compiled with gcc
-    (-ffp-contract=off) into oracle/_gen/."""
+    (-ffp-contract=off) into a temporary directory of this process, so that a read-only checkout can run it."""
 
     def __init__(self, nlp, options):
         import hashlib
         src = nlp.c_source()
-        gen = os.path.join(_HERE, "_gen")
-        os.makedirs(gen, exist_ok=True)
+        gen = _gen_dir()
         tag = hashlib.sha1(src.encode()).hexdigest()[:16]
         so = os.path.join(gen, "nlp_%s_%s.so" % (getattr(nlp, "name", "model"), tag))
         if not os.path.exists(so):
@@ -316,6 +330,7 @@ class SqpOracle:
                 f.write(src)
             subprocess.run(["gcc", "-O1", "-fPIC", "-shared", "-ffp-contract=off", "-o", so, cfile, "-lm"], check=True, capture_output=True)
         self._nlp_lib = C.CDLL(so)
+        self.evaluator = so  # the compiled evaluator (nlp_fc, nlp_all), for programs that load it themselves
         self.L = lib()
         info = nlp.Get_nlp_info()
         xl, xu, cl, cu = nlp.Get_bounds_info()

@@ -19,7 +19,6 @@ flag, outer and QP iteration counts, final iterate and objective, bit for bit.  
     uncaught); the oracle and the library reject it;
   * (outside the models tested here: hs099, hs99exp, hs107) QORE's KKT tolerance is 1e-5, the oracle's 1e-6.
 profiles/r2_reference_loop_pin.md holds the same comparison over all 149 fixture models."""
-import glob
 import os
 import subprocess
 
@@ -46,13 +45,14 @@ def run_all(binary, name, tmp_path, mode="qore", timeout=300, count=B):
     d = HS_DIR if name.startswith("hs") else CUTE_DIR
     h = AmplNLP(os.path.join(d, name + ".nl"))
     X = perturbed_starts(h, B, 4)
-    res = orc.SqpOracle(h, r.Options()).solve_batch(X)  # also compiles the C evaluator into oracle/_gen
+    so = orc.SqpOracle(h, r.Options())  # also compiles the C evaluator the reference's program loads
+    res = so.solve_batch(X)
     model = str(tmp_path / (name + ".model"))
     write_model_file(h, model, X)
-    ev = sorted(glob.glob(os.path.join(ROOT, "oracle", "_gen", "nlp_%s_*.so" % name)), key=os.path.getmtime)[-1]
+    ev = so.evaluator
     out = []
     for k in range(count):
-        p = subprocess.run([binary, model, ev, str(k)] + ([mode] if mode else []), capture_output=True, text=True, timeout=timeout)
+        p = subprocess.run([binary, model, ev, str(k)] + ([mode] if mode else []), cwd=tmp_path, capture_output=True, text=True, timeout=timeout)
         t = p.stdout.split()
         if p.returncode != 0:
             out.append(dict(rc=p.returncode, msg=p.stdout.strip()))
@@ -98,12 +98,13 @@ def test_reference_second_order_correction_equals_the_oracle(tmp_path):
     for name in ["hs006", "hs043", "hs100", "hs015", "hs113", "hs071", "hs038"]:
         h = AmplNLP(os.path.join(HS_DIR, name + ".nl"))
         X = perturbed_starts(h, B, 4)
-        res = orc.SqpOracle(h, r.Options(second_order_correction=True)).solve_batch(X)
+        so = orc.SqpOracle(h, r.Options(second_order_correction=True))
+        res = so.solve_batch(X)
         model = str(tmp_path / (name + ".model"))
         write_model_file(h, model, X)
-        ev = sorted(glob.glob(os.path.join(ROOT, "oracle", "_gen", "nlp_%s_*.so" % name)), key=os.path.getmtime)[-1]
+        ev = so.evaluator
         for k in range(B):
-            p = subprocess.run([NOCLIP, model, ev, str(k), "qore", "soc"], capture_output=True, text=True, timeout=300)
+            p = subprocess.run([NOCLIP, model, ev, str(k), "qore", "soc"], cwd=tmp_path, capture_output=True, text=True, timeout=300)
             assert p.returncode == 0, (name, k, p.stdout)
             t = p.stdout.split()
             x = np.array([float.fromhex(v) for v in t[4:]])

@@ -33,10 +33,11 @@ def main():
             try:
                 h = AmplNLP(path)
                 X = perturbed_starts(h, B, 4)
-                res = orc.SqpOracle(h, r.Options()).solve_batch(X)
+                so = orc.SqpOracle(h, r.Options())
+                res = so.solve_batch(X)
                 model = os.path.join(td, name + ".model")
                 write_model_file(h, model, X)
-                ev = sorted(glob.glob(os.path.join(ROOT, "oracle", "_gen", "nlp_%s_*.so" % name)), key=os.path.getmtime)[-1]
+                ev = so.evaluator
             except Exception as e:  # noqa: BLE001
                 rows.append((name, "-", "-", "skipped: %s" % repr(e)[:60]))
                 continue
@@ -46,7 +47,7 @@ def main():
                 same = labels = other = 0
                 notes = []
                 for k in range(B):
-                    p = subprocess.run([exe, model, ev, str(k), "qore"], capture_output=True, text=True, timeout=600)
+                    p = subprocess.run([exe, model, ev, str(k), "qore"], cwd=td, capture_output=True, text=True, timeout=600)
                     t = p.stdout.split()
                     if p.returncode != 0:
                         other += 1
