@@ -305,6 +305,33 @@ int sqpb200_sqp_phase(const sqpb200_sqp_state* st, int phase, int* counters_host
  * refreshes both constraint sides (mode 3 of sqpb200_qphandler_bounds), 0 = the reference's stale-ubA behaviour (mode 1). */
 int sqpb200_sqp_optimize(sqpb200_sqp_state* st, sqpb200_handle qp, sqpb200_handle lp, sqpb200_nlp nlp, int second_order_correction,
                          int refresh_ubA, int* first, double* f_tmp, double* c_tmp, long long* launches, void* stream);
+/* Streamed solves: N starting points through the B = st->B instances ("slots") of the state.  A slot whose instance has stopped
+ * hands its results to out[instance] and takes the next starting point of the queue, so the batch does not wait for its slowest
+ * instance.  Every array is device memory owned by the caller; the function sets slot_id to -1, *head to 0 and refill to 0 itself. */
+typedef struct {
+    long long N;              /* number of starting points */
+    int refill_min;           /* a refill round runs once at least this many occupied slots have stopped (>= 1), or when none is active */
+    const double* x0_all;     /* [N][n] starting points (shifted into the bounds as initialization() does) */
+    const double* lam_start;  /* [m] starting constraint multipliers (NULL if m = 0) */
+    /* results by instance (input order): final iterate, objective, exit flag (as sqpb200_sqp_optimize leaves them), outer and QP
+     * iterations, KKT error, penalty parameter, trust-region radius */
+    double* x;                /* [N][n] */
+    double *obj, *kkt_err, *rho, *delta;
+    int *exitflag, *iter;
+    long long* qp_iter;
+    long long* slot_id;       /* [B] instance held by each slot, -1 = free */
+    unsigned long long* head; /* [1] next queue index (advanced with atomicAdd; may end above N) */
+    unsigned char* refill;    /* [B] slots filled by the last refill round */
+    long long rounds;         /* out: refill rounds, the initial fill included */
+} sqpb200_sqp_stream;
+/* Algorithm::Optimize for every starting point of `sd`, same arguments as sqpb200_sqp_optimize otherwise.  Each instance follows
+ * exactly the trajectory it follows in one batch with all N (instances do not influence each other).  Needs per-instance backend
+ * state machines (st->qp_inst and st->lp_inst set): with handle-level modes the instances of a handle share its init / hotstart
+ * decision, so SQPB200_ERR_INVALID.  Returns when the queue is empty and every instance has been collected; the state's own
+ * per-instance arrays then hold the slots' last instances. */
+int sqpb200_sqp_optimize_stream(sqpb200_sqp_state* st, sqpb200_handle qp, sqpb200_handle lp, sqpb200_nlp nlp,
+                                int second_order_correction, int refresh_ubA, int* first, double* f_tmp, double* c_tmp,
+                                sqpb200_sqp_stream* sd, long long* launches, void* stream);
 /* Forget every solve so far: the next solve is an init (cold start) again, as for a freshly constructed backend
  * (firstQPsolved_ = false, matrix status UNDEFINED, Update_* flags cleared; src/qpOASESInterface.cpp:35-50).  Structures and
  * device buffers are kept, so one handle can serve batch after batch. */

@@ -29,7 +29,7 @@ EXPORTS = [
     "sqpb200_solve_config", "sqpb200_last_solve_ms", "sqpb200_get_profile", "sqpb200_io_layout", "sqpb200_solve_host", "sqpb200_vector_reduce", "sqpb200_vector_elementwise",
     "sqpb200_nlp_compile", "sqpb200_nlp_cubin_size", "sqpb200_nlp_load", "sqpb200_nlp_eval", "sqpb200_nlp_destroy",
     "sqpb200_nlp_launch_count", "sqpb200_nlp_last_error",
-    "sqpb200_sqp_phase", "sqpb200_sqp_optimize", "sqpb200_reset", "sqpb200_solve_device_mask", "sqpb200_device_buffers", "sqpb200_solve_per_instance",
+    "sqpb200_sqp_phase", "sqpb200_sqp_optimize", "sqpb200_sqp_optimize_stream", "sqpb200_reset", "sqpb200_solve_device_mask", "sqpb200_device_buffers", "sqpb200_solve_per_instance",
     # QORE layout: compressed-row matrices, stacked bounds / primal / dual / working set
     "sqpb200_set_structure_A_csr", "sqpb200_set_structure_H_csr", "sqpb200_set_structure_csr", "sqpb200_get_structure_csr",
     "sqpb200_set_values_csr", "sqpb200_get_values_csr", "sqpb200_set_bounds_stacked", "sqpb200_get_bounds_stacked",
@@ -76,6 +76,8 @@ def lib():
         L.sqpb200_vector_elementwise.argtypes = [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_void_p, C.c_void_p, C.c_double, C.c_int, C.c_void_p]
         L.sqpb200_sqp_optimize.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                            C.c_void_p, C.c_void_p]
+        L.sqpb200_sqp_optimize_stream.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.sqpb200_solve_host.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.sqpb200_last_solve_ms.restype = C.c_float
         L.sqpb200_last_solve_ms.argtypes = [C.c_void_p]

@@ -185,22 +185,67 @@ void BatchedAlgorithm::reset(const double* x0) {
     check(sqpb200_reset(lp_), "sqpb200_reset(LP)");
 }
 
+namespace {
+// per-instance results [count] from device arrays
+BatchedResult download(size_t count, size_t n, const double* x, const double* obj, const double* kkt, const double* rho, const double* delta,
+                       const int* exitflag, const int* iter, const long long* qp_iter) {
+    BatchedResult r;
+    r.x.resize(count * n); r.obj.resize(count); r.KKT_error.resize(count); r.rho.resize(count); r.delta.resize(count);
+    r.exitflag.resize(count); r.iter.resize(count); r.qp_iter.resize(count);
+    auto down = [&](void* dst, const void* src, size_t bytes) { if (bytes) cuda_check(cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost), "cudaMemcpy(result)"); };
+    down(r.x.data(), x, count * n * 8); down(r.obj.data(), obj, count * 8); down(r.KKT_error.data(), kkt, count * 8);
+    down(r.rho.data(), rho, count * 8); down(r.delta.data(), delta, count * 8);
+    down(r.exitflag.data(), exitflag, count * 4); down(r.iter.data(), iter, count * 4); down(r.qp_iter.data(), qp_iter, count * 8);
+    return r;
+}
+}  // namespace
+
 BatchedResult BatchedAlgorithm::Optimize() {
     long long nl = 0;
     check(sqpb200_sqp_optimize(&S_, qp_, lp_, eval_, opt_.second_order_correction ? 1 : 0, /*refresh_ubA=*/1, &first_, f_tmp_, c_tmp_, &nl,
                                nullptr), "sqpb200_sqp_optimize");
     launches_ += nl;
     cuda_check(cudaDeviceSynchronize(), "cudaDeviceSynchronize");
-    const size_t B = (size_t)B_, n = (size_t)n_;
-    BatchedResult r;
-    r.x.resize(B * n); r.obj.resize(B); r.KKT_error.resize(B); r.rho.resize(B); r.delta.resize(B);
-    r.exitflag.resize(B); r.iter.resize(B); r.qp_iter.resize(B);
-    auto down = [&](void* dst, const void* src, size_t bytes) { cuda_check(cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost), "cudaMemcpy(result)"); };
-    down(r.x.data(), S_.x_k, B * n * 8); down(r.obj.data(), S_.f_k, B * 8); down(r.KKT_error.data(), S_.kkt_err, B * 8);
-    down(r.rho.data(), S_.rho, B * 8); down(r.delta.data(), S_.delta, B * 8);
-    down(r.exitflag.data(), S_.exitflag, B * 4); down(r.iter.data(), S_.iter, B * 4); down(r.qp_iter.data(), S_.qp_iter, B * 8);
+    BatchedResult r = download(B_, n_, S_.x_k, S_.f_k, S_.kkt_err, S_.rho, S_.delta, S_.exitflag, S_.iter, S_.qp_iter);
     r.launches = launches_;
     return r;
+}
+
+BatchedResult BatchedAlgorithm::OptimizeStream(const double* x0_all, long long N, int refill_min, long long* rounds) {
+    if (N < 0 || (N > 0 && !x0_all)) throw std::invalid_argument("OptimizeStream: no starting points");
+    const size_t n = (size_t)n_, m = (size_t)m_, d = sizeof(double), Nz = (size_t)N, B = (size_t)B_;
+    // inputs, results by instance and the queue in one arena
+    Carver c;
+    sqpb200_sqp_stream sd;
+    std::memset(&sd, 0, sizeof sd);
+    const size_t o_x0 = c.take(Nz * n * d), o_lam = c.take(m * d), o_x = c.take(Nz * n * d), o_obj = c.take(Nz * d), o_kkt = c.take(Nz * d),
+                 o_rho = c.take(Nz * d), o_delta = c.take(Nz * d), o_ex = c.take(Nz * 4), o_it = c.take(Nz * 4), o_qi = c.take(Nz * 8),
+                 o_slot = c.take(B * 8), o_head = c.take(8), o_refill = c.take(B);
+    char* mem = nullptr;
+    cuda_check(cudaMalloc((void**)&mem, c.off), "cudaMalloc(stream arena)");
+    try {
+        if (N > 0) cuda_check(cudaMemcpy(mem + o_x0, x0_all, Nz * n * d, cudaMemcpyHostToDevice), "cudaMemcpy(x0_all)");
+        if (m) cuda_check(cudaMemcpy(mem + o_lam, nlp_.lam_start.data(), m * d, cudaMemcpyHostToDevice), "cudaMemcpy(lam_start)");
+        sd.N = N;
+        sd.refill_min = refill_min > 0 ? refill_min : (B_ / 16 > 0 ? B_ / 16 : 1);
+        sd.x0_all = (const double*)(mem + o_x0); sd.lam_start = m ? (const double*)(mem + o_lam) : nullptr;
+        sd.x = (double*)(mem + o_x); sd.obj = (double*)(mem + o_obj); sd.kkt_err = (double*)(mem + o_kkt); sd.rho = (double*)(mem + o_rho);
+        sd.delta = (double*)(mem + o_delta); sd.exitflag = (int*)(mem + o_ex); sd.iter = (int*)(mem + o_it); sd.qp_iter = (long long*)(mem + o_qi);
+        sd.slot_id = (long long*)(mem + o_slot); sd.head = (unsigned long long*)(mem + o_head); sd.refill = (unsigned char*)(mem + o_refill);
+        long long nl = 0;
+        check(sqpb200_sqp_optimize_stream(&S_, qp_, lp_, eval_, opt_.second_order_correction ? 1 : 0, /*refresh_ubA=*/1, &first_, f_tmp_, c_tmp_,
+                                          &sd, &nl, nullptr), "sqpb200_sqp_optimize_stream");
+        launches_ += nl;
+        cuda_check(cudaDeviceSynchronize(), "cudaDeviceSynchronize");
+        BatchedResult r = download(Nz, n, sd.x, sd.obj, sd.kkt_err, sd.rho, sd.delta, sd.exitflag, sd.iter, sd.qp_iter);
+        r.launches = launches_;
+        if (rounds) *rounds = sd.rounds;
+        cudaFree(mem);
+        return r;
+    } catch (...) {
+        cudaFree(mem);
+        throw;
+    }
 }
 
 }  // namespace sqpb200

@@ -64,6 +64,11 @@ public:
     void reset(const double* x0);
     /** Algorithm::Optimize for every instance. */
     BatchedResult Optimize();
+    /** Algorithm::Optimize for N starting points x0_all[N][n] (host memory) streamed through the batch's instances as slots
+     *  (sqpb200_sqp_optimize_stream): a slot whose instance has stopped takes the next starting point on the device.  Returns N
+     *  entries in input order, each what one batch over all N gives.  refill_min: stopped slots that trigger a refill round
+     *  (<= 0: batch / 16, at least 1).  rounds (if not null) receives the number of refill rounds, the initial fill included. */
+    BatchedResult OptimizeStream(const double* x0_all, long long N, int refill_min = 0, long long* rounds = nullptr);
 
     int get_num_var() const { return n_; }
     int get_num_constr() const { return m_; }

@@ -44,6 +44,18 @@ class SqpState(C.Structure):
                 [(k, _D) for k in ("delta0", "rho0", "eps10")])
 
 
+class SqpStream(C.Structure):
+    """sqpb200_sqp_stream of include/sqpb200.h"""
+    _fields_ = ([("N", C.c_longlong), ("refill_min", _I)] +
+                [(k, _P) for k in ("x0_all", "lam_start", "x", "obj", "kkt_err", "rho", "delta", "exitflag", "iter", "qp_iter",
+                                   "slot_id", "head", "refill")] +
+                [("rounds", C.c_longlong)])
+
+
+#: default refill_min of solve_stream as a fraction of the slot count (see solve_stream)
+REFILL_MIN_FRACTION = 16
+
+
 class DeviceBatchedSQP:
     def __init__(self, nlp, x0=None, options: Options = None, device=0, per_instance_modes=True):
         """per_instance_modes: the backend's init/hotstart decision is made per instance, as the reference does for its single
@@ -231,21 +243,77 @@ class DeviceBatchedSQP:
         if host_sequenced:
             return self._optimize_py()
         T = self.T
-        if self.first_:  # structures of both backends (first set_A / set_H call of setupQP / setupLP, values follow in the loop)
-            self.myQP_.solverInterface_.set_A(SpTripletMat(self.nlp_.J_row1, self.nlp_.J_col1, None, self.nCon_, self.nVar_, False), self.myQP_.I_info_A_)
-            self.myQP_.solverInterface_.set_H(SpTripletMat(self.nlp_.H_row1, self.nlp_.H_col1, None, self.nVar_, self.nVar_, True))
-        if not self.myLP_.solverInterface_._A_set:
-            self.myLP_.solverInterface_.set_A(SpTripletMat(self.nlp_.J_row1, self.nlp_.J_col1, None, self.nCon_, self.nVar_, False), self.myLP_.I_info_A_)
+        self._structures()
         first, nl = C.c_int(1 if self.first_ else 0), C.c_longlong(0)
         rc = self.L.sqpb200_sqp_optimize(C.byref(self.S), self.myQP_.solverInterface_.h, self.myLP_.solverInterface_.h, self.nlp_.h,
                                          int(bool(self.options_.second_order_correction)), 1, C.byref(first),
                                          C.c_void_p(T["f_tmp"].data_ptr()), C.c_void_p(T["c_tmp"].data_ptr()), C.byref(nl), None)
-        if rc != 0:
-            raise capi.SqpB200Error("sqpb200_sqp_optimize failed (%d): %s / %s" % (
-                rc, self.L.sqpb200_last_error(self.myQP_.solverInterface_.h).decode(), self.L.sqpb200_last_error(self.myLP_.solverInterface_.h).decode()))
+        self._check(rc, "sqpb200_sqp_optimize")
         self.first_ = bool(first.value)
         self.launches += int(nl.value)
         return self._result()
+
+    def solve_stream(self, x0_all, refill_min=None):
+        """Algorithm::Optimize for N starting points x0_all[N][n] through the `batch` instances of this object used as slots: a slot
+        whose instance has stopped takes the next starting point on the device, so no batch waits for its slowest instance and
+        device memory stays that of `batch` instances (plus the N-row inputs and results).  Returns an SQPResult with N rows in input
+        order; each row is bit for bit what one batch over all N gives.  Needs per-instance backend state machines.
+
+        refill_min: a refill round (retire the stopped instances, refill their slots, one evaluation of the whole batch at the new
+        starts) runs once at least this many occupied slots have stopped, or when no slot is active.  Default batch // 16 (at least 1):
+        on the B200 (profiles/r3_sqp_stream.md) batch // 64, // 16 and // 4 were within 1 % of each other, while 1 (a refill round in
+        nearly every iteration) was up to 30 % slower.  self.stream_rounds holds the number of
+        refill rounds of the last call, the initial fill included.  The object serves reset() / Optimize() afterwards as before."""
+        torch, T, B, n, m = self.torch, self.T, self.batch, self.nVar_, self.nCon_
+        if not self.per_instance_modes:
+            raise ValueError("solve_stream needs per_instance_modes=True: with handle-level modes the instances of a handle share "
+                             "its init / hotstart decision, so a refilled slot would inherit a hot start")
+        x0 = np.asarray(x0_all, dtype=np.float64)
+        if x0.ndim != 2 or x0.shape[1] != n:
+            raise ValueError("solve_stream needs starting points of shape (N, %d), got %s" % (n, x0.shape))
+        refill_min = max(1, B // REFILL_MIN_FRACTION) if refill_min is None else int(refill_min)
+        if refill_min < 1:
+            raise ValueError("refill_min must be at least 1")
+        N = x0.shape[0]
+        dev, f64, i32 = self.dev, torch.float64, torch.int32
+        up = lambda a: torch.as_tensor(np.ascontiguousarray(a)).to(dev)
+        O = dict(x0_all=up(x0), lam_start=up(self._lam_start.reshape(-1)), x=torch.empty((N, n), dtype=f64, device=dev),
+                 obj=torch.empty(N, dtype=f64, device=dev), kkt_err=torch.empty(N, dtype=f64, device=dev),
+                 rho=torch.empty(N, dtype=f64, device=dev), delta=torch.empty(N, dtype=f64, device=dev),
+                 exitflag=torch.empty(N, dtype=i32, device=dev), iter=torch.empty(N, dtype=i32, device=dev),
+                 qp_iter=torch.empty(N, dtype=torch.int64, device=dev), slot_id=torch.empty(B, dtype=torch.int64, device=dev),
+                 head=torch.empty(1, dtype=torch.int64, device=dev), refill=torch.empty(B, dtype=torch.uint8, device=dev))
+        D = SqpStream()
+        D.N, D.refill_min = N, refill_min
+        for k, t in O.items():
+            setattr(D, k, t.data_ptr() if t.numel() else None)
+        self._structures()
+        first, nl = C.c_int(1 if self.first_ else 0), C.c_longlong(0)
+        rc = self.L.sqpb200_sqp_optimize_stream(C.byref(self.S), self.myQP_.solverInterface_.h, self.myLP_.solverInterface_.h, self.nlp_.h,
+                                                int(bool(self.options_.second_order_correction)), 1, C.byref(first),
+                                                C.c_void_p(T["f_tmp"].data_ptr()), C.c_void_p(T["c_tmp"].data_ptr()), C.byref(D),
+                                                C.byref(nl), None)
+        self._check(rc, "sqpb200_sqp_optimize_stream")
+        self.first_ = bool(first.value)
+        self.launches += int(nl.value)
+        self.stream_rounds = int(D.rounds)
+        torch.cuda.synchronize()
+        h = lambda k: O[k].cpu().numpy()
+        return SQPResult(x=h("x"), obj=h("obj"), exitflag=h("exitflag"), iters=h("iter").astype(np.int64), qp_iter=h("qp_iter"),
+                         KKT_error=h("kkt_err"), rho=h("rho"), delta=h("delta"))
+
+    def _structures(self):
+        """structures of both backends (first set_A / set_H call of setupQP / setupLP, values follow in the loop)"""
+        if self.first_:
+            self.myQP_.solverInterface_.set_A(SpTripletMat(self.nlp_.J_row1, self.nlp_.J_col1, None, self.nCon_, self.nVar_, False), self.myQP_.I_info_A_)
+            self.myQP_.solverInterface_.set_H(SpTripletMat(self.nlp_.H_row1, self.nlp_.H_col1, None, self.nVar_, self.nVar_, True))
+        if not self.myLP_.solverInterface_._A_set:
+            self.myLP_.solverInterface_.set_A(SpTripletMat(self.nlp_.J_row1, self.nlp_.J_col1, None, self.nCon_, self.nVar_, False), self.myLP_.I_info_A_)
+
+    def _check(self, rc, what):
+        if rc != 0:
+            raise capi.SqpB200Error("%s failed (%d): %s / %s" % (
+                what, rc, self.L.sqpb200_last_error(self.myQP_.solverInterface_.h).decode(), self.L.sqpb200_last_error(self.myLP_.solverInterface_.h).decode()))
 
     def _result(self):
         T = self.T
