@@ -252,21 +252,38 @@ struct QPT {
     static constexpr int DOT_N_SMALL = QP_DOT_UNROLL_N;  // a macro is not expanded inside the pragma's string
     typedef typename PatIdx<TEAM>::type pidx;
     // ---------------------------------------------------------------- sparse products
+    // One entry of each product, summed in storage order.  The mul* functions below run one lane per entry and end in a
+    // barrier; the fused phases (step_direction, drift_correction, ramping, ensure_li) call these directly so that an entry
+    // is formed by the lane that consumes it, with the same terms in the same order.
+    static __device__ __forceinline__ double H_row(const pidx* pat, const double* Hv, const double* v, int c) {  // ((H + reg I) v)[c]
+        const pidx *Hp = pat + sA.pHp, *Hi = pat + sA.pHi;
+        const double reg = sA.is_lp ? QP_EPS_REG : 0.0;
+        double s = 0.0;
+        if (sA.has_H && !sA.is_lp) {
+            int e1 = Hp[c + 1];
+            QP_U1 for (int e = Hp[c]; e < e1; e++) s += Hv[e] * v[Hi[e]];
+        }
+        if (reg != 0.0) s += reg * v[c];
+        return s;
+    }
+    static __device__ __forceinline__ double A_row(const pidx* pat, const double* Av, const double* v, int r) {  // (A v)[r]
+        const pidx *Arp = pat + sA.pArp, *Aci = pat + sA.pAci, *Aperm = pat + sA.pAperm;
+        double s = 0.0;
+        int k1 = Arp[r + 1];
+        QP_U1 for (int k = Arp[r]; k < k1; k++) s += Av[Aperm[k]] * v[Aci[k]];
+        return s;
+    }
+    static __device__ __forceinline__ double AT_col(const pidx* pat, const double* Av, const double* yc, int c) {  // (A' yc)[c]
+        const pidx *Ap = pat + sA.pAp, *Ai = pat + sA.pAi;
+        double s = 0.0;
+        int e1 = Ap[c + 1];
+        QP_U1 for (int e = Ap[c]; e < e1; e++) s += Av[e] * yc[Ai[e]];
+        return s;
+    }
     static __device__ QP_FN void mulH(const double* v, double* out) {  // out = (H + reg I) v (H symmetric: column gather)
         QP_CTX QP_PAT
-        const pidx *Hp = pat + sA.pHp, *Hi = pat + sA.pHi;
         const double* Hv = V_(Hv);
-        const bool has_H = sA.has_H && !sA.is_lp;
-        const double reg = sA.is_lp ? QP_EPS_REG : 0.0;
-        QP_U1 for (int c = lane; c < nV; c += TEAM) {
-            double s = 0.0;
-            if (has_H) {
-                int e1 = Hp[c + 1];
-                QP_U1 for (int e = Hp[c]; e < e1; e++) s += Hv[e] * v[Hi[e]];
-            }
-            if (reg != 0.0) s += reg * v[c];
-            out[c] = s;
-        }
+        QP_U1 for (int c = lane; c < nV; c += TEAM) out[c] = H_row(pat, Hv, v, c);
         SYNC();
     }
     static __device__ QP_FN void mulH_noreg(const double* v, double* out) {  // out = H v (objective / KKT epilogue)
@@ -286,26 +303,14 @@ struct QPT {
     }
     static __device__ QP_FN void mulA(const double* v, double* out) {
         QP_CTX QP_PAT
-        const pidx *Arp = pat + sA.pArp, *Aci = pat + sA.pAci, *Aperm = pat + sA.pAperm;
         const double* Av = V_(Av);
-        QP_U1 for (int r = lane; r < nC; r += TEAM) {
-            double s = 0.0;
-            int k1 = Arp[r + 1];
-            QP_U1 for (int k = Arp[r]; k < k1; k++) s += Av[Aperm[k]] * v[Aci[k]];
-            out[r] = s;
-        }
+        QP_U1 for (int r = lane; r < nC; r += TEAM) out[r] = A_row(pat, Av, v, r);
         SYNC();
     }
     static __device__ QP_FN void mulAT(const double* yc, double* out) {
         QP_CTX QP_PAT
-        const pidx *Ap = pat + sA.pAp, *Ai = pat + sA.pAi;
         const double* Av = V_(Av);
-        QP_U1 for (int c = lane; c < nV; c += TEAM) {
-            double s = 0.0;
-            int e1 = Ap[c + 1];
-            QP_U1 for (int e = Ap[c]; e < e1; e++) s += Av[e] * yc[Ai[e]];
-            out[c] = s;
-        }
+        QP_U1 for (int c = lane; c < nV; c += TEAM) out[c] = AT_col(pat, Av, yc, c);
         SYNC();
     }
     // A[r][c] via the CSR view (duplicates summed)
@@ -1690,6 +1695,47 @@ struct QPT {
         if (lane == 0) { AC_[nAC] = (short)c; posAC_[c] = (short)nAC; sC_[c] = (short)status; hdr[1] = nAC + 1; }
         SYNC();
     }
+    // The rotation chain of a removal, warp kernel with nAC <= TEAM.  Rotation i (i0 <= i < nAC) acts on the columns
+    // (cL, cL+1), cL = c0 - i, of rows i.. of T (it zeroes T_(i, cL)) and of every row of Q.  Lane ii owns row ii of T and
+    // carries in a register the entry of column cL+1 that rotation i-1 left; T_(ii, cL) is still untouched in shared memory.
+    // Lane i's pair is broadcast and every lane forms (cs, sn) from it, stores the entry that became final and carries the
+    // other one on.  Q is then rotated one lane per row, right to left, carrying Q[p][cL+1].  Every element sees the same
+    // operations on the same operands in the same order as in the barrier-per-rotation loop of the callers (nAC > TEAM),
+    // so the factors are bit-identical; the chain costs one broadcast and the givens() of one pair per rotation, and the
+    // removal two barriers in all.  Ends without a barrier (the caller's next phase decides).  Needs nAC > i0.
+    static __device__ QP_FN void removal_chain_regs(int i0, int c0) {
+        QP_CTX
+        const int nFR = hdr[0], nAC = hdr[1];
+        double *Q = V_(Q), *RT = V_(RT), *t2 = V_(t2), *t3 = V_(t3);
+        const unsigned tm = team_mask<TEAM>();
+        constexpr int W = TEAM <= 32 ? TEAM : 32;
+        const bool own = lane >= i0 && lane < nAC;
+        double tb = own ? T_(lane, c0 - i0 + 1) : 0.0;  // running entry of column cL+1 of row `lane`
+        QP_U1 for (int i = i0; i < nAC; i++) {
+            const int cL = c0 - i;
+            const bool act = own && lane >= i;
+            const double ta = act ? T_(lane, cL) : 0.0;
+            double cs, sn, r;
+            givens(__shfl_sync(tm, ta, i, W), __shfl_sync(tm, tb, i, W), cs, sn, r);
+            if (act) {
+                T_(lane, cL + 1) = sn * ta + cs * tb;
+                tb = cs * ta - sn * tb;
+                if (lane == i) { T_(lane, cL) = 0.0; t2[i - i0] = cs; t3[i - i0] = sn; }
+            }
+        }
+        SYNC();
+        QP_U1 for (int p = lane; p < nFR; p += TEAM) {
+            double* q = Q + p * ld;
+            double qb = q[c0 - i0 + 1];
+            QP_U1 for (int i = i0; i < nAC; i++) {
+                const int cL = c0 - i;
+                const double cs = t2[i - i0], sn = t3[i - i0], qa = q[cL];
+                q[cL + 1] = sn * qa + cs * qb;
+                qb = cs * qa - sn * qb;
+            }
+            q[c0 - nAC + 1] = qb;
+        }
+    }
     static __device__ QP_FN void remove_constraint(int c) {
         QP_CTX
         const int nFR = hdr[0], nAC = hdr[1];
@@ -1697,6 +1743,9 @@ struct QPT {
         short *AC = AC_, *posAC = posAC_;
         const int k = posAC[c];
         SYNC();  // every thread holds nAC and k before lane 0 rewrites them below (the loops may be empty)
+        if (TEAM <= 32 && nAC <= TEAM) {
+            if (k + 1 < nAC) removal_chain_regs(k + 1, nFR - 1);  // its pass over Q and the row shift of T below share a phase
+        } else {
         QP_U1 for (int i = k + 1; i < nAC; i++) {
             int cL = nFR - 1 - i;
             double cs, sn, r;
@@ -1720,6 +1769,7 @@ struct QPT {
             }
             }
             SYNC();
+        }
         }
 #ifndef QP_EXACT
         if constexpr (TEAM > 32) rot_rows_auto(sA.oQ, nFR, nAC - k, sA.ot2, sA.ot3, nFR - 1 - k, -1);
@@ -1824,6 +1874,10 @@ struct QPT {
         if (lane == 0) { Q[nFR * ld + nFR] = 1.0; FR_[nFR] = (short)v; posFR_[v] = (short)nFR; sB_[v] = 0; hdr[0] = nFR + 1; if (nFR + 1 > hdr[6]) hdr[6] = nFR + 1; }
         nFR++;
         SYNC();
+        if (TEAM <= 32 && nAC <= TEAM) {
+            if (nAC > 0) { removal_chain_regs(0, nFR - 2); SYNC(); }
+            return 0;
+        }
         QP_U1 for (int i = 0; i < nAC; i++) {
             int cL = nFR - 2 - i;
             double cs, sn, r;
@@ -1927,19 +1981,21 @@ struct QPT {
     }
 
     // ---------------------------------------------------------------- step direction
-    // dxFX: full-length vector holding the bound shift of every fixed variable; dbAC by AC position; dgvec: gradient shift
+    // dxFX: full-length vector holding the bound shift of every fixed variable; dbAC by AC position; dgvec: gradient shift.
+    // Writes dx, dy and dAx = A dx.  The first loop reads only the entries of dxFX (and the caller's dbAC, dgvec) that the
+    // same lane wrote, so the caller needs no barrier between setting them up and this call; a product is formed by the lane
+    // that consumes its entry wherever the lane mappings allow it (same terms, same order as mulA / mulH / mulAT).
     static __device__ QP_FN void step_direction(const double* dgvec, const double* dxFX, double* dbAC) {
-        QP_CTX
+        QP_CTX QP_PAT
         const int nT = nV + nC;
         const int nFR = hdr[0], nAC = hdr[1], nZ = nFR - nAC;
-        double *dx = V_(dx), *dy = V_(dy), *t1 = V_(t1), *t2 = V_(t2), *t3 = V_(t3), *yv = V_(yv), *zv = V_(zv);
-        const double *Q = V_(Q), *RT = V_(RT);
+        double *dx = V_(dx), *dy = V_(dy), *dAx = V_(dAx), *t1 = V_(t1), *t3 = V_(t3), *yv = V_(yv), *zv = V_(zv);
+        const double *Q = V_(Q), *RT = V_(RT), *Av = V_(Av), *Hv = V_(Hv);
         const short *sB = sB_, *FR = FR_, *AC = AC_;
         QP_U1 for (int i = lane; i < nV; i += TEAM) dx[i] = (sB[i] != 0) ? dxFX[i] : 0.0;
         SYNC();
         if (nAC > 0) {
-            mulA(dx, t2);
-            QP_U1 for (int i = lane; i < nAC; i += TEAM) t3[i] = dbAC[i] - t2[AC[i]];
+            QP_U1 for (int i = lane; i < nAC; i += TEAM) t3[i] = dbAC[i] - A_row(pat, Av, dx, AC[i]);
             SYNC();
             solve_T(t3, yv);
 #ifndef QP_EXACT
@@ -1965,10 +2021,12 @@ struct QPT {
             } else
 #endif
             {
+            double* rinv = V_(dy);  // pivot reciprocals of the substitutions below (dy is dead here, rewritten below)
             QP_U1 for (int j = lane; j < nZ; j += TEAM) {
                 double s = 0.0;
                 DOT_UNROLL for (int p = 0; p < nFR; p++) { int v = FR[p]; s += Q[p * ld + j] * (t1[v] + dgvec[v]); }
                 zv[j] = -s;
+                rinv[j] = 1.0 / R_(j, j);
             }
             SYNC();
             }
@@ -1979,9 +2037,7 @@ struct QPT {
                 bwd_solve_R_blocked(zv, nZ);
                 PROF2_ADD(PR_RSOLVE);
             } else {
-                double* rinv = V_(dy);  // dy is dead here (rewritten below)
-                QP_U1 for (int k = lane; k < nZ; k += TEAM) rinv[k] = 1.0 / R_(k, k);
-                SYNC();
+                const double* rinv = V_(dy);
                 QP_U1 for (int k = 0; k < nZ; k++) {
                     double uk = quot(zv[k], R_(k, k), rinv[k]);
                     SYNC();
@@ -2011,8 +2067,7 @@ struct QPT {
             SYNC();
             }
         }
-        mulH(dx, t1);
-        QP_U1 for (int i = lane; i < nV; i += TEAM) t1[i] += dgvec[i];
+        QP_U1 for (int i = lane; i < nV; i += TEAM) t1[i] = H_row(pat, Hv, dx, i) + dgvec[i];
         QP_U1 for (int i = lane; i < nT; i += TEAM) dy[i] = 0.0;
         SYNC();
         if (nAC > 0) {
@@ -2034,52 +2089,62 @@ struct QPT {
             solve_Tt(yv, t3);
             QP_U1 for (int i = lane; i < nAC; i += TEAM) dy[nV + AC[i]] = t3[i];
             SYNC();
-            mulAT(dy + nV, t2);
-            QP_U1 for (int i = lane; i < nV; i += TEAM) if (sB[i] != 0) dy[i] = t1[i] - t2[i];
+            QP_U1 for (int i = lane; i < nV; i += TEAM) if (sB[i] != 0) dy[i] = t1[i] - AT_col(pat, Av, dy + nV, i);
         } else {
             QP_U1 for (int i = lane; i < nV; i += TEAM) if (sB[i] != 0) dy[i] = t1[i];
         }
+        QP_U1 for (int r = lane; r < nC; r += TEAM) dAx[r] = A_row(pat, Av, dx, r);
         SYNC();
     }
 
     // ---------------------------------------------------------------- drift correction / ramping
-    static __device__ QP_FN void stationarity_gradient() {  // g = A'y_c + y_b - (H+regI) x
-        QP_CTX
-        double *g = V_(g), *t1 = V_(t1), *t2 = V_(t2);
-        const double *x = V_(x), *y = V_(y);
-        mulAT(y + nV, t2);
-        mulH(x, t1);
-        QP_U1 for (int i = lane; i < nV; i += TEAM) g[i] = t2[i] + y[i] - t1[i];
+    // g = A'y_c + y_b - (H+regI) x, second phase: t1 = (H+regI) x is complete, and so is y.  One lane per column forms the
+    // column's product with y_c and combines it with the entries of y and t1 that the same lane wrote in the first phase.
+    static __device__ QP_FN void stationarity_gradient_tail() {
+        QP_CTX QP_PAT
+        double* g = V_(g);
+        const double *t1 = V_(t1), *y = V_(y), *Av = V_(Av);
+        QP_U1 for (int i = lane; i < nV; i += TEAM) g[i] = AT_col(pat, Av, y + nV, i) + y[i] - t1[i];
         SYNC();
     }
-    static __device__ QP_FN void drift_correction() {
+    static __device__ QP_FN void stationarity_gradient() {  // g = A'y_c + y_b - (H+regI) x
         QP_CTX
-        double *x = V_(x), *y = V_(y), *Ax = V_(Ax), *lb = V_(lb), *ub = V_(ub), *lbA = V_(lbA), *ubA = V_(ubA);
+        mulH(V_(x), V_(t1));
+        stationarity_gradient_tail();
+    }
+    // Two phases: (1) A x, the bounds and the clamped multipliers, each lane on the entries it owns, and t1 = (H+regI) x;
+    // (2) the gradient (stationarity_gradient_tail).  The clamps of y depend only on the statuses and y itself, and lane r
+    // updates lbA[r] / ubA[r] from the (A x)[r] it holds in a register.
+    static __device__ QP_FN void drift_correction() {
+        QP_CTX QP_PAT
+        double *x = V_(x), *y = V_(y), *Ax = V_(Ax), *lb = V_(lb), *ub = V_(ub), *lbA = V_(lbA), *ubA = V_(ubA), *t1 = V_(t1);
+        const double *Av = V_(Av), *Hv = V_(Hv);
         const short *sB = sB_, *sC = sC_;
-        mulA(x, Ax);
         QP_U1 for (int i = lane; i < nV; i += TEAM) {
             int s = sB[i]; double xi = x[i];
             if (s < 0) { lb[i] = xi; if (ub[i] < xi) ub[i] = xi; if (y[i] < 0) y[i] = 0.0; }
             else if (s > 0) { ub[i] = xi; if (lb[i] > xi) lb[i] = xi; if (y[i] > 0) y[i] = 0.0; }
             else { if (lb[i] > xi) lb[i] = xi; if (ub[i] < xi) ub[i] = xi; y[i] = 0.0; }
+            t1[i] = H_row(pat, Hv, x, i);
         }
         QP_U1 for (int i = lane; i < nC; i += TEAM) {
-            int s = sC[i]; double ax = Ax[i];
+            int s = sC[i]; double ax = A_row(pat, Av, x, i);
+            Ax[i] = ax;
             if (s < 0) { lbA[i] = ax; if (ubA[i] < ax) ubA[i] = ax; if (y[nV + i] < 0) y[nV + i] = 0.0; }
             else if (s > 0) { ubA[i] = ax; if (lbA[i] > ax) lbA[i] = ax; if (y[nV + i] > 0) y[nV + i] = 0.0; }
             else { if (lbA[i] > ax) lbA[i] = ax; if (ubA[i] < ax) ubA[i] = ax; y[nV + i] = 0.0; }
         }
         SYNC();
-        stationarity_gradient();
+        stationarity_gradient_tail();
     }
-    static __device__ QP_FN void ramping() {
-        QP_CTX
-        double *x = V_(x), *y = V_(y), *Ax = V_(Ax), *lb = V_(lb), *ub = V_(ub), *lbA = V_(lbA), *ubA = V_(ubA);
+    static __device__ QP_FN void ramping() {  // same two phases as drift_correction
+        QP_CTX QP_PAT
+        double *x = V_(x), *y = V_(y), *Ax = V_(Ax), *lb = V_(lb), *ub = V_(ub), *lbA = V_(lbA), *ubA = V_(ubA), *t1 = V_(t1);
+        const double *Av = V_(Av), *Hv = V_(Hv);
         const short *sB = sB_, *sC = sC_;
         const int ramp_offset = hdr[2];
         const int nRamp = nV + nC + nC + nV;
         const double r0 = 0.5, r1 = 1.0;
-        mulA(x, Ax);
         QP_U1 for (int i = lane; i < nV; i += TEAM) {
             double tP = (double)((i + ramp_offset) % nRamp) / (double)(nRamp - 1);
             double rP = (1.0 - tP) * r0 + tP * r1;
@@ -2093,13 +2158,15 @@ struct QPT {
             if (s < 0) { lb[i] = xi; y[i] = rD; }
             if (s > 0) { ub[i] = xi; y[i] = -rD; }
             if (s == 0) y[i] = 0.0;
+            t1[i] = H_row(pat, Hv, x, i);
         }
         QP_U1 for (int i = lane; i < nC; i += TEAM) {
             double tP = (double)((nV + i + ramp_offset) % nRamp) / (double)(nRamp - 1);
             double rP = (1.0 - tP) * r0 + tP * r1;
             double tD = (double)((nV + nC + nV + i + ramp_offset) % nRamp) / (double)(nRamp - 1);
             double rD = (1.0 - tD) * r0 + tD * r1;
-            double ax = Ax[i];
+            double ax = A_row(pat, Av, x, i);
+            Ax[i] = ax;
             double sca = fabs(ax) > 1.0 ? fabs(ax) : 1.0;
             int s = sC[i];
             if (s >= 0) lbA[i] = ax - sca * rP;
@@ -2108,10 +2175,9 @@ struct QPT {
             if (s > 0) { ubA[i] = ax; y[nV + i] = -rD; }
             if (s == 0) y[nV + i] = 0.0;
         }
-        SYNC();
-        stationarity_gradient();
+        SYNC();  // also: every lane has read ramp_offset
         if (lane == 0) hdr[2] = ramp_offset + 1;
-        SYNC();
+        stationarity_gradient_tail();
     }
 
     // ---------------------------------------------------------------- exchange (ensure LI)
@@ -2119,21 +2185,19 @@ struct QPT {
     static __device__ QP_FN int ensure_li(int c, int v, int status) {
         QP_CTX QP_PAT
         const int nFR = hdr[0], nAC = hdr[1], nZ = nFR - nAC;
-        double *xiC = V_(zv), *xiB = V_(dx), *yv = V_(yv), *t2 = V_(t2), *t3 = V_(t3), *y = V_(y);
-        const double *w = V_(w), *Av = V_(Av);
+        double *xiC = V_(zv), *xiB = V_(dx), *t3 = V_(t3), *y = V_(y), *w = V_(w);
+        const double* Av = V_(Av);
         const short *sB = sB_, *sC = sC_, *AC = AC_, *posAC = posAC_;
-        QP_U1 for (int j = nZ + lane; j < nFR; j += TEAM) yv[j] = w[j];
-        SYNC();
-        solve_Tt(yv, xiC);
+        (void)nZ;
+        solve_Tt(w, xiC);  // may destroy w[nZ..nFR): the caller forms w again after the exchange
         QP_U1 for (int i = lane; i < nC; i += TEAM) { int p = posAC[i]; t3[i] = (p >= 0) ? xiC[p] : 0.0; }
         SYNC();
-        mulAT(t3, t2);
         QP_U1 for (int i = lane; i < nV; i += TEAM) {
             if (sB[i] == 0) { xiB[i] = 0.0; continue; }
             double ai = (c >= 0) ? A_entry(pat, Av, c, i) : 0.0;
-            xiB[i] = ai - t2[i];
+            xiB[i] = ai - AT_col(pat, Av, t3, i);
         }
-        SYNC();
+        // no barrier: the scan reads only the xiB[i] this lane wrote, and xiC, complete since solve_Tt's barrier
         const double sgn = (status < 0) ? 1.0 : -1.0;
         double best = QP_INFTY; int bpos = 0x7fffffff;
         QP_U1 for (int i = lane; i < nAC; i += TEAM) {
@@ -2188,9 +2252,7 @@ struct QPT {
                 a[i] = gN[i] - g[i];
             }
             QP_U1 for (int i = lane; i < nAC; i += TEAM) { int ci = AC[i]; w[nV + i] = sC[ci] < 0 ? (lbAN[ci] - lbA[ci]) : (ubAN[ci] - ubA[ci]); }
-            SYNC();
-            step_direction(a, w, w + nV);
-            mulA(dx, dAx);
+            step_direction(a, w, w + nV);  // reads w[i] of this lane before its first barrier (no barrier needed here); dAx too
             PROF_ADD(PR_STEPDIR);
 
             // ---- ratio tests: position = scan order of the sequential rule
