@@ -21,11 +21,9 @@ HEADERS = [os.path.join(CSRC, f) for f in ("qp_kernel.cuh", "l0_kernels.cuh", "t
 TEAMS = [(32, 128, 16), (32, 64, 16), (32, 32, 16), (32, 128, 32),
          # sub-warp teams: 16 / 8 lanes per QP (2 / 4 QPs per warp) for QPs with nV <= 16 / <= 8
          (16, 128, 16), (8, 128, 16)]
-LARGE_CTA = int(os.environ.get("SQPB200_LARGE_CTA", "512"))  # threads of the one-QP-per-CTA kernel (large QPs)
 QP_EXTRA_FLAGS = os.environ.get("SQPB200_QP_FLAGS", "").split()
-# SQPB200_FMAD=true: experiment only -- contraction into FMA breaks the bit-for-bit agreement of the warp kernel with the oracle
-NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
-              "-fmad=" + os.environ.get("SQPB200_FMAD", "false"), "-Xcompiler", "-fPIC"]
+NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-fmad=false",
+              "-Xcompiler", "-fPIC"]
 
 
 def _nvcc():
@@ -41,8 +39,7 @@ def _units():
         # multi-warp teams are compiled fully inlined (see the QP_INLINE_ALL note in qp_kernel.cuh)
         units.append((os.path.join(CSRC, "qp_solve_inst.cu"), os.path.join(OBJDIR, "qp_solve_%d_%d_w%d.o" % (team, cta, wps)),
                       ["-DQP_TEAM=%d" % team, "-DQP_CTA=%d" % cta, "-DQP_WPS=%d" % wps] + QP_EXTRA_FLAGS))
-    units.append((os.path.join(CSRC, "qp_solve_large_inst.cu"), os.path.join(OBJDIR, "qp_solve_large.o"),
-                  ["-DQP_CTA=%d" % LARGE_CTA] + QP_EXTRA_FLAGS))
+    units.append((os.path.join(CSRC, "qp_solve_large_inst.cu"), os.path.join(OBJDIR, "qp_solve_large.o"), QP_EXTRA_FLAGS))
     return units
 
 

@@ -710,7 +710,7 @@ static bool config_for_cap(sqpb200_handle h, int cap, SolveCfg& cfg, bool allow_
     const size_t slice_bytes = (size_t)a.slice_doubles * 8, pat_bytes = (size_t)a.pat_shorts * 2;
     const size_t SMEM_MAX = 227 * 1024, SMEM_SM = 228 * 1024;
     cfg.lanes = 32;
-    if (allow_subwarp && h->nV <= 16 && !getenv("SQPB200_NO_SUBWARP")) {
+    if (allow_subwarp && h->nV <= 16) {
         const int lanes = h->nV <= 8 ? 8 : 16, teams = 128 / lanes;
         const size_t smem = (size_t)teams * slice_bytes + pat_bytes;
         if (smem <= SMEM_MAX) {
@@ -725,9 +725,7 @@ static bool config_for_cap(sqpb200_handle h, int cap, SolveCfg& cfg, bool allow_
     }
     int best_teams = 0;
     size_t best_res = 0;
-    const char* force = getenv("SQPB200_QPS_PER_CTA");  // experiment knob: force 1, 2 or 4 QPs per CTA
     for (int teams = 4; teams >= 1; teams >>= 1) {
-        if (force && atoi(force) != teams) continue;
         size_t smem = (size_t)teams * slice_bytes + pat_bytes;
         if (smem > SMEM_MAX) continue;
         size_t ctas = SMEM_SM / (smem + 1024 + 512);  // 1 KiB per CTA reserved by the driver + the static argument copy
@@ -796,7 +794,6 @@ cudaError_t launch_qp_solve_32_32_w16(const QPKernelArgs&, int, cudaStream_t);
 cudaError_t launch_qp_solve_16_128_w16(const QPKernelArgs&, int, cudaStream_t);
 cudaError_t launch_qp_solve_8_128_w16(const QPKernelArgs&, int, cudaStream_t);
 cudaError_t launch_qp_solve_large(const QPKernelArgs&, cudaStream_t);
-int qp_solve_large_threads();
 }
 
 // global-memory slices and the 32-bit pattern of the one-QP-per-CTA kernel
@@ -852,15 +849,6 @@ int sqpb200_device_buffers(sqpb200_handle h, void** out) {
     out[0] = h->dx; out[1] = h->dy; out[2] = h->dobj; out[3] = h->dstatus; out[4] = h->diters; out[5] = h->dkkt;
     return 0;
 }
-// SQPB200_LARGE_RECOMPUTE=1: the one-QP-per-cluster kernel recomputes R after every addition instead of updating it
-static bool large_recompute() {
-    static const bool v = [] { const char* e = getenv("SQPB200_LARGE_RECOMPUTE"); return e && e[0] == '1'; }();
-    return v;
-}
-static bool flip_as_hotstart() {
-    static const bool v = [] { const char* e = getenv("SQPB200_FLIP_AS_HOTSTART"); return e && e[0] == '1'; }();
-    return v;
-}
 static int solve_impl(sqpb200_handle h, int mode_qp, int maxiter, const unsigned char* active_mask, bool mask_on_device, signed char* inst_state) {
     if (!h) return SQPB200_ERR_INVALID;
     CK(cudaSetDevice(h->device));
@@ -892,7 +880,7 @@ static int solve_impl(sqpb200_handle h, int mode_qp, int maxiter, const unsigned
     a.max_iter = maxiter > 0 ? maxiter : (is_lp ? h->opt.lp_maxiter : h->opt.qp_maxiter);
     a.flags = (h->opt.enable_flipping ? FLAG_FLIPPING : 0) | (h->opt.enable_ramping ? FLAG_RAMPING : 0) |
               (h->opt.enable_drift ? FLAG_DRIFT : 0) | (h->opt.keep_state ? FLAG_KEEP_STATE : 0) |
-              (h->opt.debug_force_error_branch ? FLAG_FORCE_GUESS : 0) | ((large_recompute() || h->opt.refactorise_every == 1) ? FLAG_NO_CARRY : 0) | (flip_as_hotstart() ? FLAG_FLIP_AS_HOTSTART : 0);
+              (h->opt.debug_force_error_branch ? FLAG_FORCE_GUESS : 0) | (h->opt.refactorise_every == 1 ? FLAG_NO_CARRY : 0);
     a.mode = mode;
     a.Ap = h->dAp; a.Ai = h->dAi; a.Arp = h->dArp; a.Aci = h->dAci; a.Aperm = h->dAperm;
     a.Hp = h->dHp; a.Hi = h->dHi;

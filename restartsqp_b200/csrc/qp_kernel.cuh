@@ -59,8 +59,7 @@ enum { MODE_COLD = 0, MODE_HOT_FIXED = 1, MODE_HOT_VARIED = 2,
        MODE_REINIT = 3 /* FIXED <-> VARIED flip of the matrix status: init from the previous solution (src/qpOASESInterface.cpp:202-207) */ };
 enum { FLAG_FLIPPING = 1, FLAG_RAMPING = 2, FLAG_DRIFT = 4, FLAG_KEEP_STATE = 8,
        FLAG_FORCE_GUESS = 16 /* test hook: take handle_error's infeasible branch whatever the first attempt returned */,
-       FLAG_NO_CARRY = 32 /* one-QP-per-cluster kernel: recompute R after every addition (as the warp kernel does) instead of updating it */,
-       FLAG_FLIP_AS_HOTSTART = 64 /* experiment (SQPB200_FLIP_AS_HOTSTART=1): the matrix-status flip as a hot start with new matrices, round 1's approximation */ };
+       FLAG_NO_CARRY = 32 /* one-QP-per-cluster kernel: recompute R after every addition (as the warp kernel does) instead of updating it */ };
 
 struct QPKernelArgs {
     int batch, nV, nC;
@@ -169,14 +168,9 @@ __device__ __forceinline__ double quot(double x, double d, double ri) {
 }
 
 #define QP_FN __noinline__
-// loop unrolling of the solver's loops: 1 = smallest code (10.6 k SASS instructions).  Measured with -DQP_UNROLL_N=4 (59 k
+// loop unrolling of the solver's loops: 1 = smallest code (10.6 k SASS instructions).  Measured with unroll 4 (59 k
 // instructions): 1.3x-3x slower on every dumped QP (instruction-cache misses), so 1 is what ships.
-#ifndef QP_UNROLL_N
-#define QP_UNROLL_N 1
-#endif
-#define QP_STR_(x) #x
-#define QP_STR(x) QP_STR_(x)
-#define QP_U1 _Pragma(QP_STR(unroll QP_UNROLL_N))
+#define QP_U1 _Pragma("unroll 1")
 // Phase timers of a -DQP_PROFILE build (tools/large_try.py, tools/per_fixture.py print them): the first thread of every team adds
 // the clock64() cycles it spent in phase i to A.prof[i].  Phase boundaries are team barriers, so one thread's clock is the team's.
 #ifdef QP_PROFILE
@@ -241,15 +235,11 @@ __shared__ int sRedP[32];
 #define T_(i, j) RT[(cap - 1 - (i)) * ld + (j)]
 // inner sequential sums: not unrolled in the warp kernel (instruction-cache footprint), unrolled 8x in the CTA kernel so
 // that the loads of consecutive terms overlap (the additions stay in order: no reassociation without fast-math)
-#ifndef QP_DOT_UNROLL_N
-#define QP_DOT_UNROLL_N 1
-#endif
-#define DOT_UNROLL _Pragma("unroll (TEAM <= 32 ? DOT_N_SMALL : 8)")
+#define DOT_UNROLL _Pragma("unroll (TEAM <= 32 ? 1 : 8)")
 #define SYNC() do { if (TEAM <= 32) __syncwarp(team_mask<TEAM>()); else __syncthreads(); } while (0)
 
 template <int TEAM>
 struct QPT {
-    static constexpr int DOT_N_SMALL = QP_DOT_UNROLL_N;  // a macro is not expanded inside the pragma's string
     typedef typename PatIdx<TEAM>::type pidx;
     // ---------------------------------------------------------------- sparse products
     // One entry of each product, summed in storage order.  The mul* functions below run one lane per entry and end in a
@@ -370,12 +360,10 @@ struct QPT {
         if (sA.is_lp) {
             double sr = sqrt(QP_EPS_REG);
             QP_U1 for (int k = lane; k < nZ * nZ; k += TEAM) { int a_ = k / nZ, b_ = k % nZ; R_(a_, b_) = (a_ == b_) ? sr : 0.0; }
-#ifndef QP_EXACT
             if constexpr (TEAM > 32) {  // block inverses used by the triangular solves
                 double* W = V_(W);
                 for (int k = lane; k < nZ * 64; k += TEAM) { const int a_ = k >> 6, c_ = k & 63; if (c_ < ld) W[(size_t)a_ * ld + c_] = (c_ == (a_ & 63)) ? 1.0 / sr : 0.0; }
             }
-#endif
             SYNC();
             return 0;
         }
@@ -440,207 +428,11 @@ struct QPT {
         PROF_ADD(PR_REFAC_CHOL);
         return 0;
     }
-#ifdef QP_EXACT
-    // ---- CTA kernel: blocked refactorisation.  Same arithmetic as the column-by-column version above, term for term and in
-    // the same order per element (every sum runs over its index in ascending order), reorganised so that the O(nZ^2 nFR)
-    // and O(nZ^3) parts are shared-memory tiled contractions instead of latency-bound dot products:
-    //   A  W[p][b] = ((H + reg I) z_b)[FR[p]]            sparse x dense, one thread per entry
-    //   B  M[a][b] = sum_p Q[p][a] W[p][b], a <= b        tiles of TA x 64 outputs, 16 terms per stage
-    //   C  left-looking Cholesky by blocks of TA rows: the terms k < i0 of a block row as a tiled contraction (C1), the
-    //      terms i0 <= k < i row by row inside the block (C2).
-    // C(a0+., b0+.) (+|-)= sum_{k<K} X[k][xo+a] Y[k][yo+b]; tile TA x 64; stores only entries with a <= b (global indices
-    // ga = a0+a, gb = b0+b relative to the same origin), ga < na, gb < nb.
-    template <int SIGN>
-    static __device__ __forceinline__ void tile_contract(const double* X, int xo, const double* Y, int yo, int K, double* C,
-                                                         int a0, int na, int b0, int nb, int ld, bool init_zero) {
-        constexpr int TA = TEAM / 8, TB = 64, KC = 16;
-        __shared__ double Xs[KC][TA + 2];
-        __shared__ double Ys[KC][TB + 2];
-        const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-        const int ga0 = a0 + ty * 2, gb0 = b0 + tx * 4;
-        double acc[2][4];
-#pragma unroll
-        for (int i = 0; i < 2; i++)
-#pragma unroll
-            for (int j = 0; j < 4; j++) {
-                const int ga = ga0 + i, gb = gb0 + j;
-                acc[i][j] = (!init_zero && ga < na && gb < nb && ga <= gb) ? C[ga * ld + gb] : 0.0;
-            }
-        QP_U1 for (int k0 = 0; k0 < K; k0 += KC) {
-            const int kc = (K - k0 < KC) ? K - k0 : KC;
-            __syncthreads();  // previous stage consumed
-            for (int e = tid; e < KC * TA; e += TEAM) {
-                const int k = e / TA, c = e % TA;
-                Xs[k][c] = (k < kc && a0 + c < na) ? X[(k0 + k) * ld + xo + a0 + c] : 0.0;
-            }
-            for (int e = tid; e < KC * TB; e += TEAM) {
-                const int k = e / TB, c = e % TB;
-                Ys[k][c] = (k < kc && b0 + c < nb) ? Y[(k0 + k) * ld + yo + b0 + c] : 0.0;
-            }
-            __syncthreads();
-            _Pragma("unroll 4") for (int k = 0; k < kc; k++) {
-                const double x0 = Xs[k][ty * 2], x1 = Xs[k][ty * 2 + 1];
-                const double y0 = Ys[k][tx * 4], y1 = Ys[k][tx * 4 + 1], y2 = Ys[k][tx * 4 + 2], y3 = Ys[k][tx * 4 + 3];
-                if (SIGN > 0) {
-                    acc[0][0] += x0 * y0; acc[0][1] += x0 * y1; acc[0][2] += x0 * y2; acc[0][3] += x0 * y3;
-                    acc[1][0] += x1 * y0; acc[1][1] += x1 * y1; acc[1][2] += x1 * y2; acc[1][3] += x1 * y3;
-                } else {
-                    acc[0][0] -= x0 * y0; acc[0][1] -= x0 * y1; acc[0][2] -= x0 * y2; acc[0][3] -= x0 * y3;
-                    acc[1][0] -= x1 * y0; acc[1][1] -= x1 * y1; acc[1][2] -= x1 * y2; acc[1][3] -= x1 * y3;
-                }
-            }
-        }
-#pragma unroll
-        for (int i = 0; i < 2; i++)
-#pragma unroll
-            for (int j = 0; j < 4; j++) {
-                const int ga = ga0 + i, gb = gb0 + j;
-                if (ga < na && gb < nb && ga <= gb) C[ga * ld + gb] = acc[i][j];
-            }
-    }
-    static __device__ QP_FN int recompute_R_blocked() {
-        QP_CTX QP_PAT
-        constexpr int TA = TEAM / 8;
-        const int nFR = hdr[0], nAC = hdr[1], nZ = nFR - nAC;
-        double *RT = V_(RT), *W = V_(W);
-        const double *Q = V_(Q), *Hv = V_(Hv);
-        const short *FR = FR_, *posFR = posFR_;
-        const pidx *Hp = pat + sA.pHp, *Hi = pat + sA.pHi;
-        const bool has_H = sA.has_H && !sA.is_lp;
-        PROF_T0
-        // A: W[p][b]
-        QP_U1 for (int e = lane; e < nFR * nZ; e += TEAM) {
-            const int p = e / nZ, b = e % nZ;
-            double s = 0.0;
-            if (has_H) {
-                const int c = FR[p], e1 = Hp[c + 1];
-                QP_U1 for (int h = Hp[c]; h < e1; h++) {
-                    const int pr = posFR[Hi[h]];
-                    s += Hv[h] * ((pr >= 0) ? Q[pr * ld + b] : 0.0);
-                }
-            }
-            W[p * ld + b] = s;
-        }
-        SYNC();
-        PROF_ADD(PR_REFAC_W);
-        // B: M (upper triangle) into R
-        QP_U1 for (int b0 = 0; b0 < nZ; b0 += 64)
-            QP_U1 for (int a0 = 0; a0 < b0 + 64 && a0 < nZ; a0 += TA)
-                tile_contract<1>(Q, 0, W, 0, nFR, RT, a0, nZ, b0, nZ, ld, true);
-        SYNC();
-        PROF_ADD(PR_REFAC_M);
-        // C: Cholesky by block rows
-        QP_U1 for (int i0 = 0; i0 < nZ; i0 += TA) {
-            const int i1 = (i0 + TA < nZ) ? i0 + TA : nZ;
-            if (i0 > 0) {
-                // rows i0..i1, columns >= i0: subtract the terms k < i0.  Row/column indices are taken relative to i0 so that
-                // the tile's "a <= b" rule is the upper-triangle rule of the block row.
-                QP_U1 for (int b0 = 0; b0 < nZ - i0; b0 += 64)
-                    tile_contract<-1>(RT, i0, RT, i0, i0, RT + i0 * ld + i0, 0, i1 - i0, b0, nZ - i0, ld, false);
-                SYNC();
-            }
-            QP_U1 for (int i = i0; i < i1; i++) {
-                QP_U1 for (int j = i + lane; j < nZ; j += TEAM) {
-                    double s = R_(i, j);
-                    DOT_UNROLL for (int k = i0; k < i; k++) s -= R_(k, i) * R_(k, j);
-                    R_(i, j) = s;
-                }
-                SYNC();
-                const double d = R_(i, i);
-                SYNC();
-                if (!(d > QP_ZERO)) return 1 + i;
-                const double dd = sqrt(d);
-                QP_U1 for (int j = i + lane; j < nZ; j += TEAM) R_(i, j) = (j == i) ? dd : R_(i, j) / dd;
-                QP_U1 for (int j = lane; j < i; j += TEAM) R_(i, j) = 0.0;
-                SYNC();
-            }
-        }
-        PROF_ADD(PR_REFAC_CHOL);
-        return 0;
-    }
-    // ---- CTA kernel: blocked triangular solves with R.  The column-oriented substitutions above need two team barriers per
-    // unknown; here one warp solves a 32 x 32 diagonal block out of shared memory (shuffles, no barrier) and the whole team
-    // then applies the block's 32 columns to the trailing unknowns.  Per unknown the terms are subtracted in the same order
-    // (ascending k forward, descending k backward) and divided by the same pivot, so results are bit-identical.
-    static __device__ __forceinline__ double (*diag_tile())[33] {
-        __shared__ double Ds[32][33];
-        return Ds;
-    }
-    // R' u = z (n unknowns, in place); col >= 0: also R(k, col) = u_k
-    static __device__ QP_FN void fwd_solve_R_blocked(double* z, int n, int col) {
-        QP_CTX
-        double* RT = V_(RT);
-        double (*Ds)[33] = diag_tile();
-        const int l = lane & 31;
-        // the diagonal tile of block I+1 is fetched while block I's columns are applied to the trailing unknowns
-        auto load_tile = [&](int j0) {
-            const int mb = (n - j0 < 32) ? n - j0 : 32;
-            QP_U1 for (int e = lane; e < 32 * 32; e += TEAM) { const int k = e >> 5, i = e & 31; if (k < mb && i < mb && k <= i) Ds[k][i] = R_(j0 + k, j0 + i); }
-        };
-        if (n > 0) load_tile(0);
-        SYNC();
-        QP_U1 for (int i0 = 0; i0 < n; i0 += 32) {
-            const int nb = (n - i0 < 32) ? n - i0 : 32;
-            if (lane < 32) {
-                double zi = (l < nb) ? z[i0 + l] : 0.0;
-                const double ri = (l < nb) ? 1.0 / Ds[l][l] : 0.0;  // pivot reciprocals in parallel; the chain only multiplies
-                QP_U1 for (int k = 0; k < nb; k++) {
-                    const double uk = quot(__shfl_sync(0xffffffffu, zi, k), Ds[k][k], __shfl_sync(0xffffffffu, ri, k));
-                    if (l == k) zi = uk;
-                    else if (l > k && l < nb) zi -= Ds[k][l] * uk;
-                }
-                if (l < nb) { z[i0 + l] = zi; if (col >= 0) R_(i0 + l, col) = zi; }
-            }
-            SYNC();
-            QP_U1 for (int i = i0 + nb + lane; i < n; i += TEAM) {
-                double s = z[i];
-                _Pragma("unroll 16") for (int k = 0; k < nb; k++) s -= R_(i0 + k, i) * z[i0 + k];  // 16 loads in flight per thread
-                z[i] = s;
-            }
-            if (i0 + 32 < n) load_tile(i0 + 32);
-            SYNC();
-        }
-    }
-    // R v = z (n unknowns, in place)
-    static __device__ QP_FN void bwd_solve_R_blocked(double* z, int n) {
-        QP_CTX
-        const double* RT = V_(RT);
-        double (*Ds)[33] = diag_tile();
-        const int l = lane & 31;
-        auto load_tile = [&](int j0) {
-            const int mb = (n - j0 < 32) ? n - j0 : 32;
-            QP_U1 for (int e = lane; e < 32 * 32; e += TEAM) { const int k = e >> 5, i = e & 31; if (k < mb && i < mb && k <= i) Ds[k][i] = R_(j0 + k, j0 + i); }
-        };
-        if (n > 0) load_tile(((n - 1) >> 5) << 5);
-        SYNC();
-        QP_U1 for (int i0 = ((n - 1) >> 5) << 5; i0 >= 0; i0 -= 32) {
-            const int nb = (n - i0 < 32) ? n - i0 : 32;
-            if (lane < 32) {
-                double zi = (l < nb) ? z[i0 + l] : 0.0;
-                const double ri = (l < nb) ? 1.0 / Ds[l][l] : 0.0;
-                QP_U1 for (int k = nb - 1; k >= 0; k--) {
-                    const double zk = quot(__shfl_sync(0xffffffffu, zi, k), Ds[k][k], __shfl_sync(0xffffffffu, ri, k));
-                    if (l == k) zi = zk;
-                    else if (l < k) zi -= Ds[l][k] * zk;
-                }
-                if (l < nb) z[i0 + l] = zi;
-            }
-            SYNC();
-            QP_U1 for (int i = lane; i < i0; i += TEAM) {
-                double s = z[i];
-                _Pragma("unroll 16") for (int k = nb - 1; k >= 0; k--) s -= R_(i, i0 + k) * z[i0 + k];
-                z[i] = s;
-            }
-            if (i0 >= 32) load_tile(i0 - 32);
-            SYNC();
-        }
-    }
-#else
 
     // =====================================================================================================================
     // One-QP-per-CTA kernel (TEAM == 512), B200 form of the O(n^3) part and of the triangular solves.  Parity gate for
     // this kernel is north_star's (identical working sets, 1e-8 relative): sums run on the FP64 tensor cores, whose
-    // accumulation order differs from the oracle's; -DQP_EXACT keeps the bit-exact scalar version above for debugging.
+    // accumulation order differs from the oracle's.
     //
     //   * contraction tiles C(64x64) (+|-)= X' Y on FP64 DMMA (mma.sync.m8n8k4.f64; 16 warps x (16x16) sub-tiles), operands
     //     staged by 1-D TMA bulk copies (one per 512-byte tile row, issued by warp 0) into a 3-stage shared-memory ring
@@ -1162,10 +954,7 @@ struct QPT {
     // ---- operations the leader shares with its helper CTAs: arguments go through the slice header (ints 4..15), offsets are
     // in doubles from the slice base.  Worth two cluster barriers only when the operand is large.
     enum { OP_REFAC = 1, OP_EXIT = 2, OP_COLSUMS = 3, OP_ROWSUMS = 4, OP_ROTROWS = 5, OP_DINV = 6 };
-#ifndef QP_DIST_MIN_ELEMS
-#define QP_DIST_MIN_ELEMS (1 << 16)
-#endif
-    static constexpr int DIST_MIN_ELEMS = QP_DIST_MIN_ELEMS;  // below ~0.5 MB of factor data the leader works alone (measured: 1 << 16 beats 1 << 17 by 3-6 %, 1 << 19 loses 10-20 %)
+    static constexpr int DIST_MIN_ELEMS = 1 << 16;  // below ~0.5 MB of factor data the leader works alone (measured: 1 << 16 beats 1 << 17 by 3-6 %, 1 << 19 loses 10-20 %)
     static __device__ __forceinline__ void run_op(int cmd, int rank, int cs) {
         QP_CTX
         volatile int* vh = hdr;
@@ -1207,10 +996,7 @@ struct QPT {
     // (Z G)'H(Z G) restricted to the kept columns, the same matrix a recomputation factorises, in O(nZ^2) (qpOASES's own
     // update under its default options).  A full recomputation still runs every REFAC_EVERY additions, after an exchange
     // step (R is one column short there) and after a flipped bound.
-#ifndef QP_REFAC_EVERY
-#define QP_REFAC_EVERY 64
-#endif
-    static constexpr int REFAC_EVERY = QP_REFAC_EVERY;
+    static constexpr int REFAC_EVERY = 64;
     // inverses of the 64 x 64 diagonal blocks of R (n x n) into W, block b by CTA b % cs
     static __device__ __forceinline__ void dinv_blocks(int n, int rank, int cs) {
         QP_CTX
@@ -1382,13 +1168,10 @@ struct QPT {
         PROF_T0
         rot_rows_auto(sA.oRT, nZ, nZ, sA.ot2, sA.ot3, 0, 1, true);
         PROF_ADD(PR_REFAC_W);  // (profile build: the three slots of the recomputation show the update's steps)
-#ifndef QP_RETRI_DEPTH
-#define QP_RETRI_DEPTH 4
-#endif
         // (a panel variant -- one warp eliminating 32 columns out of registers, then all threads applying the 32 rotations to
         // their columns -- measured no faster: the chain of dependent FP64 operations per rotation, ~0.3 us, is what bounds all
         // three forms)
-        if (m <= TEAM) retriangularise<1, QP_RETRI_DEPTH>(nZ);
+        if (m <= TEAM) retriangularise<1, 4>(nZ);
         else if (m <= 4 * TEAM) retriangularise4(nZ);
         else retriangularise<8, 4>(nZ);
         PROF_ADD(PR_REFAC_M);
@@ -1535,7 +1318,6 @@ struct QPT {
         } else if (tid == c) W[(size_t)(i0 + c) * ld + c] = 1.0 / rho;
         __syncthreads();
     }
-#endif  // QP_EXACT
     // border R with the new last null-space column; returns 1 if curvature acceptable
     static __device__ QP_FN int extend_R(int check_curvature) {
         QP_CTX
@@ -1545,22 +1327,18 @@ struct QPT {
             QP_U1 for (int a_ = lane; a_ < b; a_ += TEAM) { R_(a_, b) = 0.0; R_(b, a_) = 0.0; }
             if (lane == 0) R_(b, b) = sqrt(QP_EPS_REG);
             SYNC();
-#ifndef QP_EXACT
             if constexpr (TEAM > 32) extend_Dinv(b, sqrt(QP_EPS_REG));
-#endif
             return 1;
         }
         const double *Q = V_(Q), *t2 = V_(t2);
         const short* FR = FR_;
         proj_column(b);
-#ifndef QP_EXACT
         if constexpr (TEAM > 32) {
             double* tmp = V_(a);  // dead between two homotopy steps
             for (int p = lane; p < nFR; p += TEAM) tmp[p] = t2[FR[p]];
             SYNC();
             col_sums_auto(sA.oQ, nFR, 0, b + 1, sA.oa, sA.ow, false);
         } else
-#endif
         {
         QP_U1 for (int a_ = lane; a_ <= b; a_ += TEAM) {
             double s = 0.0;
@@ -1584,13 +1362,11 @@ struct QPT {
         }
         }
         double rho2 = w[b];
-#ifndef QP_EXACT
         if constexpr (TEAM > 32) {
             double part = 0.0;
             for (int k = lane; k < b; k += TEAM) part += R_(k, b) * R_(k, b);
             rho2 -= team_sum(part);
         } else
-#endif
         {
         DOT_UNROLL for (int k = 0; k < b; k++) rho2 -= R_(k, b) * R_(k, b);
         }
@@ -1600,9 +1376,7 @@ struct QPT {
         if (lane == 0) R_(b, b) = sqrt(rho2);
         QP_U1 for (int a_ = lane; a_ < b; a_ += TEAM) R_(b, a_) = 0.0;
         SYNC();
-#ifndef QP_EXACT
         if constexpr (TEAM > 32) extend_Dinv(b, sqrt(rho2));
-#endif
         return 1;
     }
 
@@ -1615,7 +1389,6 @@ struct QPT {
         const short* FR = FR_;
         QP_U1 for (int p = lane; p < nFR; p += TEAM) a[p] = A_entry(pat, Av, c, FR[p]);
         SYNC();
-#ifndef QP_EXACT
         if constexpr (TEAM > 32) {
             col_sums_auto(sA.oQ, nFR, 0, nFR, sA.oa, sA.ow, false);
             double s2p = 0.0, z2p = 0.0;
@@ -1625,7 +1398,6 @@ struct QPT {
             SYNC();
             return;
         }
-#endif
         QP_U1 for (int j = lane; j < nFR; j += TEAM) {
             double s = 0.0;
             DOT_UNROLL for (int p = 0; p < nFR; p++) s += Q[p * ld + j] * a[p];
@@ -1673,12 +1445,10 @@ struct QPT {
         double *Q = V_(Q), *RT = V_(RT);
         const double *t2 = V_(t2), *t3 = V_(t3), *w = V_(w);
         double r = rotation_chain(nZ);
-#ifndef QP_EXACT
         if constexpr (TEAM > 32) {
             rot_rows_auto(sA.oQ, nFR, nZ, sA.ot2, sA.ot3);
             if (carry_R) update_R_after_add(nZ);  // before the new row of T below: with nFR == cap it lands on row nZ-1 of R
         } else
-#endif
         {
         QP_U1 for (int p = lane; p < nFR; p += TEAM) {
             double* q = Q + p * ld;
@@ -1756,11 +1526,9 @@ struct QPT {
                 T_(ii, cL) = (ii == i) ? 0.0 : cs * ta - sn * tb;
                 T_(ii, cL + 1) = sn * ta + cs * tb;
             }
-#ifndef QP_EXACT
             if constexpr (TEAM > 32) {  // Q is rotated afterwards, all rotations in one coalesced pass (rot_rows, right to left)
                 if (lane == 0) { V_(t2)[i - k - 1] = cs; V_(t3)[i - k - 1] = -sn; }
             } else
-#endif
             {
             QP_U1 for (int p = lane; p < nFR; p += TEAM) {
                 double qa = Q[p * ld + cL], qb = Q[p * ld + cL + 1];
@@ -1771,9 +1539,7 @@ struct QPT {
             SYNC();
         }
         }
-#ifndef QP_EXACT
         if constexpr (TEAM > 32) rot_rows_auto(sA.oQ, nFR, nAC - k, sA.ot2, sA.ot3, nFR - 1 - k, -1);
-#endif
         // shift rows k+1.. up by one (row i -> i-1): every thread moves its own columns, so no barrier between the rows
         QP_U1 for (int j = lane; j < nFR; j += TEAM)
             QP_U1 for (int i = k + 1; i < nAC; i++) T_(i - 1, j) = T_(i, j);
@@ -1791,7 +1557,6 @@ struct QPT {
         const double* Q = V_(Q);
         QP_U1 for (int j = lane; j < nFR; j += TEAM) w[j] = Q[p * ld + j];
         SYNC();
-#ifndef QP_EXACT
         if constexpr (TEAM > 32) {
             double z2p = 0.0;
             for (int j = lane; j < nZ; j += TEAM) z2p += w[j] * w[j];
@@ -1799,7 +1564,6 @@ struct QPT {
             SYNC();
             return z2s;
         }
-#endif
         double z2 = 0.0;
         DOT_UNROLL for (int j = 0; j < nZ; j++) z2 += w[j] * w[j];
         SYNC();
@@ -1813,12 +1577,10 @@ struct QPT {
         short *FR = FR_, *posFR = posFR_;
         const int p = posFR[v];
         rotation_chain(nFR);
-#ifndef QP_EXACT
         if constexpr (TEAM > 32) {
             rot_rows_auto(sA.oQ, nFR, nFR, sA.ot2, sA.ot3);
             if (carry_R) update_R_after_add(nZ);  // the first nZ-1 rotations of the chain act inside the null space
         } else
-#endif
         {
         QP_U1 for (int pp = lane; pp < nFR; pp += TEAM) {
             double* q = Q + pp * ld;
@@ -1888,11 +1650,9 @@ struct QPT {
                 T_(ii, cL) = (ii == i) ? 0.0 : cs * ta - sn * tb;
                 T_(ii, cL + 1) = sn * ta + cs * tb;
             }
-#ifndef QP_EXACT
             if constexpr (TEAM > 32) {
                 if (lane == 0) { V_(t2)[i] = cs; V_(t3)[i] = -sn; }
             } else
-#endif
             {
             QP_U1 for (int p = lane; p < nFR; p += TEAM) {
                 double qa = Q[p * ld + cL], qb = Q[p * ld + cL + 1];
@@ -1902,9 +1662,7 @@ struct QPT {
             }
             SYNC();
         }
-#ifndef QP_EXACT
         if constexpr (TEAM > 32) rot_rows_auto(sA.oQ, nFR, nAC + 1, sA.ot2, sA.ot3, nFR - 1, -1);
-#endif
         return 0;
     }
 
@@ -1914,9 +1672,7 @@ struct QPT {
         QP_CTX
         const int nFR = hdr[0], nAC = hdr[1];
         const double* RT = V_(RT);
-#ifndef QP_EXACT
         if constexpr (TEAM > 32) { solve_T_blocked(b, v); return; }
-#endif
         if (TEAM <= 32 && nAC <= TEAM) {
             // whole right-hand side in registers (lane k holds b_k and its pivot): the substitution chain is one shuffle and
             // the three operations of quot() per unknown, no barrier and no shared-memory round trip.  Same operations on
@@ -1951,9 +1707,7 @@ struct QPT {
         QP_CTX
         const int nFR = hdr[0], nAC = hdr[1];
         const double* RT = V_(RT);
-#ifndef QP_EXACT
         if constexpr (TEAM > 32) { solve_Tt_blocked(r, u); return; }
-#endif
         if (TEAM <= 32 && nAC <= TEAM) {  // register form, see solve_T
             const bool act = lane < nAC;
             double rk = act ? r[nFR - 1 - lane] : 0.0;
@@ -1998,10 +1752,8 @@ struct QPT {
             QP_U1 for (int i = lane; i < nAC; i += TEAM) t3[i] = dbAC[i] - A_row(pat, Av, dx, AC[i]);
             SYNC();
             solve_T(t3, yv);
-#ifndef QP_EXACT
             if constexpr (TEAM > 32) row_sums_auto(sA.oQ, nFR, nZ, nFR, sA.oyv, sA.odx, true, false);
             else
-#endif
             {
             QP_U1 for (int p = lane; p < nFR; p += TEAM) {
                 double s = 0.0;
@@ -2013,13 +1765,11 @@ struct QPT {
         }
         if (nZ > 0) {
             mulH(dx, t1);
-#ifndef QP_EXACT
             if constexpr (TEAM > 32) {
                 for (int p = lane; p < nFR; p += TEAM) { const int v = FR[p]; yv[p] = t1[v] + dgvec[v]; }  // yv is dead here
                 SYNC();
                 col_sums_auto(sA.oQ, nFR, 0, nZ, sA.oyv, sA.ozv, true);
             } else
-#endif
             {
             double* rinv = V_(dy);  // pivot reciprocals of the substitutions below (dy is dead here, rewritten below)
             QP_U1 for (int j = lane; j < nZ; j += TEAM) {
@@ -2054,10 +1804,8 @@ struct QPT {
                 }
                 PROF2_ADD(PR_RSOLVE);
             }
-#ifndef QP_EXACT
             if constexpr (TEAM > 32) row_sums_auto(sA.oQ, nFR, 0, nZ, sA.ozv, sA.odx, true, true);
             else
-#endif
             {
             QP_U1 for (int p = lane; p < nFR; p += TEAM) {
                 double s = 0.0;
@@ -2071,13 +1819,11 @@ struct QPT {
         QP_U1 for (int i = lane; i < nT; i += TEAM) dy[i] = 0.0;
         SYNC();
         if (nAC > 0) {
-#ifndef QP_EXACT
             if constexpr (TEAM > 32) {
                 for (int p = lane; p < nFR; p += TEAM) zv[p] = t1[FR[p]];  // zv is dead here
                 SYNC();
                 col_sums_auto(sA.oQ, nFR, nZ, nFR, sA.ozv, sA.oyv, false);
             } else
-#endif
             {
             QP_U1 for (int j = nZ + lane; j < nFR; j += TEAM) {
                 double s = 0.0;
@@ -2374,9 +2120,7 @@ struct QPT {
                 // one-QP-per-cluster kernel: R is carried through the addition (update_R_after_add) unless an exchange step left
                 // it one column short or REFAC_EVERY updates have accumulated
                 bool carry = false;
-#ifndef QP_EXACT
                 if constexpr (TEAM > 32) carry = !sA.is_lp && carried < REFAC_EVERY && hdr[0] - hdr[1] <= UPDATE_MAX_NZ && !(sA.flags & FLAG_NO_CARRY);
-#endif
                 if (bc_isbound) {
                     double z2 = bound_w(bc_idx);
                     PROF_ADD(PR_WVEC);
@@ -2713,7 +2457,6 @@ template <int TEAM> static __device__ __forceinline__ void qp_solve_one(const QP
         __syncwarp(team_mask<TEAM>());  // every lane has read the state
         if (lane == 0 && !A.rescue) qp_instance_store(A.inst_state + 8 * (size_t)b, mode, oms, nms);
     }
-    if (mode == MODE_REINIT && (A.flags & FLAG_FLIP_AS_HOTSTART)) mode = MODE_HOT_VARIED;
     int status = 0;
     if (mode != MODE_COLD) {
         // restore the pre-solve image: everything but the factors verbatim, then Q (nFR x nFR), R (nZ x nZ), T (nAC x nFR)
@@ -2805,10 +2548,8 @@ __global__ void __launch_bounds__(CTA_THREADS, 1) qp_solve_large_kernel(const __
     typedef QPT<CTA_THREADS> S;
     const int tid = threadIdx.x;
     unsigned cs = 1, rank = 0;
-#ifndef QP_EXACT
     asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(cs));
     asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
-#endif
     const int b = blockIdx.x / cs;  // the CTAs of a cluster share one QP: rank 0 solves, the others help with refactorisations
     {
         const int* src = reinterpret_cast<const int*>(&A);
@@ -2828,9 +2569,7 @@ __global__ void __launch_bounds__(CTA_THREADS, 1) qp_solve_large_kernel(const __
     const int nV = A.nV, nC = A.nC;
     double* slice = A.gwork + (size_t)b * A.slice_doubles;
     int* hdr = reinterpret_cast<int*>(slice);
-#ifndef QP_EXACT
     if (rank != 0) { S::helper_loop((int)rank, (int)cs); return; }
-#endif
 
     int mode = A.mode;
     if (A.inst_state) {
@@ -2882,11 +2621,9 @@ __global__ void __launch_bounds__(CTA_THREADS, 1) qp_solve_large_kernel(const __
     PROF_ADD(PR_TOTAL);
     S::epilogue(b, status, total_iters);
     PROF_ADD(PR_EPILOGUE);
-#ifndef QP_EXACT
     if (tid == 0) hdr[4] = S::OP_EXIT;
     __syncthreads();
     S::large_sync();
-#endif
 }
 
 #endif  // __CUDACC__

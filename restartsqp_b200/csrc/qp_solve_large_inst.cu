@@ -1,19 +1,13 @@
-// qp_solve_large_inst.cu -- instantiation of qp_solve_large_kernel<QP_CTA>: one QP per CTA (or per thread-block cluster), the
+// qp_solve_large_inst.cu -- instantiation of qp_solve_large_kernel<CTA_THREADS>: one QP per CTA (or per thread-block cluster), the
 // slice (vectors and the nV x nV factors) in global memory.  Used when a QP does not fit the shared-memory resident warp kernel.
 #include "qp_kernel.cuh"
 
-#include <cstdlib>
-
-#ifndef QP_CTA
-#define QP_CTA 512
-#endif
-
 namespace sqpb200 {
+constexpr int CTA_THREADS = 512;  // threads per CTA: the DMMA tile mapping (QPT::mma_tile) assumes 16 warps
+
 // CTAs per QP: the largest power of two <= 16 that keeps batch * cluster <= SM count, so that a batch smaller than the GPU still
 // fills it (16 is a non-portable cluster size: opt-in attribute, and a fall-back to 8 if the launch is refused).
-// SQPB200_CLUSTER overrides (1, 2, 4, 8, 16).
 static int cluster_for_batch(int batch, int nV) {
-    if (const char* e = getenv("SQPB200_CLUSTER")) { int v = atoi(e); if (v >= 1 && v <= 16 && (v & (v - 1)) == 0) return v; }
     int dev = 0, sms = 148;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     // Every shared primitive costs two cluster barriers, and since R is carried through additions the refactorisation (the
@@ -27,44 +21,31 @@ static int cluster_for_batch(int batch, int nV) {
 }
 
 cudaError_t launch_qp_solve_large(const QPKernelArgs& a, cudaStream_t stream) {
-#ifdef QP_EXACT
-    qp_solve_large_kernel<QP_CTA><<<a.batch, QP_CTA, 0, stream>>>(a);
-    return cudaGetLastError();
-#else
     int cs = cluster_for_batch(a.batch, a.nV);
-    const size_t smem = (size_t)QPT<QP_CTA>::LS_TOTAL * sizeof(double);
-    cudaError_t e = cudaFuncSetAttribute(qp_solve_large_kernel<QP_CTA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const size_t smem = (size_t)QPT<CTA_THREADS>::LS_TOTAL * sizeof(double);
+    cudaError_t e = cudaFuncSetAttribute(qp_solve_large_kernel<CTA_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     if (cs > 8) {
-        e = cudaFuncSetAttribute(qp_solve_large_kernel<QP_CTA>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+        e = cudaFuncSetAttribute(qp_solve_large_kernel<CTA_THREADS>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
         if (e != cudaSuccess) return e;
     }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)a.batch * cs);
-    cfg.blockDim = dim3(QP_CTA);
+    cfg.blockDim = dim3(CTA_THREADS);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = cs; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    e = cudaLaunchKernelEx(&cfg, qp_solve_large_kernel<QP_CTA>, a);
+    e = cudaLaunchKernelEx(&cfg, qp_solve_large_kernel<CTA_THREADS>, a);
     if (e != cudaSuccess && cs > 8) {  // non-portable size refused on this device / partition: portable maximum
         (void)cudaGetLastError();
         cs = 8;
         cfg.gridDim = dim3((unsigned)a.batch * cs);
         attr[0].val.clusterDim.x = cs;
-        e = cudaLaunchKernelEx(&cfg, qp_solve_large_kernel<QP_CTA>, a);
+        e = cudaLaunchKernelEx(&cfg, qp_solve_large_kernel<CTA_THREADS>, a);
     }
     return e;
-#endif
-}
-int qp_solve_large_threads() { return QP_CTA; }
-int qp_solve_large_cluster(int batch, int nV) {
-#ifdef QP_EXACT
-    (void)batch; (void)nV; return 1;
-#else
-    return cluster_for_batch(batch, nV);
-#endif
 }
 }  // namespace sqpb200

@@ -316,7 +316,7 @@ def test_factor_capacity_rescue_path(gpu_lib, cap):
 def test_dumped_qp_on_cta_per_qp_kernel(gpu_lib, name):
     """The one-QP-per-CTA kernel (slice in global memory) runs the same active-set code with the refactorisation on the
     FP64 tensor cores (DMMA accumulates in a different order than the oracle's scalar sums, and the factor is updated rather
-    than recomputed after most additions; -DQP_EXACT builds the bit-exact scalar variant).  Its gate is north_star's: same status, and where the oracle solves the QP the same objective to 1e-8 and
+    than recomputed after most additions).  Its gate is north_star's: same status, and where the oracle solves the QP the same objective to 1e-8 and
     a KKT point by the reference's own test.  On the rho = 1e8 scaled dump (hs104) the homotopy path is rounding-sensitive,
     so iteration counts may differ while the solution does not; the well-scaled hs116 must keep the oracle's working set."""
     q = [f for f in FIX if f["name"] == name][0]
@@ -454,7 +454,7 @@ def test_hotstart_state_is_bitwise_the_oracles(gpu_lib, team):
             st = solvers[b].hotstart(g[b], lb[b], ub[b], lbA[b], ubA[b])
             xo, yo, _, ito = solvers[b].solution()
             assert st == int(s.get_status()[b])
-            if team == 1024:  # CTA kernel: DMMA sums -> north_star's 1e-8 gate (bit-exact only in a -DQP_EXACT build)
+            if team == 1024:  # CTA kernel: DMMA sums -> north_star's 1e-8 gate
                 assert relerr(x[b], xo) <= RTOL and relerr(np.concatenate([yb[b], yc[b]]), yo) <= 10 * RTOL, (rnd, b)
             else:
                 assert ito == int(it[b])

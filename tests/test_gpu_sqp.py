@@ -278,27 +278,6 @@ def test_device_loop_qp_unchanged_guard(gpu_lib):
     dev.close()
 
 
-@pytest.mark.parametrize("name,soc", [("hs071", False), ("hs100", False), ("hs043", True), ("hs116", False)])
-def test_cxx_sequenced_loop_equals_python_sequenced_loop(gpu_lib, name, soc):
-    """sqpb200_sqp_optimize (the whole of Algorithm::Optimize behind one C call) against the same launch sequence issued from
-    Python (DeviceBatchedSQP.Optimize(host_sequenced=True)): identical results, bit for bit."""
-    import os
-    from restartsqp_b200.nl_reader import AmplNLP, DeviceNLP
-    from restartsqp_b200.sqp_device import DeviceBatchedSQP
-    from test_hs_suite import HS_DIR, perturbed_starts
-    dev = DeviceNLP(AmplNLP(os.path.join(HS_DIR, name + ".nl")))
-    X = perturbed_starts(dev.host, 128, 7)
-    opt = lambda: r.Options(iter_max=120, second_order_correction=soc)
-    a1 = DeviceBatchedSQP(dev, x0=X, options=opt())
-    r1 = a1.Optimize()
-    a2 = DeviceBatchedSQP(dev, x0=X, options=opt())
-    r2 = a2.Optimize(host_sequenced=True)
-    assert (r1.exitflag == r2.exitflag).all() and (r1.iters == r2.iters).all() and (r1.qp_iter == r2.qp_iter).all()
-    assert np.array_equal(r1.x, r2.x, equal_nan=True) and np.array_equal(r1.rho, r2.rho) and np.array_equal(r1.delta, r2.delta)
-    assert a1.launches > 0
-    a1.close(); a2.close(); dev.close()
-
-
 def test_reset_serves_batch_after_batch(gpu_lib):
     """DeviceBatchedSQP.reset(x0): the same object (handles, buffers, compiled NLP) re-initialised for a new batch gives bit for bit
     what a freshly constructed object gives, with and without per-instance backend state machines."""

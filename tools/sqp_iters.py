@@ -1,5 +1,5 @@
 """One HS problem x B perturbed starts through the device-resident SQP loop on one reused object: time per batch, SQP / QP iteration
-statistics (mean, max) and launch count.  SQPB200_FLIP_AS_HOTSTART=1 switches the matrix-status flip back to round 1's hot start."""
+statistics (mean, max) and launch count."""
 import sys, os, time, numpy as np
 R = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path.insert(0, R); sys.path.insert(0, R + "/tests")
 from restartsqp_b200.nl_reader import AmplNLP, DeviceNLP
