@@ -332,6 +332,26 @@ typedef struct {
 int sqpb200_sqp_optimize_stream(sqpb200_sqp_state* st, sqpb200_handle qp, sqpb200_handle lp, sqpb200_nlp nlp,
                                 int second_order_correction, int refresh_ubA, int* first, double* f_tmp, double* c_tmp,
                                 sqpb200_sqp_stream* sd, long long* launches, void* stream);
+/* Asynchronous solves: the loop of sqpb200_sqp_optimize recorded once as a CUDA graph whose branches (does any instance remain
+ * active, need the penalty update, continue the penalty loop, enter the second-order correction, is a refill round due) are
+ * conditional nodes set on the device from the counters.  A launch queues the whole solve on `stream` and returns: nothing is read
+ * back and nothing is waited for, so solves of several states can run concurrently on several streams from one host thread.
+ * Results are bit-identical with the synchronous calls for the same sequence of calls on a state.
+ *
+ * sqpb200_sqp_graph_create: same preconditions and arguments as sqpb200_sqp_optimize (structures set, start evaluated; `stream` is
+ * the stream of both handles), plus per-instance backend state machines (st->qp_inst and st->lp_inst), else SQPB200_ERR_INVALID.
+ * It makes the handles' first-solve allocations and records the loop (synchronising nothing).  `st` is kept by pointer: it and every
+ * array it names must stay valid and unchanged, except clear_flags, until sqpb200_sqp_graph_destroy; the handles' stream too.
+ * sqpb200_sqp_graph_launch: sd == NULL queues one sqpb200_sqp_optimize; sd != NULL one sqpb200_sqp_optimize_stream over the
+ * descriptor (recording its loop again, since the descriptor is part of the graph: the launch then costs a capture and an
+ * instantiation).  *first as in those calls, updated when the launch is queued; sd->rounds and launch counts are not reported.
+ * The results are in place once the stream reaches them (an event recorded after the launch).
+ * sqpb200_sqp_graph_destroy: a graph still running is released when it completes. */
+typedef struct sqpb200_sqp_graph_s* sqpb200_sqp_graph;
+int sqpb200_sqp_graph_create(sqpb200_sqp_state* st, sqpb200_handle qp, sqpb200_handle lp, sqpb200_nlp nlp, int second_order_correction,
+                             int refresh_ubA, double* f_tmp, double* c_tmp, void* stream, sqpb200_sqp_graph* out);
+int sqpb200_sqp_graph_launch(sqpb200_sqp_graph g, int* first, sqpb200_sqp_stream* sd);
+int sqpb200_sqp_graph_destroy(sqpb200_sqp_graph g);
 /* Forget every solve so far: the next solve is an init (cold start) again, as for a freshly constructed backend
  * (firstQPsolved_ = false, matrix status UNDEFINED, Update_* flags cleared; src/qpOASESInterface.cpp:35-50).  Structures and
  * device buffers are kept, so one handle can serve batch after batch. */

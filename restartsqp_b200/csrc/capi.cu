@@ -849,18 +849,39 @@ int sqpb200_device_buffers(sqpb200_handle h, void** out) {
     out[0] = h->dx; out[1] = h->dy; out[2] = h->dobj; out[3] = h->dstatus; out[4] = h->diters; out[5] = h->dkkt;
     return 0;
 }
-static int solve_impl(sqpb200_handle h, int mode_qp, int maxiter, const unsigned char* active_mask, bool mask_on_device, signed char* inst_state) {
+// What the first solve of a handle allocates -- the launch configuration, the hot-start images of the warp kernel, the global-memory
+// slices and pattern of the one-QP-per-cluster kernel -- made without solving.  sqpb200_sqp_graph_create calls it before it records
+// solves into a CUDA graph, where an allocation and the memset that zeroes it must not happen.  (Not part of the public header.)
+int sqpb200_solve_prepare(sqpb200_handle h) {
     if (!h) return SQPB200_ERR_INVALID;
     CK(cudaSetDevice(h->device));
     if (!h->A_set) { h->err = "set_structure_A has not been called"; return SQPB200_ERR_STATE; }
-    bool is_lp = (mode_qp == SQPB200_LP);
-    if (mode_qp != h->qptype) { h->err = "solve mode differs from the handle's QPType (the reference keeps one backend per type)"; return SQPB200_ERR_INVALID; }
-    if (!is_lp && !h->H_set) { h->err = "set_structure_H has not been called"; return SQPB200_ERR_STATE; }
+    if (h->qptype == SQPB200_QP && !h->H_set) { h->err = "set_structure_H has not been called"; return SQPB200_ERR_STATE; }
     int rc = choose_config(h);
     if (rc) return rc;
     if (!h->large && h->opt.keep_state && !h->dstate) {
         if (dev_alloc(h, &h->dstate, (size_t)h->batch * h->cfg_main.state_doubles)) return SQPB200_ERR_CUDA;
     }
+    if (h->large) {
+        QPKernelArgs a;
+        fill_dims(h, a, h->nV);
+        return prepare_large(h, a);
+    }
+    return 0;
+}
+
+static int solve_impl(sqpb200_handle h, int mode_qp, int maxiter, const unsigned char* active_mask, bool mask_on_device, signed char* inst_state) {
+    if (!h) return SQPB200_ERR_INVALID;
+    CK(cudaSetDevice(h->device));
+    bool is_lp = (mode_qp == SQPB200_LP);
+    if (mode_qp != h->qptype) { h->err = "solve mode differs from the handle's QPType (the reference keeps one backend per type)"; return SQPB200_ERR_INVALID; }
+    int rc = sqpb200_solve_prepare(h);
+    if (rc) return rc;
+    // a solve recorded into a CUDA graph (sqpb200_sqp_graph_create) reads nothing back and records no timing events: the capacity
+    // frozen in the graph affects speed, never results (the rescue launch)
+    cudaStreamCaptureStatus capture = cudaStreamCaptureStatusNone;
+    CK(cudaStreamIsCapturing(h->stream, &capture));
+    const bool recording = capture != cudaStreamCaptureStatusNone;
     // init / hotstart decision: src/qpOASESInterface.cpp:141-211 with get_Matrix_change_status :817-833
     int mode = MODE_COLD;
     if (h->first_solved && h->opt.keep_state) {
@@ -899,19 +920,17 @@ static int solve_impl(sqpb200_handle h, int mode_qp, int maxiter, const unsigned
     a.prof = h->dprof;
     a.inst_state = inst_state;  // per-instance init/hotstart decisions (made in the kernel) replace the handle-level `mode`
     if (h->large) {
-        rc = prepare_large(h, a);
-        if (rc) return rc;
         a.gpat = h->dgpat; a.gwork = h->dgwork;
-        CK(cudaEventRecord(h->ev0, h->stream));
+        if (!recording) CK(cudaEventRecord(h->ev0, h->stream));
         cudaError_t el = launch_qp_solve_large(a, h->stream);
         if (el != cudaSuccess) { h->err = std::string("qp_solve_large_kernel launch: ") + cudaGetErrorString(el); return SQPB200_ERR_CUDA; }
-        CK(cudaEventRecord(h->ev1, h->stream));
+        if (!recording) CK(cudaEventRecord(h->ev1, h->stream));
         h->launches++;
         h->upd_A = h->upd_H = h->upd_g = h->upd_bounds = false;
         h->first_solved = true;
         return 0;
     }
-    CK(cudaEventRecord(h->ev0, h->stream));
+    if (!recording) CK(cudaEventRecord(h->ev0, h->stream));
     if (h->cfg_main.cap < h->nV) CK(cudaMemsetAsync(h->dncap, 0, sizeof(int), h->stream));
     cudaError_t e = launch_cfg(h->cfg_main, a, h->stream);
     if (e != cudaSuccess) { h->err = std::string("qp_solve_kernel launch: ") + cudaGetErrorString(e); return SQPB200_ERR_CUDA; }
@@ -927,9 +946,9 @@ static int solve_impl(sqpb200_handle h, int mode_qp, int maxiter, const unsigned
             h->launches++;
         }
     }
-    CK(cudaEventRecord(h->ev1, h->stream));
+    if (!recording) CK(cudaEventRecord(h->ev1, h->stream));
     h->launches++;
-    if (h->opt.factor_cap == 0) {  // learn the capacity for later solves (asynchronous: never waited for)
+    if (h->opt.factor_cap == 0 && !recording) {  // learn the capacity for later solves (asynchronous: never waited for)
         CK(cudaMemcpyAsync(h->maxfr_host, h->dmaxfr, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
         CK(cudaEventRecord(h->ev_maxfr, h->stream));
         h->maxfr_pending = true;

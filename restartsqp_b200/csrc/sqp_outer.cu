@@ -26,6 +26,10 @@
 
 #include <cuda_runtime.h>
 
+#include <vector>
+
+int sqpb200_solve_prepare(sqpb200_handle h);  // capi.cu: a handle's first-solve allocations, made before a solve is recorded
+
 namespace {
 
 enum { EX_OPTIMAL = 0, EX_EXCEED_MAX_ITER = 2, EX_TRUST_REGION_TOO_SMALL = 4, EX_UNKNOWN = -99,
@@ -43,6 +47,21 @@ struct StreamArgs {
     sqpb200_sqp_stream d;
     double *f_tmp, *c_tmp;
 };
+
+// the branch points of the loop: the host decides them from the counters it reads back (synchronous solves), a CUDA graph of the loop
+// from the device counters (sqp_branch_kernel)
+enum { BR_ACTIVE, BR_PENALTY, BR_PEN_GO, BR_SOC, BR_STREAM_LOOP, BR_REFILL };
+__host__ __device__ __forceinline__ bool branch_taken(int br, const int* cnt, unsigned long long head, long long N, int refill_min) {
+    const bool queued = head < (unsigned long long)N;
+    switch (br) {
+    case BR_ACTIVE: return cnt[0] > 0;                 // instances active in PH_FLAGS: the outer loop goes on
+    case BR_PENALTY: return cnt[2] > 0;                // PH_AFTER_QP: instances that need the penalty update
+    case BR_PEN_GO: return cnt[3] > 0;                 // PH_PEN_CHECK: the penalty loop goes on
+    case BR_SOC: return cnt[5] > 0;                    // PH_SOC_PREP: rejected steps enter the second-order correction
+    case BR_STREAM_LOOP: return cnt[0] > 0 || queued;  // streamed: active slots or starting points left
+    default: return queued && (cnt[CNT_STOPPED] >= refill_min || cnt[0] == 0);  // BR_REFILL: a refill round is due
+    }
+}
 
 __device__ __forceinline__ double cal_infea(const sqpb200_sqp_state& S, const double* c, int b) {
     double s = 0.0;
@@ -431,6 +450,12 @@ __global__ void sqp_phase_kernel(const __grid_constant__ sqpb200_sqp_state S, in
     }
 }
 
+// sets the condition of a conditional node of a recorded loop: one thread, after the phase that counted
+__global__ void sqp_branch_kernel(cudaGraphConditionalHandle hc, const int* counters, int br, const unsigned long long* head, long long N,
+                                  int refill_min) {
+    cudaGraphSetConditional(hc, branch_taken(br, counters, head ? *head : 0ULL, N, refill_min) ? 1u : 0u);
+}
+
 }  // namespace
 
 static int launch_phase(const sqpb200_sqp_state* st, int phase, const StreamArgs& X, int* counters_host, cudaStream_t stream) {
@@ -474,10 +499,54 @@ struct OuterLoop {
     long long launches;
     int rc;
     StreamArgs X{};  // the streamed phases' arguments (zero outside a streamed solve) and the scratch buffers f_tmp / c_tmp
+    bool recording = false;  // the launches are being recorded into a CUDA graph (sqpb200_sqp_graph_create / _launch)
     bool ph(int phase, bool read = false) {
-        rc = launch_phase(S, phase, X, read ? cnt : nullptr, stream);
+        rc = launch_phase(S, phase, X, read && !recording ? cnt : nullptr, stream);
         launches++;
         return rc == 0;
+    }
+    bool cuda(cudaError_t e) {
+        rc = e == cudaSuccess ? 0 : SQPB200_ERR_CUDA;
+        return rc == 0;
+    }
+    bool set_branch(cudaGraphConditionalHandle hc, int br) {
+        sqp_branch_kernel<<<1, 1, 0, stream>>>(hc, S->counters, br, X.d.head, X.d.N, X.d.refill_min);
+        return cuda(cudaGetLastError());
+    }
+    // A branch point: `body` runs once (loop = false) or as long as the condition holds (loop = true; the body's last phase counts
+    // again).  Synchronous solves test the counters read back last.  While the loop is recorded, the branch becomes a conditional
+    // node (IF / WHILE) set by sqp_branch_kernel: the capture of the enclosing graph ends in front of the node, the body is recorded
+    // into the node's body graph on the same stream, and the enclosing capture resumes behind the node.
+    template <class F>
+    bool branch(int br, bool loop, F body) {
+        if (!recording) {
+            while (branch_taken(br, cnt, 0, 0, 0)) {
+                if (!body()) return false;
+                if (!loop) break;
+            }
+            return true;
+        }
+        cudaStreamCaptureStatus cs;
+        cudaGraph_t g, t;
+        const cudaGraphNode_t* d = nullptr;
+        size_t nd = 0;
+        cudaGraphConditionalHandle hc;
+        if (!cuda(cudaStreamGetCaptureInfo(stream, &cs, nullptr, &g)) || !cuda(cudaGraphConditionalHandleCreate(&hc, g, 0, 0)) ||
+            !set_branch(hc, br) || !cuda(cudaStreamGetCaptureInfo(stream, &cs, nullptr, &g, &d, &nd)))
+            return false;
+        std::vector<cudaGraphNode_t> deps(d, d + nd);
+        if (!cuda(cudaStreamEndCapture(stream, &t))) return false;
+        cudaGraphNodeParams p = {};
+        p.type = cudaGraphNodeTypeConditional;
+        p.conditional.handle = hc;
+        p.conditional.type = loop ? cudaGraphCondTypeWhile : cudaGraphCondTypeIf;
+        p.conditional.size = 1;
+        cudaGraphNode_t node;
+        if (!cuda(cudaGraphAddNode(&node, g, deps.data(), deps.size(), &p)) ||
+            !cuda(cudaStreamBeginCaptureToGraph(stream, p.conditional.phGraph_out[0], nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed)))
+            return false;
+        if (!body() || (loop && !set_branch(hc, br)) || !cuda(cudaStreamEndCapture(stream, &t))) return false;
+        return cuda(cudaStreamBeginCaptureToGraph(stream, g, &node, nullptr, 1, cudaStreamCaptureModeRelaxed));
     }
     bool solve(sqpb200_handle h, int type, const unsigned char* mask, signed char* inst) {
         rc = inst ? sqpb200_solve_per_instance(h, type, 0, mask, inst) : sqpb200_solve_device_mask(h, type, 0, mask);
@@ -527,29 +596,32 @@ struct OuterLoop {
     // update_penalty_parameter, src/Algorithm.cpp:886-1028
     bool penalty() {
         if (!bounds(lp, 0, S->x_k, S->c_k) || !grad(lp, nullptr, S->rho) || !valsA(lp)) return false;  // setupLP :700-704
-        if (!solve(lp, SQPB200_LP, S->need, S->lp_inst) || !ph(SQPB200_PH_LP_AFTER)) return false;
-        for (;;) {
-            if (!ph(SQPB200_PH_PEN_CHECK, true)) return false;
-            if (cnt[3] == 0) break;
-            if (!grad(qp, nullptr, S->rho_trial) || !solve(qp, SQPB200_QP, S->go, S->qp_inst) || !ph(SQPB200_PH_PEN_AFTER)) return false;
-        }
-        return ph(SQPB200_PH_PEN_FINAL);
+        if (!solve(lp, SQPB200_LP, S->need, S->lp_inst) || !ph(SQPB200_PH_LP_AFTER) || !ph(SQPB200_PH_PEN_CHECK, true)) return false;
+        return branch(BR_PEN_GO, true, [&] {
+            return grad(qp, nullptr, S->rho_trial) && solve(qp, SQPB200_QP, S->go, S->qp_inst) && ph(SQPB200_PH_PEN_AFTER) &&
+                   ph(SQPB200_PH_PEN_CHECK, true);
+        }) && ph(SQPB200_PH_PEN_FINAL);
     }
     // second_order_correction, src/Algorithm.cpp:1140-1211
     bool soc() {
         if (!ph(SQPB200_PH_SOC_PREP, true)) return false;
-        if (cnt[5] == 0) return true;
-        if (!grad(qp, S->soc_g, nullptr) || !bounds(qp, bounds_update_mode, S->soc_x, S->soc_c)) return false;
-        if (!solve(qp, SQPB200_QP, S->rej, S->qp_inst) || !ph(SQPB200_PH_SOC_AFTER)) return false;
-        rc = sqpb200_nlp_eval(nlp, 0, S->B, S->x_trial, nullptr, S->f_trial, S->c_trial, nullptr, nullptr, nullptr, SQPB200_LOC_DEVICE, stream);
-        if (rc) return false;
-        launches++;
-        if (!ph(SQPB200_PH_SOC_RATIO)) return false;
-        return grad(qp, S->grad, nullptr) && bounds(qp, bounds_update_mode, S->x_k, S->c_k);
+        return branch(BR_SOC, false, [&] {
+            if (!grad(qp, S->soc_g, nullptr) || !bounds(qp, bounds_update_mode, S->soc_x, S->soc_c)) return false;
+            if (!solve(qp, SQPB200_QP, S->rej, S->qp_inst) || !ph(SQPB200_PH_SOC_AFTER)) return false;
+            rc = sqpb200_nlp_eval(nlp, 0, S->B, S->x_trial, nullptr, S->f_trial, S->c_trial, nullptr, nullptr, nullptr, SQPB200_LOC_DEVICE, stream);
+            if (rc) return false;
+            launches++;
+            if (!ph(SQPB200_PH_SOC_RATIO)) return false;
+            return grad(qp, S->grad, nullptr) && bounds(qp, bounds_update_mode, S->x_k, S->c_k);
+        });
+    }
+    // the start of an outer iteration of a per-instance-mode solve: flags, QP data, QP solve, its acceptance
+    bool qp_step(int* first) {
+        return ph(SQPB200_PH_FLAGS) && setupQP(first) && solve(qp, SQPB200_QP, S->active, S->qp_inst) && ph(SQPB200_PH_AFTER_QP);
     }
     // one outer iteration after the QP solve, for the instances that were active in PH_FLAGS
     bool rest_of_iteration(int second_order_correction) {
-        if (cnt[2] > 0 && !penalty()) return false;
+        if (!branch(BR_PENALTY, false, [&] { return penalty(); })) return false;
         if (!ph(SQPB200_PH_TRIAL)) return false;
         // get_trial_point_info :414-429
         rc = sqpb200_nlp_eval(nlp, 0, S->B, S->x_trial, nullptr, S->f_trial, S->c_trial, nullptr, nullptr, nullptr, SQPB200_LOC_DEVICE, stream);
@@ -600,6 +672,12 @@ int sqpb200_sqp_optimize(sqpb200_sqp_state* st, sqpb200_handle qp, sqpb200_handl
     return 0;
 }
 
+static bool stream_desc_ok(const sqpb200_sqp_state* st, const sqpb200_sqp_stream* sd) {
+    if (sd->N < 0 || sd->refill_min < 1 || !sd->slot_id || !sd->head || !sd->refill) return false;
+    return sd->N == 0 || (sd->x0_all && sd->x && sd->obj && sd->kkt_err && sd->rho && sd->delta && sd->exitflag && sd->iter && sd->qp_iter &&
+                          (st->m == 0 || sd->lam_start));
+}
+
 // The same loop over a queue of N starting points.  A slot whose instance has stopped keeps its state (nothing changes a stopped
 // instance's results) until a refill round retires it to out[instance] and hands it the next starting point; the refilled slot
 // then runs initialization() and starts cold in both backends (PH_INIT_REFILLED), so its trajectory is the one it has in any batch.
@@ -611,11 +689,7 @@ int sqpb200_sqp_optimize_stream(sqpb200_sqp_state* st, sqpb200_handle qp, sqpb20
                                 sqpb200_sqp_stream* sd, long long* launches, void* stream) {
     if (!st || !qp || !lp || !nlp || !first || !sd || st->B <= 0) return SQPB200_ERR_INVALID;
     // handle-level init / hotstart decisions: a refilled slot would inherit its handle's hot start
-    if (!st->qp_inst || !st->lp_inst) return SQPB200_ERR_INVALID;
-    if (sd->N < 0 || sd->refill_min < 1 || !sd->slot_id || !sd->head || !sd->refill) return SQPB200_ERR_INVALID;
-    if (sd->N > 0 && (!sd->x0_all || !sd->x || !sd->obj || !sd->kkt_err || !sd->rho || !sd->delta || !sd->exitflag || !sd->iter ||
-                      !sd->qp_iter || (st->m > 0 && !sd->lam_start)))
-        return SQPB200_ERR_INVALID;
+    if (!st->qp_inst || !st->lp_inst || !stream_desc_ok(st, sd)) return SQPB200_ERR_INVALID;
     cudaStream_t cs = (cudaStream_t)stream;
     OuterLoop L{st, qp, lp, nlp, cs, refresh_ubA ? 3 : 1, {0, 0, 0, 0, 0, 0, 0, 0}, 0, 0};
     L.X.d = *sd;
@@ -627,8 +701,7 @@ int sqpb200_sqp_optimize_stream(sqpb200_sqp_state* st, sqpb200_handle qp, sqpb20
     if (!L.refill()) return L.rc;
     unsigned long long head = 0;
     for (;;) {
-        if (!L.ph(SQPB200_PH_FLAGS) || !L.setupQP(first) || !L.solve(qp, SQPB200_QP, st->active, st->qp_inst) || !L.ph(SQPB200_PH_AFTER_QP))
-            return L.rc;
+        if (!L.qp_step(first)) return L.rc;
         // the loop's one read-back per outer iteration: active and stopped slots (PH_FLAGS), penalty updates (PH_AFTER_QP), queue head
         if (cudaMemcpyAsync(L.cnt, st->counters, 8 * sizeof(int), cudaMemcpyDeviceToHost, cs) != cudaSuccess ||
             cudaMemcpyAsync(&head, sd->head, sizeof head, cudaMemcpyDeviceToHost, cs) != cudaSuccess || cudaStreamSynchronize(cs) != cudaSuccess)
@@ -641,5 +714,117 @@ int sqpb200_sqp_optimize_stream(sqpb200_sqp_state* st, sqpb200_handle qp, sqpb20
     if (!L.ph(PH_RETIRE)) return L.rc;
     sd->rounds = L.X.d.rounds;
     if (launches) *launches = L.launches;
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// The same loops recorded once as CUDA graphs, every host branch a conditional node (OuterLoop::branch), so that a solve is queued on
+// the stream and returns without waiting.  What a recorded launch freezes and how the calls keep results bit-identical:
+//   - the state goes in by value: the loop is recorded with clear_flags = 1 and with setupQP's update_bounds (first = 0), so the
+//     first iteration -- PH_FLAGS with the caller's clear_flags, setupQP(first), the QP solve, PH_AFTER_QP -- is queued as ordinary
+//     launches in front of the graph, and PH_FINAL (PH_RETIRE) behind it;
+//   - the streamed descriptor goes in by value too: a streamed launch records its loop again (a graph per call);
+//   - a recorded solve neither allocates nor reads back (sqpb200_solve_prepare before, solve_impl skips the capacity read-back).
+// The loop is recorded on a private stream, both handles moved there meanwhile: the caller's stream may be the legacy default
+// stream, which cannot be captured.
+// ---------------------------------------------------------------------------------------------------------------------
+struct sqpb200_sqp_graph_s {
+    sqpb200_sqp_state* st;
+    sqpb200_handle qp, lp;
+    sqpb200_nlp nlp;
+    int second_order_correction, bounds_update_mode;
+    double *f_tmp, *c_tmp;
+    cudaStream_t stream;                      // the caller's: where launches are queued
+    cudaStream_t rec = nullptr;               // where the loops are recorded
+    cudaGraphExec_t optimize = nullptr, streamed = nullptr;
+};
+
+// records fn(L) into *out (replacing what it held)
+template <class F>
+static int record(sqpb200_sqp_graph g, const StreamArgs& X, cudaGraphExec_t* out, F fn) {
+    sqpb200_sqp_state S = *g->st;
+    S.clear_flags = 1;
+    OuterLoop L{&S, g->qp, g->lp, g->nlp, g->rec, g->bounds_update_mode, {0, 0, 0, 0, 0, 0, 0, 0}, 0, 0};
+    L.X = X;
+    L.recording = true;
+    cudaGraph_t top = nullptr;
+    int rc = sqpb200_set_stream(g->qp, g->rec);
+    if (!rc) rc = sqpb200_set_stream(g->lp, g->rec);
+    if (!rc && cudaGraphCreate(&top, 0) != cudaSuccess) rc = SQPB200_ERR_CUDA;
+    if (!rc && cudaStreamBeginCaptureToGraph(g->rec, top, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed) != cudaSuccess) rc = SQPB200_ERR_CUDA;
+    if (!rc && !fn(L)) rc = L.rc ? L.rc : SQPB200_ERR_CUDA;
+    // a failure may leave a capture open, in a body graph
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(g->rec, &cs) == cudaSuccess && cs != cudaStreamCaptureStatusNone) {
+        cudaGraph_t t;
+        if (cudaStreamEndCapture(g->rec, &t) != cudaSuccess && !rc) rc = SQPB200_ERR_CUDA;
+    }
+    const int r1 = sqpb200_set_stream(g->qp, g->stream), r2 = sqpb200_set_stream(g->lp, g->stream);
+    if (!rc) rc = r1 ? r1 : r2;
+    cudaGraphExec_t e = nullptr;
+    if (!rc && cudaGraphInstantiate(&e, top, 0) != cudaSuccess) rc = SQPB200_ERR_CUDA;
+    if (!rc) {
+        if (*out) cudaGraphExecDestroy(*out);  // an exec still running is freed when it completes
+        *out = e;
+    }
+    if (top) cudaGraphDestroy(top);
+    return rc;
+}
+
+int sqpb200_sqp_graph_create(sqpb200_sqp_state* st, sqpb200_handle qp, sqpb200_handle lp, sqpb200_nlp nlp, int second_order_correction,
+                             int refresh_ubA, double* f_tmp, double* c_tmp, void* stream, sqpb200_sqp_graph* out) {
+    if (!out) return SQPB200_ERR_INVALID;
+    *out = nullptr;
+    if (!st || !qp || !lp || !nlp || st->B <= 0 || !st->qp_inst || !st->lp_inst) return SQPB200_ERR_INVALID;
+    int rc = sqpb200_solve_prepare(qp);
+    if (!rc) rc = sqpb200_solve_prepare(lp);
+    if (rc) return rc;
+    sqpb200_sqp_graph g = new sqpb200_sqp_graph_s{st, qp, lp, nlp, second_order_correction, refresh_ubA ? 3 : 1, f_tmp, c_tmp,
+                                                  (cudaStream_t)stream};
+    if (cudaStreamCreateWithFlags(&g->rec, cudaStreamNonBlocking) != cudaSuccess) { delete g; return SQPB200_ERR_CUDA; }
+    StreamArgs X{};
+    X.f_tmp = f_tmp; X.c_tmp = c_tmp;
+    rc = record(g, X, &g->optimize, [&](OuterLoop& L) {
+        int first = 0;
+        return L.branch(BR_ACTIVE, true, [&] { return L.rest_of_iteration(second_order_correction) && L.qp_step(&first); });
+    });
+    if (rc) { sqpb200_sqp_graph_destroy(g); return rc; }
+    *out = g;
+    return 0;
+}
+
+int sqpb200_sqp_graph_launch(sqpb200_sqp_graph g, int* first, sqpb200_sqp_stream* sd) {
+    if (!g || !first) return SQPB200_ERR_INVALID;
+    StreamArgs X{};
+    X.f_tmp = g->f_tmp; X.c_tmp = g->c_tmp;
+    if (sd) {
+        if (!stream_desc_ok(g->st, sd)) return SQPB200_ERR_INVALID;
+        X.d = *sd;
+        const int soc = g->second_order_correction;
+        const int rc = record(g, X, &g->streamed, [&](OuterLoop& L) {
+            int zero = 0;
+            return L.branch(BR_STREAM_LOOP, true, [&] {
+                return L.branch(BR_ACTIVE, false, [&] { return L.rest_of_iteration(soc); }) &&
+                       L.branch(BR_REFILL, false, [&] { return L.ph(PH_RETIRE) && L.refill(); }) && L.qp_step(&zero);
+            });
+        });
+        if (rc) return rc;
+    }
+    OuterLoop L{g->st, g->qp, g->lp, g->nlp, g->stream, g->bounds_update_mode, {0, 0, 0, 0, 0, 0, 0, 0}, 0, 0};
+    L.X = X;
+    if (sd && (cudaMemsetAsync(sd->slot_id, 0xff, (size_t)g->st->B * sizeof(long long), g->stream) != cudaSuccess ||
+               cudaMemsetAsync(sd->head, 0, sizeof(unsigned long long), g->stream) != cudaSuccess))
+        return SQPB200_ERR_CUDA;
+    if ((sd && !L.refill()) || !L.qp_step(first)) return L.rc;
+    if (cudaGraphLaunch(sd ? g->streamed : g->optimize, g->stream) != cudaSuccess) return SQPB200_ERR_CUDA;
+    return L.ph(sd ? PH_RETIRE : SQPB200_PH_FINAL) ? 0 : L.rc;
+}
+
+int sqpb200_sqp_graph_destroy(sqpb200_sqp_graph g) {
+    if (!g) return SQPB200_ERR_INVALID;
+    if (g->optimize) cudaGraphExecDestroy(g->optimize);
+    if (g->streamed) cudaGraphExecDestroy(g->streamed);
+    if (g->rec) cudaStreamDestroy(g->rec);
+    delete g;
     return 0;
 }

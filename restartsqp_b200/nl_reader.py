@@ -902,10 +902,12 @@ class DeviceNLP:
             raise self._capi.SqpB200Error("sqpb200_nlp_eval failed (%d): %s" % (rc, self.L.sqpb200_nlp_last_error().decode()))
         return f, c, g, jv, hv
 
-    def eval_device(self, which, B, x, lam=None, f=None, c=None, grad=None, jac=None, hess=None):
-        """Evaluation with every array already in device memory (CUDA tensors); asynchronous on the default stream."""
+    def eval_device(self, which, B, x, lam=None, f=None, c=None, grad=None, jac=None, hess=None, stream=None):
+        """Evaluation with every array already in device memory (CUDA tensors); asynchronous on `stream` (a torch.cuda.Stream; None:
+        the default stream)."""
         p = lambda t: None if t is None else self._C.c_void_p(t.data_ptr())
-        rc = self.L.sqpb200_nlp_eval(self.h, which, B, p(x), p(lam), p(f), p(c), p(grad), p(jac), p(hess), self._capi.LOC_DEVICE, None)
+        s = None if stream is None else self._C.c_void_p(stream.cuda_stream)
+        rc = self.L.sqpb200_nlp_eval(self.h, which, B, p(x), p(lam), p(f), p(c), p(grad), p(jac), p(hess), self._capi.LOC_DEVICE, s)
         if rc != 0:
             raise self._capi.SqpB200Error("sqpb200_nlp_eval failed (%d): %s" % (rc, self.L.sqpb200_nlp_last_error().decode()))
 

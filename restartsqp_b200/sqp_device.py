@@ -6,6 +6,9 @@ of one CUDA kernel (csrc/sqp_outer.cu, one thread per instance), the NLP is eval
 `DeviceNLP`, QP data is built by the qphandler kernels and the QP/LP solves take their instance mask from device memory.  The
 host sequences launches and reads eight counters per outer iteration.  torch is used for device memory only.
 
+optimize_async / solve_stream_async queue the same solves without any read-back: the loop is recorded once as a CUDA graph whose
+branches are decided on the device (sqpb200_sqp_graph_*), so objects on different streams solve concurrently from one thread.
+
 By default the backend's init / hotstart decision (src/qpOASESInterface.cpp:141-211, 817-833) is made per instance inside the solve
 kernel, so every instance of the batch follows the reference's single-instance semantics: tests/test_gpu_sqp.py compares it bitwise
 with the C oracle of the loop (oracle/oracle_sqp.c), and, with per_instance_modes=False, with BatchedSQP.
@@ -54,16 +57,47 @@ class SqpStream(C.Structure):
 REFILL_MIN_FRACTION = 16
 
 
+class PendingSQP:
+    """A solve queued by optimize_async / solve_stream_async.  Its results are copied on the object's stream into tensors this object
+    owns, so later calls on the object (reset, further solves) do not change them.  `event` is recorded behind the copies."""
+
+    def __init__(self, out, event, keep=None):
+        self._out, self.event, self._keep = out, event, keep
+
+    def done(self):
+        return self.event.query()
+
+    def wait(self):
+        self.event.synchronize()
+        return self
+
+    def result(self):
+        self.wait()
+        h = lambda k: self._out[k].cpu().numpy()
+        return SQPResult(x=h("x"), obj=h("obj"), exitflag=h("exitflag"), iters=h("iter").astype(np.int64), qp_iter=h("qp_iter"),
+                         KKT_error=h("kkt_err"), rho=h("rho"), delta=h("delta"))
+
+
 class DeviceBatchedSQP:
-    def __init__(self, nlp, x0=None, options: Options = None, device=0, per_instance_modes=True):
+    def __init__(self, nlp, x0=None, options: Options = None, device=0, per_instance_modes=True, stream=None):
         """per_instance_modes: the backend's init/hotstart decision is made per instance, as the reference does for its single
-        instance (and as oracle/oracle_sqp.c does); False: per handle, which is what the numpy mirror BatchedSQP does."""
+        instance (and as oracle/oracle_sqp.c does); False: per handle, which is what the numpy mirror BatchedSQP does.
+        stream: a torch.cuda.Stream on which everything this object does runs (both handles, the NLP evaluations, the phases and its
+        torch work); None: the default stream."""
         import torch
         if not hasattr(nlp, "eval_device"):
             raise TypeError("DeviceBatchedSQP needs a DeviceNLP (device-side evaluation)")
         self.torch, self.nlp_, self.L = torch, nlp, capi.lib()
         self.dev = torch.device("cuda", device)
         torch.cuda.set_device(self.dev)
+        self.stream = stream
+        self._sp = None if stream is None else C.c_void_p(stream.cuda_stream)
+        self._graph = None
+        with torch.cuda.stream(stream):
+            self._init(nlp, x0, options, device, per_instance_modes)
+
+    def _init(self, nlp, x0, options, device, per_instance_modes):
+        torch = self.torch
         o = self.options_ = options if options is not None else Options()
         info = self.info = nlp.Get_nlp_info()
         n, m = self.nVar_, self.nCon_ = info.nVar, info.nCon
@@ -73,6 +107,9 @@ class DeviceBatchedSQP:
         zJ, zH = len(nlp.J_row1), len(nlp.H_row1)
         self.myQP_ = QPhandler(info, QPType.QP, o, batch=B, device=device, refresh_ubA=True)  # src/Algorithm.cpp:561-562
         self.myLP_ = QPhandler(info, QPType.LP, o, batch=B, device=device, refresh_ubA=True)
+        if self.stream is not None:
+            for hd in (self.myQP_, self.myLP_):
+                hd.solverInterface_.set_stream(self.stream.cuda_stream)
         f64 = lambda *shape: torch.zeros(shape, dtype=torch.float64, device=self.dev)
         u8 = lambda: torch.zeros(B, dtype=torch.uint8, device=self.dev)
         up = lambda a, dt=torch.float64: torch.as_tensor(np.ascontiguousarray(a), dtype=dt).to(self.dev)
@@ -112,7 +149,7 @@ class DeviceBatchedSQP:
                 T[k] = torch.zeros((B, 8), dtype=torch.int8, device=self.dev)
                 T[k][:, 2:4] = -1  # matrix status undefined (get_Matrix_change_status, src/qpOASESInterface.cpp:817-833)
         # initialization(), src/Algorithm.cpp:438-472: f, c, grad, Jacobian, Hessian at the (shifted) start in one launch
-        nlp.eval_device(1, B, T["x_k"], T["neg_lam"], T["f_k"], T["c_k"], T["grad"], T["jac"], T["hess"])
+        nlp.eval_device(1, B, T["x_k"], T["neg_lam"], T["f_k"], T["c_k"], T["grad"], T["jac"], T["hess"], stream=self.stream)
         S = self.S = SqpState()
         S.B, S.n, S.m, S.zJ, S.zH = B, n, m, zJ, zH
         S.iter_max, S.penalty_update, S.penalty_iter_max, S.clear_flags = o.iter_max, int(o.penalty_update), o.penalty_iter_max, 0
@@ -139,15 +176,20 @@ class DeviceBatchedSQP:
         """Algorithm::initialization (src/Algorithm.cpp:438-472) for a new batch of `batch` starting points on the same object:
         handles, device buffers and the compiled NLP are kept, so the per-batch cost is one upload, one evaluation and one
         state-reset launch."""
-        torch, T, B = self.torch, self.T, self.batch
+        B = self.batch
         x0 = np.ascontiguousarray(np.atleast_2d(np.asarray(x0, dtype=np.float64)))
         if x0.shape != (B, self.nVar_):
             raise ValueError("reset() needs %d starting points of dimension %d" % (B, self.nVar_))
+        with self.torch.cuda.stream(self.stream):
+            self._reset(x0)
+
+    def _reset(self, x0):
+        torch, T, B = self.torch, self.T, self.batch
         T["x_k"].copy_(torch.from_numpy(x0), non_blocking=False)
         torch.minimum(torch.maximum(T["x_k"], T["x_l"]), T["x_u"], out=T["x_k"])  # shift_starting_point
         T["lam_c"].copy_(torch.from_numpy(self._lam_start).to(self.dev).expand(B, -1))
         torch.neg(T["lam_c"], out=T["neg_lam"])
-        self.nlp_.eval_device(1, B, T["x_k"], T["neg_lam"], T["f_k"], T["c_k"], T["grad"], T["jac"], T["hess"])
+        self.nlp_.eval_device(1, B, T["x_k"], T["neg_lam"], T["f_k"], T["c_k"], T["grad"], T["jac"], T["hess"], stream=self.stream)
         self.S.clear_flags = 0
         self._phase(PH_INIT)
         for hd in (self.myQP_, self.myLP_):
@@ -156,7 +198,7 @@ class DeviceBatchedSQP:
 
     # ---- helpers
     def _phase(self, phase, read=False):
-        rc = self.L.sqpb200_sqp_phase(C.byref(self.S), phase, self._counters if read else None, None)
+        rc = self.L.sqpb200_sqp_phase(C.byref(self.S), phase, self._counters if read else None, self._sp)
         if rc != 0:
             raise capi.SqpB200Error("sqpb200_sqp_phase(%d) failed: %d" % (phase, rc))
         self.launches += 1
@@ -170,7 +212,7 @@ class DeviceBatchedSQP:
         first, nl = C.c_int(1 if self.first_ else 0), C.c_longlong(0)
         rc = self.L.sqpb200_sqp_optimize(C.byref(self.S), self.myQP_.solverInterface_.h, self.myLP_.solverInterface_.h, self.nlp_.h,
                                          int(bool(self.options_.second_order_correction)), 1, C.byref(first),
-                                         C.c_void_p(T["f_tmp"].data_ptr()), C.c_void_p(T["c_tmp"].data_ptr()), C.byref(nl), None)
+                                         C.c_void_p(T["f_tmp"].data_ptr()), C.c_void_p(T["c_tmp"].data_ptr()), C.byref(nl), self._sp)
         self._check(rc, "sqpb200_sqp_optimize")
         self.first_ = bool(first.value)
         self.launches += int(nl.value)
@@ -187,35 +229,14 @@ class DeviceBatchedSQP:
         on the B200 (profiles/r3_sqp_stream.md) batch // 64, // 16 and // 4 were within 1 % of each other, while 1 (a refill round in
         nearly every iteration) was up to 30 % slower.  self.stream_rounds holds the number of
         refill rounds of the last call, the initial fill included.  The object serves reset() / Optimize() afterwards as before."""
-        torch, T, B, n, m = self.torch, self.T, self.batch, self.nVar_, self.nCon_
-        if not self.per_instance_modes:
-            raise ValueError("solve_stream needs per_instance_modes=True: with handle-level modes the instances of a handle share "
-                             "its init / hotstart decision, so a refilled slot would inherit a hot start")
-        x0 = np.asarray(x0_all, dtype=np.float64)
-        if x0.ndim != 2 or x0.shape[1] != n:
-            raise ValueError("solve_stream needs starting points of shape (N, %d), got %s" % (n, x0.shape))
-        refill_min = max(1, B // REFILL_MIN_FRACTION) if refill_min is None else int(refill_min)
-        if refill_min < 1:
-            raise ValueError("refill_min must be at least 1")
-        N = x0.shape[0]
-        dev, f64, i32 = self.dev, torch.float64, torch.int32
-        up = lambda a: torch.as_tensor(np.ascontiguousarray(a)).to(dev)
-        O = dict(x0_all=up(x0), lam_start=up(self._lam_start.reshape(-1)), x=torch.empty((N, n), dtype=f64, device=dev),
-                 obj=torch.empty(N, dtype=f64, device=dev), kkt_err=torch.empty(N, dtype=f64, device=dev),
-                 rho=torch.empty(N, dtype=f64, device=dev), delta=torch.empty(N, dtype=f64, device=dev),
-                 exitflag=torch.empty(N, dtype=i32, device=dev), iter=torch.empty(N, dtype=i32, device=dev),
-                 qp_iter=torch.empty(N, dtype=torch.int64, device=dev), slot_id=torch.empty(B, dtype=torch.int64, device=dev),
-                 head=torch.empty(1, dtype=torch.int64, device=dev), refill=torch.empty(B, dtype=torch.uint8, device=dev))
-        D = SqpStream()
-        D.N, D.refill_min = N, refill_min
-        for k, t in O.items():
-            setattr(D, k, t.data_ptr() if t.numel() else None)
+        torch, T = self.torch, self.T
+        O, D = self._stream_buffers("solve_stream", x0_all, refill_min)
         self._structures()
         first, nl = C.c_int(1 if self.first_ else 0), C.c_longlong(0)
         rc = self.L.sqpb200_sqp_optimize_stream(C.byref(self.S), self.myQP_.solverInterface_.h, self.myLP_.solverInterface_.h, self.nlp_.h,
                                                 int(bool(self.options_.second_order_correction)), 1, C.byref(first),
                                                 C.c_void_p(T["f_tmp"].data_ptr()), C.c_void_p(T["c_tmp"].data_ptr()), C.byref(D),
-                                                C.byref(nl), None)
+                                                C.byref(nl), self._sp)
         self._check(rc, "sqpb200_sqp_optimize_stream")
         self.first_ = bool(first.value)
         self.launches += int(nl.value)
@@ -224,6 +245,83 @@ class DeviceBatchedSQP:
         h = lambda k: O[k].cpu().numpy()
         return SQPResult(x=h("x"), obj=h("obj"), exitflag=h("exitflag"), iters=h("iter").astype(np.int64), qp_iter=h("qp_iter"),
                          KKT_error=h("kkt_err"), rho=h("rho"), delta=h("delta"))
+
+    def _need_per_instance_modes(self, what):
+        if not self.per_instance_modes:
+            raise ValueError("%s needs per_instance_modes=True: with handle-level modes the instances of a handle share its init / "
+                             "hotstart decision (a refilled slot would inherit a hot start; the host reads the Update_* bits back)"
+                             % what)
+
+    def _stream_buffers(self, what, x0_all, refill_min):
+        """inputs, results and slot bookkeeping of a streamed solve (device tensors, queued on the object's stream) and their
+        sqpb200_sqp_stream descriptor"""
+        torch, B, n = self.torch, self.batch, self.nVar_
+        self._need_per_instance_modes(what)
+        x0 = np.asarray(x0_all, dtype=np.float64)
+        if x0.ndim != 2 or x0.shape[1] != n:
+            raise ValueError("%s needs starting points of shape (N, %d), got %s" % (what, n, x0.shape))
+        refill_min = max(1, B // REFILL_MIN_FRACTION) if refill_min is None else int(refill_min)
+        if refill_min < 1:
+            raise ValueError("refill_min must be at least 1")
+        N = x0.shape[0]
+        dev, f64, i32 = self.dev, torch.float64, torch.int32
+        # pinned host copies: the upload is queued on the stream instead of waiting for it
+        up = lambda a: torch.as_tensor(np.ascontiguousarray(a)).pin_memory().to(dev, non_blocking=True)
+        with torch.cuda.stream(self.stream):
+            O = dict(x0_all=up(x0), lam_start=up(self._lam_start.reshape(-1)), x=torch.empty((N, n), dtype=f64, device=dev),
+                 obj=torch.empty(N, dtype=f64, device=dev), kkt_err=torch.empty(N, dtype=f64, device=dev),
+                 rho=torch.empty(N, dtype=f64, device=dev), delta=torch.empty(N, dtype=f64, device=dev),
+                 exitflag=torch.empty(N, dtype=i32, device=dev), iter=torch.empty(N, dtype=i32, device=dev),
+                 qp_iter=torch.empty(N, dtype=torch.int64, device=dev), slot_id=torch.empty(B, dtype=torch.int64, device=dev),
+                     head=torch.empty(1, dtype=torch.int64, device=dev), refill=torch.empty(B, dtype=torch.uint8, device=dev))
+        D = SqpStream()
+        D.N, D.refill_min = N, refill_min
+        for k, t in O.items():
+            setattr(D, k, t.data_ptr() if t.numel() else None)
+        return O, D
+
+    # ---- asynchronous solves (sqpb200_sqp_graph_*)
+    def optimize_async(self):
+        """Optimize() queued on the object's stream; returns a PendingSQP at once.  Bit for bit what Optimize() gives for the same
+        sequence of calls on the object.  Needs per-instance backend state machines."""
+        self._need_per_instance_modes("optimize_async")
+        T = self.T
+        self._launch_graph(None)
+        with self.torch.cuda.stream(self.stream):
+            out = {k: T[s].clone() for k, s in (("x", "x_k"), ("obj", "f_k"), ("exitflag", "exitflag"), ("iter", "iter"),
+                                                 ("qp_iter", "qp_iter"), ("kkt_err", "kkt_err"), ("rho", "rho"), ("delta", "delta"))}
+        return self._pending(out)
+
+    def solve_stream_async(self, x0_all, refill_min=None):
+        """solve_stream() queued on the object's stream; returns a PendingSQP at once (stream_rounds is not set).  Each call records
+        its loop again: the descriptor of the call is part of the graph."""
+        O, D = self._stream_buffers("solve_stream_async", x0_all, refill_min)
+        self._launch_graph(D)
+        return self._pending(O, keep=D)
+
+    def _create_graph(self):
+        """records the loop of Optimize (once per object; close() releases it)"""
+        T = self.T
+        self._structures()
+        g = C.c_void_p()
+        rc = self.L.sqpb200_sqp_graph_create(C.byref(self.S), self.myQP_.solverInterface_.h, self.myLP_.solverInterface_.h, self.nlp_.h,
+                                             int(bool(self.options_.second_order_correction)), 1, C.c_void_p(T["f_tmp"].data_ptr()),
+                                             C.c_void_p(T["c_tmp"].data_ptr()), self._sp, C.byref(g))
+        self._check(rc, "sqpb200_sqp_graph_create")
+        self._graph = g
+
+    def _launch_graph(self, D):
+        if self._graph is None:
+            self._create_graph()
+        first = C.c_int(1 if self.first_ else 0)
+        rc = self.L.sqpb200_sqp_graph_launch(self._graph, C.byref(first), None if D is None else C.byref(D))
+        self._check(rc, "sqpb200_sqp_graph_launch")
+        self.first_ = bool(first.value)
+
+    def _pending(self, out, keep=None):
+        ev = self.torch.cuda.Event()
+        ev.record(self.stream if self.stream is not None else self.torch.cuda.current_stream(self.dev))
+        return PendingSQP(out, ev, keep)
 
     def _structures(self):
         """structures of both backends (first set_A / set_H call of setupQP / setupLP, values follow in the loop)"""
@@ -246,5 +344,8 @@ class DeviceBatchedSQP:
                          KKT_error=h("kkt_err"), rho=h("rho"), delta=h("delta"))
 
     def close(self):
+        if self._graph is not None:
+            self.L.sqpb200_sqp_graph_destroy(self._graph)
+            self._graph = None
         self.myQP_.solverInterface_.close()
         self.myLP_.solverInterface_.close()
