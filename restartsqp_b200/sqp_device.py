@@ -56,6 +56,16 @@ class SqpStream(C.Structure):
 #: default refill_min of solve_stream as a fraction of the slot count (see solve_stream)
 REFILL_MIN_FRACTION = 16
 
+#: the state tensor each result is read from, keyed as the result arrays of SqpStream
+_STATE_RESULTS = dict(x="x_k", obj="f_k", exitflag="exitflag", iter="iter", qp_iter="qp_iter", kkt_err="kkt_err", rho="rho", delta="delta")
+
+
+def _sqp_result(out):
+    """SQPResult from finished device tensors keyed as the result arrays of SqpStream"""
+    h = lambda k: out[k].cpu().numpy()
+    return SQPResult(x=h("x"), obj=h("obj"), exitflag=h("exitflag"), iters=h("iter").astype(np.int64), qp_iter=h("qp_iter"),
+                     KKT_error=h("kkt_err"), rho=h("rho"), delta=h("delta"))
+
 
 class PendingSQP:
     """A solve queued by optimize_async / solve_stream_async.  Its results are copied on the object's stream into tensors this object
@@ -73,9 +83,7 @@ class PendingSQP:
 
     def result(self):
         self.wait()
-        h = lambda k: self._out[k].cpu().numpy()
-        return SQPResult(x=h("x"), obj=h("obj"), exitflag=h("exitflag"), iters=h("iter").astype(np.int64), qp_iter=h("qp_iter"),
-                         KKT_error=h("kkt_err"), rho=h("rho"), delta=h("delta"))
+        return _sqp_result(self._out)
 
 
 class DeviceBatchedSQP:
@@ -164,7 +172,6 @@ class DeviceBatchedSQP:
         self.L.sqpb200_device_buffers(self.myLP_.solverInterface_.h, bl)
         S.qp_x, S.qp_y, S.qp_obj, S.qp_status, S.qp_iters, S.qp_kkt = bq[0], bq[1], bq[2], bq[3], bq[4], bq[5]
         S.lp_x, S.lp_status, S.lp_iters = bl[0], bl[3], bl[4]
-        self._counters = (C.c_int * 8)()
         self.first_ = True
         self.launches = 0
         S.delta0, S.rho0, S.eps10 = float(o.delta), float(o.rho), float(o.eps1)
@@ -197,12 +204,11 @@ class DeviceBatchedSQP:
         self.first_ = True
 
     # ---- helpers
-    def _phase(self, phase, read=False):
-        rc = self.L.sqpb200_sqp_phase(C.byref(self.S), phase, self._counters if read else None, self._sp)
+    def _phase(self, phase):
+        rc = self.L.sqpb200_sqp_phase(C.byref(self.S), phase, None, self._sp)
         if rc != 0:
             raise capi.SqpB200Error("sqpb200_sqp_phase(%d) failed: %d" % (phase, rc))
         self.launches += 1
-        return list(self._counters) if read else None
 
     # ---- src/Algorithm.cpp:55-168
     def Optimize(self):
@@ -216,7 +222,8 @@ class DeviceBatchedSQP:
         self._check(rc, "sqpb200_sqp_optimize")
         self.first_ = bool(first.value)
         self.launches += int(nl.value)
-        return self._result()
+        self.torch.cuda.synchronize()
+        return _sqp_result({k: T[s] for k, s in _STATE_RESULTS.items()})
 
     def solve_stream(self, x0_all, refill_min=None):
         """Algorithm::Optimize for N starting points x0_all[N][n] through the `batch` instances of this object used as slots: a slot
@@ -242,9 +249,7 @@ class DeviceBatchedSQP:
         self.launches += int(nl.value)
         self.stream_rounds = int(D.rounds)
         torch.cuda.synchronize()
-        h = lambda k: O[k].cpu().numpy()
-        return SQPResult(x=h("x"), obj=h("obj"), exitflag=h("exitflag"), iters=h("iter").astype(np.int64), qp_iter=h("qp_iter"),
-                         KKT_error=h("kkt_err"), rho=h("rho"), delta=h("delta"))
+        return _sqp_result(O)
 
     def _need_per_instance_modes(self, what):
         if not self.per_instance_modes:
@@ -288,8 +293,7 @@ class DeviceBatchedSQP:
         T = self.T
         self._launch_graph(None)
         with self.torch.cuda.stream(self.stream):
-            out = {k: T[s].clone() for k, s in (("x", "x_k"), ("obj", "f_k"), ("exitflag", "exitflag"), ("iter", "iter"),
-                                                 ("qp_iter", "qp_iter"), ("kkt_err", "kkt_err"), ("rho", "rho"), ("delta", "delta"))}
+            out = {k: T[s].clone() for k, s in _STATE_RESULTS.items()}
         return self._pending(out)
 
     def solve_stream_async(self, x0_all, refill_min=None):
@@ -335,13 +339,6 @@ class DeviceBatchedSQP:
         if rc != 0:
             raise capi.SqpB200Error("%s failed (%d): %s / %s" % (
                 what, rc, self.L.sqpb200_last_error(self.myQP_.solverInterface_.h).decode(), self.L.sqpb200_last_error(self.myLP_.solverInterface_.h).decode()))
-
-    def _result(self):
-        T = self.T
-        self.torch.cuda.synchronize()
-        h = lambda k: T[k].cpu().numpy()
-        return SQPResult(x=h("x_k"), obj=h("f_k"), exitflag=h("exitflag"), iters=h("iter").astype(np.int64), qp_iter=h("qp_iter"),
-                         KKT_error=h("kkt_err"), rho=h("rho"), delta=h("delta"))
 
     def close(self):
         if self._graph is not None:
