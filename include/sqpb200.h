@@ -110,14 +110,23 @@ const char* sqpb200_last_error(sqpb200_handle h);
  * (src/qpOASESInterface.cpp:426-437, 400-417; src/SpHbMat.cpp:196-268, 284-355).
  * Triplets are 1-based (FORTRAN style, src/SQPTNLP.cpp:18).  The identity blocks are the
  * IdentityInfo of include/sqphot/Types.hpp:36-42.  Runs the device segmented sort/scan.
- * Returns the number of CSC entries (>= 0) or a negative error. */
+ * Returns the number of CSC entries (>= 0) or a negative error.
+ * Every structure call (these, sqpb200_set_structure_csc and the compressed-row forms below)
+ * checks all of its input before it changes the handle: malformed input (an index out of
+ * range, a malformed pointer array) returns SQPB200_ERR_INVALID and leaves the handle as it
+ * was.  A structure may be set again, the last call winning, until a solve has allocated the
+ * handle's solve buffers, which are sized by the structures (the first solve does, unless
+ * keep_state = 0 and the QPs fit the shared-memory kernel); from then on a structure call
+ * returns SQPB200_ERR_STATE and leaves the handle as it was. */
 int sqpb200_set_structure_A(sqpb200_handle h, int zJ, const int* row1, const int* col1, int I_len,
                             const int* I_irow, const int* I_jcol, const int* I_size,
                             const double* I_value);
 int sqpb200_set_structure_H(sqpb200_handle h, int zH, const int* row1, const int* col1,
                             int is_symmetric);
 /* Direct CSC structure (the data constructor used by the replay driver,
- * src/qpOASESInterface.cpp:54-94, test/QPsolvers_testers.cpp:220-221). */
+ * src/qpOASESInterface.cpp:54-94, test/QPsolvers_testers.cpp:220-221): colptr[nV+1] with
+ * colptr[0] = 0, non-decreasing, colptr[nV] = nnz; rowidx[nnz], 0-based rows below nC (A) or
+ * nV (H).  Returns nnz or a negative error; the rules above apply. */
 int sqpb200_set_structure_csc(sqpb200_handle h, int which, int nnz, const int* colptr,
                               const int* rowidx);
 /* Copy the CSC index arrays back to the host for parity checks: colptr[ncol+1], rowidx[nnz],
@@ -377,13 +386,15 @@ int sqpb200_device_buffers(sqpb200_handle h, void** out);
  * sqpb200_set_structure_A_csr / _H_csr: first call of QOREInterface::set_A / set_H (src/QOREInterface.cpp:643-659) ->
  * SpHbMat(..., isCompressedRow = true)::setStructure (src/SpHbMat.cpp:238-250, 324-337): same arguments as
  * sqpb200_set_structure_A / _H, same device sort with the key (row, column, counter); later sqpb200_set_values_A / _H calls take
- * triplet-ordered values as before.  Return the number of entries or a negative error. */
+ * triplet-ordered values as before.  Return the number of entries or a negative error.  The rules of sqpb200_set_structure_A
+ * (validation before any change, no structure call once the solve buffers exist) apply to all three structure calls here. */
 int sqpb200_set_structure_A_csr(sqpb200_handle h, int zJ, const int* row1, const int* col1, int I_len,
                                 const int* I_irow, const int* I_jcol, const int* I_size, const double* I_value);
 int sqpb200_set_structure_H_csr(sqpb200_handle h, int zH, const int* row1, const int* col1, int is_symmetric);
 /* Direct compressed-row structure: the data constructor QOREInterface(H, A, g, lb, ub, options) of the replay driver
- * (src/QOREInterface.cpp:36-60, test/QPsolvers_testers.cpp:74-75, 172-175).  rowptr[nrow+1], colidx[nnz], 0-based, entries of a
- * row in ascending column order.  Values then arrive in this storage order through sqpb200_set_values_csr. */
+ * (src/QOREInterface.cpp:36-60, test/QPsolvers_testers.cpp:74-75, 172-175).  rowptr[nrow+1] with rowptr[0] = 0, non-decreasing,
+ * rowptr[nrow] = nnz; colidx[nnz], 0-based columns below nV, entries of a row in ascending column order.  Values then arrive in
+ * this storage order through sqpb200_set_values_csr.  Returns nnz or a negative error. */
 int sqpb200_set_structure_csr(sqpb200_handle h, int which, int nnz, const int* rowptr, const int* colidx);
 /* rowptr[nrow+1], colidx[nnz], order[nnz] (triplet entry -> storage position; any pointer may be NULL) of a handle whose
  * structure was set through one of the three calls above. */

@@ -29,26 +29,34 @@ enum { MS_UNDEFINED = -1, MS_FIXED = 0, MS_VARIED = 1 };
 
 struct SolveCfg { int cap = 0, teams = 0, smem = 0, slice_doubles = 0, state_doubles = 0, resident = 0, lanes = 32; };
 
+// QORE layout (compressed-row view given by the caller, sqpb200_set_structure_*_csr): row pointers, column indices, triplet ->
+// storage position, and the position maps between the two storage orders (q2c[compressed-row position] = compressed-column
+// position, c2q its inverse)
+struct CsrView { bool set = false; std::vector<int> rp, ci, order, q2c, c2q; };
+
+// One sparse matrix (A or H) of every instance: the compressed-column pattern the kernels work on and the values
+struct SparseMat {
+    bool set = false;
+    int z = 0, zin = 0;  // z: stored entries; zin: entries of a triplet-ordered value row (A: zJ, H: the triplets before mirroring)
+    std::vector<int> p, i, order, src;  // colptr, rowidx, triplet entry -> position, position -> triplet entry (-1: none)
+    int *dp = nullptr, *di = nullptr, *dsrc = nullptr;
+    double* dval = nullptr;  // [batch][z]
+    CsrView q;
+    int *dq2c = nullptr, *dc2q = nullptr;  // q's position maps, resident for the device-side value moves
+};
+
 struct sqpb200_handle_s {
     int batch = 0, nV = 0, nC = 0, qptype = SQPB200_QP, device = 0;
     sqpb200_options opt;
     cudaStream_t stream = nullptr;
     std::string err;
     // structure
-    bool A_set = false, H_set = false;
-    int zA = 0, zJ = 0, zH = 0, zHt = 0;  // zH: CSC entries of H; zHt: triplet count
-    std::vector<int> Ap, Ai, Aorder, Asrc, Hp, Hi, Horder, Hsrc;
-    std::vector<double> A_init;
-    int *dAp = nullptr, *dAi = nullptr, *dArp = nullptr, *dAci = nullptr, *dAperm = nullptr, *dAsrc = nullptr;
-    int *dHp = nullptr, *dHi = nullptr, *dHsrc = nullptr;
-    // QORE layout (compressed-row view given by the caller, sqpb200_set_structure_*_csr): row pointers, column indices, triplet ->
-    // storage position, and the position maps between the two storage orders (q2c[compressed-row position] = compressed-column
-    // position, c2q its inverse), resident for the device-side value moves
-    struct CsrView { bool set = false; std::vector<int> rp, ci, order, q2c, c2q; int *dq2c = nullptr, *dc2q = nullptr; } qA, qH;
+    SparseMat A, H;
+    std::vector<int> Arp, Aci, Aperm;  // row-wise view of A: row pointers, column and storage position of each entry
+    int *dArp = nullptr, *dAci = nullptr, *dAperm = nullptr;
     void* qscratch = nullptr;  // [batch][nC] doubles (A x) + [batch][nV+nC] int32 (working set) of sqpb200_get_solution_stacked
     size_t qscratch_bytes = 0;
     // data
-    double *dAval = nullptr, *dHval = nullptr;
     double *dg = nullptr, *dlb = nullptr, *dub = nullptr, *dlbA = nullptr, *dubA = nullptr;
     // results
     double *dx = nullptr, *dy = nullptr, *dobj = nullptr, *dkkt = nullptr;
@@ -211,11 +219,11 @@ int sqpb200_destroy(sqpb200_handle h) {
     if (!h) return SQPB200_ERR_INVALID;
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
-    void* ptrs[] = {h->dAp, h->dAi, h->dArp, h->dAci, h->dAperm, h->dAsrc, h->dHp, h->dHi, h->dHsrc, h->dAval, h->dHval,
-                    h->arena, h->dstate, h->stage, h->dgpat, h->dgwork, h->dprof, h->dmaxfr, h->dncap};
+    void* ptrs[] = {h->dArp, h->dAci, h->dAperm, h->arena, h->dstate, h->stage, h->dgpat, h->dgwork, h->dprof, h->dmaxfr,
+                    h->dncap, h->qscratch};
     for (void* p : ptrs) if (p) cudaFree(p);
-    void* qptrs[] = {h->qA.dq2c, h->qA.dc2q, h->qH.dq2c, h->qH.dc2q, h->qscratch};
-    for (void* p : qptrs) if (p) cudaFree(p);
+    for (SparseMat* M : {&h->A, &h->H})
+        for (void* p : {(void*)M->dp, (void*)M->di, (void*)M->dsrc, (void*)M->dval, (void*)M->dq2c, (void*)M->dc2q}) if (p) cudaFree(p);
     if (h->ev0) cudaEventDestroy(h->ev0);
     if (h->ev1) cudaEventDestroy(h->ev1);
     if (h->ev_maxfr) cudaEventDestroy(h->ev_maxfr);
@@ -263,10 +271,8 @@ int sqpb200_synchronize(sqpb200_handle h) {
 
 // ------------------------------------------------------------------------------ assembly
 // Runs csc_assemble_kernel over nmat segments whose triplets are already on the host.
-static int run_assembly(sqpb200_handle h, cudaStream_t stream, int nmat, const int* seg, const int* ncol,
-                        const int* row1, const int* col1, int* colptr, int* rowidx, int* order, float* ms,
-                        std::string* err) {
-    (void)h;
+static int run_assembly(cudaStream_t stream, int nmat, const int* seg, const int* ncol, const int* row1, const int* col1,
+                        int* colptr, int* rowidx, int* order, float* ms, std::string* err) {
     int ztot = seg[nmat];
     std::vector<int> cp_off(nmat + 1, 0), pad_off(nmat + 1, 0);
     for (int m = 0; m < nmat; m++) {
@@ -337,7 +343,7 @@ int sqpb200_assemble_csc_batched(int device, int nmat, const int* seg, const int
     if (nmat <= 0 || !seg || !ncol) return SQPB200_ERR_INVALID;
     if (cudaSetDevice(device) != cudaSuccess) return SQPB200_ERR_CUDA;
     std::string err;
-    return run_assembly(nullptr, nullptr, nmat, seg, ncol, row1, col1, colptr, rowidx, order, kernel_ms, &err);
+    return run_assembly(nullptr, nmat, seg, ncol, row1, col1, colptr, rowidx, order, kernel_ms, &err);
 }
 
 template <typename T>
@@ -349,147 +355,209 @@ static int upload_vec(sqpb200_handle h, T** d, const std::vector<T>& v) {
     return 0;
 }
 
-static int finish_structure_A(sqpb200_handle h) {
-    const int nV = h->nV, nC = h->nC, zA = h->zA;
-    // CSR view of the CSC pattern: entries of each row in column order (the CSC storage order)
-    std::vector<int> Arp(nC + 1, 0), Aci(zA), Aperm(zA);
-    for (int e = 0; e < zA; e++) Arp[h->Ai[e] + 1]++;
-    for (int r = 0; r < nC; r++) Arp[r + 1] += Arp[r];
-    std::vector<int> fill(Arp.begin(), Arp.end() - 1);
-    for (int c = 0; c < nV; c++)
-        for (int e = h->Ap[c]; e < h->Ap[c + 1]; e++) { int r = h->Ai[e]; Aci[fill[r]] = c; Aperm[fill[r]] = e; fill[r]++; }
+// ------------------------------------------------------------------------------ structure
+// Every structure call builds and checks a Pattern completely before it touches the handle, so a rejected call leaves the
+// handle as it was.  Three routes lead to a Pattern: the triplet setters sort an entry list on the device, either directly
+// (key column, row, counter) or through the compressed-row sort of QORE's SpHbMat (key row, column, counter) and its
+// transpose; the data constructors give the pattern as it is stored.  install() then makes it the handle's.
+
+static SparseMat& mat(sqpb200_handle h, int which) { return which == SQPB200_MAT_A ? h->A : h->H; }
+
+// The entry list of SpHbMat::setStructure: 1-based row and column, the triplet each entry comes from (-1: an identity entry)
+// and, for A, its initial value (the identity block's value, 0 for a triplet).  H has no initial values.
+struct Entries {
+    std::vector<int> row, col, src;
+    std::vector<double> init;
+};
+
+// SpHbMat::setStructure(rhs, I_info), src/SpHbMat.cpp:203-227: the triplets, then the diagonal of every identity block
+static Entries entries_A(int zJ, const int* row1, const int* col1, int I_len, const int* I_irow, const int* I_jcol,
+                         const int* I_size, const double* I_value) {
+    Entries e;
+    for (int k = 0; k < zJ; k++) { e.row.push_back(row1[k]); e.col.push_back(col1[k]); e.src.push_back(k); e.init.push_back(0.0); }
+    for (int b = 0; b < I_len; b++)
+        for (int j = 0; j < I_size[b]; j++) {
+            e.row.push_back(I_irow[b] + j); e.col.push_back(I_jcol[b] + j); e.src.push_back(-1); e.init.push_back(I_value[b]);
+        }
+    return e;
+}
+
+// SpHbMat::setStructure(rhs), src/SpHbMat.cpp:296-309: a symmetric triplet off the diagonal stands for two entries
+static Entries entries_H(int zH, const int* row1, const int* col1, int is_symmetric) {
+    Entries e;
+    for (int k = 0; k < zH; k++) {
+        e.row.push_back(row1[k]); e.col.push_back(col1[k]); e.src.push_back(k);
+        if (is_symmetric && row1[k] != col1[k]) { e.row.push_back(col1[k]); e.col.push_back(row1[k]); e.src.push_back(k); }
+    }
+    return e;
+}
+
+// A pattern on its way into the handle
+struct Pattern {
+    std::vector<int> p, i, order, src;  // as in SparseMat
+    std::vector<double> init;           // initial value of every position, the same in every instance (empty: none)
+    int zin = 0;
+    CsrView q;  // q.set: the structure was given in compressed-row form (q.rp, q.ci, q.order)
+};
+
+// The compressed-column pattern of the compressed-row one in P.q, the position map q2c and the order of the entries: entries
+// with equal keys keep their order
+static void csr_to_csc(int nrow, int ncol, Pattern& P) {
+    CsrView& q = P.q;
+    const int z = (int)q.ci.size();
+    P.p.assign(ncol + 1, 0); P.i.assign(z, 0); q.q2c.assign(z, 0); P.order.assign(z, 0);
+    for (int e = 0; e < z; e++) P.p[q.ci[e] + 1]++;
+    for (int c = 0; c < ncol; c++) P.p[c + 1] += P.p[c];
+    std::vector<int> fill(P.p.begin(), P.p.end() - 1);
+    for (int r = 0; r < nrow; r++)
+        for (int e = q.rp[r]; e < q.rp[r + 1]; e++) { const int pos = fill[q.ci[e]]++; P.i[pos] = r; q.q2c[e] = pos; }
+    for (int k = 0; k < z; k++) P.order[k] = q.q2c[q.order[k]];
+    q.set = true;
+}
+
+// position order[k] takes entry k's value source and initial value
+static void place(Pattern& P, const std::vector<int>& src, const std::vector<double>& init) {
+    const int z = (int)P.order.size();
+    P.src.assign(z, -1);
+    if (!init.empty()) P.init.assign(z, 0.0);
+    for (int k = 0; k < z; k++) {
+        P.src[P.order[k]] = src[k];
+        if (!init.empty()) P.init[P.order[k]] = init[k];
+    }
+}
+
+// The solve buffers (hot-start images, the cluster kernel's slices) are sized by the patterns when they are first allocated:
+// from then on the patterns are fixed.
+static int structure_open(sqpb200_handle h) {
+    if (!h->dstate && !h->dgwork) return 0;
+    h->err = "the structure cannot change once the handle has solved (its solve buffers are sized by it)";
+    return SQPB200_ERR_STATE;
+}
+
+// Makes P the pattern of A or H: host and device arrays (for A also the row-wise view), a zeroed value array for every
+// instance with P.init broadcast into it, the compressed-row view set or cleared.  The solve configuration and the cluster
+// kernel's pattern, both derived from the previous patterns, are dropped.
+static int install(sqpb200_handle h, int which, Pattern& P) {
+    SparseMat& M = mat(h, which);
+    const int z = (int)P.i.size();
+    M.z = z; M.zin = P.zin;
+    M.p = std::move(P.p); M.i = std::move(P.i); M.order = std::move(P.order); M.src = std::move(P.src);
+    M.q = std::move(P.q);
     int rc = 0;
-    rc |= upload_vec(h, &h->dAp, h->Ap); rc |= upload_vec(h, &h->dAi, h->Ai);
-    rc |= upload_vec(h, &h->dArp, Arp); rc |= upload_vec(h, &h->dAci, Aci); rc |= upload_vec(h, &h->dAperm, Aperm);
-    rc |= upload_vec(h, &h->dAsrc, h->Asrc);
+    rc |= upload_vec(h, &M.dp, M.p); rc |= upload_vec(h, &M.di, M.i); rc |= upload_vec(h, &M.dsrc, M.src);
+    if (which == SQPB200_MAT_A) {  // the entries of each row in column order (the storage order)
+        h->Arp.assign(h->nC + 1, 0); h->Aci.assign(z, 0); h->Aperm.assign(z, 0);
+        for (int e = 0; e < z; e++) h->Arp[M.i[e] + 1]++;
+        for (int r = 0; r < h->nC; r++) h->Arp[r + 1] += h->Arp[r];
+        std::vector<int> fill(h->Arp.begin(), h->Arp.end() - 1);
+        for (int c = 0; c < h->nV; c++)
+            for (int e = M.p[c]; e < M.p[c + 1]; e++) { const int r = M.i[e]; h->Aci[fill[r]] = c; h->Aperm[fill[r]] = e; fill[r]++; }
+        rc |= upload_vec(h, &h->dArp, h->Arp); rc |= upload_vec(h, &h->dAci, h->Aci); rc |= upload_vec(h, &h->dAperm, h->Aperm);
+    }
+    if (M.q.set) {
+        M.q.c2q.assign(z, 0);
+        for (int e = 0; e < z; e++) M.q.c2q[M.q.q2c[e]] = e;
+        rc |= upload_vec(h, &M.dq2c, M.q.q2c); rc |= upload_vec(h, &M.dc2q, M.q.c2q);
+    }
     if (rc) return SQPB200_ERR_CUDA;
-    if (h->dAval) { CK(cudaFree(h->dAval)); h->dAval = nullptr; }
-    if (dev_alloc(h, &h->dAval, (size_t)h->batch * zA)) return SQPB200_ERR_CUDA;
-    if (!h->A_init.empty() && zA > 0) {  // identity entries (and zeros) in every instance
-        if (ensure_stage(h, (size_t)zA * 8)) return SQPB200_ERR_CUDA;
-        CK(cudaMemcpyAsync(h->stage, h->A_init.data(), (size_t)zA * 8, cudaMemcpyHostToDevice, h->stream));
-        long long total = (long long)h->batch * zA;
-        broadcast_rows_kernel<<<grid_for(total, 256), 256, 0, h->stream>>>(total, zA, 0, zA, (const double*)h->stage, h->dAval);
+    if (M.dval) { CK(cudaFree(M.dval)); M.dval = nullptr; }
+    if (dev_alloc(h, &M.dval, (size_t)h->batch * z)) return SQPB200_ERR_CUDA;
+    if (!P.init.empty() && z > 0) {  // identity entries (and zeros) in every instance
+        if (ensure_stage(h, (size_t)z * 8)) return SQPB200_ERR_CUDA;
+        CK(cudaMemcpyAsync(h->stage, P.init.data(), (size_t)z * 8, cudaMemcpyHostToDevice, h->stream));
+        long long total = (long long)h->batch * z;
+        broadcast_rows_kernel<<<grid_for(total, 256), 256, 0, h->stream>>>(total, z, 0, z, (const double*)h->stage, M.dval);
         h->launches++;
         CK(cudaGetLastError());
     }
-    h->A_set = true;
-    h->cfg_cap_key = -1;  // slice layout depends on zA
+    M.set = true;
+    h->cfg_cap_key = -1;  // the slice layout depends on z
     if (h->dgpat) { cudaFree(h->dgpat); h->dgpat = nullptr; }
     return 0;
+}
+
+// Triplet route: returns the number of stored entries or a negative error
+static int set_triplets(sqpb200_handle h, int which, const Entries& e, int zin, bool csr) {
+    CK(cudaSetDevice(h->device));
+    int rc = structure_open(h);
+    if (rc) return rc;
+    const int nrow = which == SQPB200_MAT_A ? h->nC : h->nV, z = (int)e.row.size();
+    for (int k = 0; k < z; k++)
+        if (e.row[k] < 1 || e.row[k] > nrow || e.col[k] < 1 || e.col[k] > h->nV) { h->err = "triplet index out of range"; return SQPB200_ERR_INVALID; }
+    Pattern P;
+    P.zin = zin;
+    const int seg[2] = {0, z};
+    if (csr) {  // compressed-row branch of SpHbMat::setStructure (src/SpHbMat.cpp:238-250, 324-337)
+        P.q.rp.assign(nrow + 1, 0); P.q.ci.assign(z, 0); P.q.order.assign(z, 0);
+        if (z > 0) rc = run_assembly(h->stream, 1, seg, &nrow, e.col.data(), e.row.data(), P.q.rp.data(), P.q.ci.data(), P.q.order.data(), nullptr, &h->err);
+    } else {
+        P.p.assign(h->nV + 1, 0); P.i.assign(z, 0); P.order.assign(z, 0);
+        if (z > 0) rc = run_assembly(h->stream, 1, seg, &h->nV, e.row.data(), e.col.data(), P.p.data(), P.i.data(), P.order.data(), nullptr, &h->err);
+    }
+    if (z > 0) h->launches++;
+    if (rc) return rc;
+    if (csr) csr_to_csc(nrow, h->nV, P);
+    place(P, e.src, e.init);
+    rc = install(h, which, P);
+    return rc ? rc : z;
+}
+
+// Direct route (the data constructors): a 0-based pattern as it is stored, compressed-column (colptr, rowidx) or compressed-row
+// (rowptr, colidx).  Values then arrive in that storage order.  Returns nnz or a negative error.
+static int set_direct(sqpb200_handle h, int which, int nnz, const int* ptr, const int* idx, bool csr) {
+    if (!h || nnz < 0 || !ptr || (nnz > 0 && !idx) || (which != SQPB200_MAT_A && which != SQPB200_MAT_H)) return SQPB200_ERR_INVALID;
+    CK(cudaSetDevice(h->device));
+    int rc = structure_open(h);
+    if (rc) return rc;
+    const int nrow = which == SQPB200_MAT_A ? h->nC : h->nV, nptr = csr ? nrow : h->nV, nidx = csr ? h->nV : nrow;
+    if (ptr[0] != 0 || ptr[nptr] != nnz) { h->err = csr ? "rowptr[0] != 0 or rowptr[nrow] != nnz" : "colptr[0] != 0 or colptr[ncol] != nnz"; return SQPB200_ERR_INVALID; }
+    for (int k = 0; k < nptr; k++)
+        if (ptr[k + 1] < ptr[k]) { h->err = csr ? "rowptr not monotone" : "colptr not monotone"; return SQPB200_ERR_INVALID; }
+    for (int e = 0; e < nnz; e++)
+        if (idx[e] < 0 || idx[e] >= nidx) { h->err = csr ? "column index out of range" : "row index out of range"; return SQPB200_ERR_INVALID; }
+    Pattern P;
+    P.zin = nnz;
+    std::vector<int> ident(nnz);
+    for (int e = 0; e < nnz; e++) ident[e] = e;
+    if (csr) {
+        P.q.rp.assign(ptr, ptr + nptr + 1); P.q.ci.assign(idx, idx + nnz); P.q.order = ident;
+        csr_to_csc(nrow, h->nV, P);
+    } else {
+        P.p.assign(ptr, ptr + nptr + 1); P.i.assign(idx, idx + nnz); P.order = ident;
+    }
+    place(P, ident, {});
+    rc = install(h, which, P);
+    return rc ? rc : nnz;
 }
 
 int sqpb200_set_structure_A(sqpb200_handle h, int zJ, const int* row1, const int* col1, int I_len,
                             const int* I_irow, const int* I_jcol, const int* I_size, const double* I_value) {
     if (!h || zJ < 0) return SQPB200_ERR_INVALID;
-    CK(cudaSetDevice(h->device));
-    // entry list of SpHbMat::setStructure(rhs, I_info), src/SpHbMat.cpp:203-227
-    std::vector<int> er, ec;
-    std::vector<double> ev;
-    for (int i = 0; i < zJ; i++) { er.push_back(row1[i]); ec.push_back(col1[i]); ev.push_back(0.0); }
-    for (int b = 0; b < I_len; b++)
-        for (int j = 0; j < I_size[b]; j++) { er.push_back(I_irow[b] + j); ec.push_back(I_jcol[b] + j); ev.push_back(I_value[b]); }
-    int z = (int)er.size();
-    for (int i = 0; i < z; i++)
-        if (er[i] < 1 || er[i] > h->nC || ec[i] < 1 || ec[i] > h->nV) { h->err = "triplet index out of range"; return SQPB200_ERR_INVALID; }
-    h->zA = z; h->zJ = zJ;
-    h->qA.set = false;  // a compressed-row view of an earlier structure no longer applies
-    h->Ap.assign(h->nV + 1, 0); h->Ai.assign(z, 0); h->Aorder.assign(z, 0);
-    int seg[2] = {0, z}, ncol[1] = {h->nV};
-    if (z > 0) {
-        int rc = run_assembly(h, h->stream, 1, seg, ncol, er.data(), ec.data(), h->Ap.data(), h->Ai.data(), h->Aorder.data(), nullptr, &h->err);
-        h->launches++;
-        if (rc) return rc;
-    }
-    h->Asrc.assign(z, -1);
-    h->A_init.assign(z, 0.0);
-    for (int i = 0; i < z; i++) {
-        if (i < zJ) h->Asrc[h->Aorder[i]] = i;
-        else h->A_init[h->Aorder[i]] = ev[i];
-    }
-    int rc = finish_structure_A(h);
-    return rc ? rc : z;
+    return set_triplets(h, SQPB200_MAT_A, entries_A(zJ, row1, col1, I_len, I_irow, I_jcol, I_size, I_value), zJ, false);
 }
 
 int sqpb200_set_structure_H(sqpb200_handle h, int zH, const int* row1, const int* col1, int is_symmetric) {
     if (!h || zH < 0) return SQPB200_ERR_INVALID;
-    CK(cudaSetDevice(h->device));
-    // entry list of SpHbMat::setStructure(rhs), src/SpHbMat.cpp:296-309
-    std::vector<int> er, ec, srct;
-    for (int i = 0; i < zH; i++) {
-        er.push_back(row1[i]); ec.push_back(col1[i]); srct.push_back(i);
-        if (is_symmetric && row1[i] != col1[i]) { er.push_back(col1[i]); ec.push_back(row1[i]); srct.push_back(i); }
-    }
-    int z = (int)er.size();
-    for (int i = 0; i < z; i++)
-        if (er[i] < 1 || er[i] > h->nV || ec[i] < 1 || ec[i] > h->nV) { h->err = "triplet index out of range"; return SQPB200_ERR_INVALID; }
-    h->zH = z; h->zHt = zH;
-    h->qH.set = false;
-    h->Hp.assign(h->nV + 1, 0); h->Hi.assign(z, 0); h->Horder.assign(z, 0);
-    int seg[2] = {0, z}, ncol[1] = {h->nV};
-    if (z > 0) {
-        int rc = run_assembly(h, h->stream, 1, seg, ncol, er.data(), ec.data(), h->Hp.data(), h->Hi.data(), h->Horder.data(), nullptr, &h->err);
-        h->launches++;
-        if (rc) return rc;
-    }
-    h->Hsrc.assign(z, -1);
-    for (int i = 0; i < z; i++) h->Hsrc[h->Horder[i]] = srct[i];
-    int rc = 0;
-    rc |= upload_vec(h, &h->dHp, h->Hp); rc |= upload_vec(h, &h->dHi, h->Hi); rc |= upload_vec(h, &h->dHsrc, h->Hsrc);
-    if (rc) return SQPB200_ERR_CUDA;
-    if (h->dHval) { CK(cudaFree(h->dHval)); h->dHval = nullptr; }
-    if (dev_alloc(h, &h->dHval, (size_t)h->batch * z)) return SQPB200_ERR_CUDA;
-    h->H_set = true;
-    h->cfg_cap_key = -1;
-    return z;
+    return set_triplets(h, SQPB200_MAT_H, entries_H(zH, row1, col1, is_symmetric), zH, false);
 }
 
 int sqpb200_set_structure_csc(sqpb200_handle h, int which, int nnz, const int* colptr, const int* rowidx) {
-    if (!h || nnz < 0 || !colptr) return SQPB200_ERR_INVALID;
-    CK(cudaSetDevice(h->device));
-    if (colptr[h->nV] != nnz) { h->err = "colptr[ncol] != nnz"; return SQPB200_ERR_INVALID; }
-    if (which == SQPB200_MAT_A) {
-        h->zA = nnz; h->zJ = nnz;
-        h->qA.set = false;
-        h->Ap.assign(colptr, colptr + h->nV + 1); h->Ai.assign(rowidx, rowidx + nnz);
-        h->Aorder.resize(nnz); h->Asrc.resize(nnz);
-        for (int i = 0; i < nnz; i++) { h->Aorder[i] = i; h->Asrc[i] = i; }
-        h->A_init.clear();
-        int rc = finish_structure_A(h);
-        return rc ? rc : nnz;
-    } else if (which == SQPB200_MAT_H) {
-        h->zH = nnz; h->zHt = nnz;
-        h->qH.set = false;
-        h->Hp.assign(colptr, colptr + h->nV + 1); h->Hi.assign(rowidx, rowidx + nnz);
-        h->Horder.resize(nnz); h->Hsrc.resize(nnz);
-        for (int i = 0; i < nnz; i++) { h->Horder[i] = i; h->Hsrc[i] = i; }
-        int rc = 0;
-        rc |= upload_vec(h, &h->dHp, h->Hp); rc |= upload_vec(h, &h->dHi, h->Hi); rc |= upload_vec(h, &h->dHsrc, h->Hsrc);
-        if (rc) return SQPB200_ERR_CUDA;
-        if (h->dHval) { CK(cudaFree(h->dHval)); h->dHval = nullptr; }
-        if (dev_alloc(h, &h->dHval, (size_t)h->batch * nnz)) return SQPB200_ERR_CUDA;
-        h->H_set = true;
-        h->cfg_cap_key = -1;
-        return nnz;
-    }
-    return SQPB200_ERR_INVALID;
+    return set_direct(h, which, nnz, colptr, rowidx, false);
 }
 
 int sqpb200_get_structure(sqpb200_handle h, int which, int* colptr, int* rowidx, int* order) {
     if (!h) return SQPB200_ERR_INVALID;
-    const std::vector<int>& P = which == SQPB200_MAT_A ? h->Ap : h->Hp;
-    const std::vector<int>& I = which == SQPB200_MAT_A ? h->Ai : h->Hi;
-    const std::vector<int>& O = which == SQPB200_MAT_A ? h->Aorder : h->Horder;
-    if (P.empty()) return SQPB200_ERR_STATE;
-    if (colptr) std::copy(P.begin(), P.end(), colptr);
-    if (rowidx) std::copy(I.begin(), I.end(), rowidx);
-    if (order) std::copy(O.begin(), O.end(), order);
+    const SparseMat& M = mat(h, which);
+    if (M.p.empty()) return SQPB200_ERR_STATE;
+    if (colptr) std::copy(M.p.begin(), M.p.end(), colptr);
+    if (rowidx) std::copy(M.i.begin(), M.i.end(), rowidx);
+    if (order) std::copy(M.order.begin(), M.order.end(), order);
     return 0;
 }
 
 int sqpb200_get_nnz(sqpb200_handle h, int which) {
     if (!h) return SQPB200_ERR_INVALID;
-    return which == SQPB200_MAT_A ? h->zA : h->zH;
+    return mat(h, which).z;
 }
 
 // ------------------------------------------------------------------------------ batched Vector operations (row A2)
@@ -547,55 +615,72 @@ int sqpb200_vector_elementwise(int device, int op, long long batch, int n, doubl
 }
 
 // ------------------------------------------------------------------------------ values
-static int set_values(sqpb200_handle h, int which, const double* vals, int loc, int broadcast, bool csc_order) {
-    if (!h || !vals) return SQPB200_ERR_INVALID;
+// Values of A or H into their compressed-column storage, rows of zin entries per instance (broadcast: one row for every
+// instance).  With a map, out[b][position] = in[b][map[position]] and positions that map to -1 keep their value (triplet order:
+// the source map of the structure; compressed-row order: c2q).  Without one the input is already in storage order.
+static int set_values(sqpb200_handle h, int which, const double* vals, int loc, int broadcast, const int* map, int zin) {
+    if (!vals) return SQPB200_ERR_INVALID;
     CK(cudaSetDevice(h->device));
-    bool isA = which == SQPB200_MAT_A;
-    if (isA ? !h->A_set : !h->H_set) { h->err = "structure not set"; return SQPB200_ERR_STATE; }
-    int z_out = isA ? h->zA : h->zH;
-    int z_in = csc_order ? z_out : (isA ? h->zJ : h->zHt);
-    if (z_out == 0 || z_in == 0) {  // empty matrix: nothing to copy, but the call still raises Update_A / Update_H (:407-409, 427-429)
+    const bool isA = which == SQPB200_MAT_A;
+    SparseMat& M = mat(h, which);
+    if (!M.set) { h->err = "structure not set"; return SQPB200_ERR_STATE; }
+    if (M.z == 0 || zin == 0) {  // empty matrix: nothing to copy, but the call still raises Update_A / Update_H (:407-409, 427-429)
         if (h->first_solved) { if (isA) h->upd_A = true; else h->upd_H = true; }
         return 0;
     }
-    size_t bytes = (size_t)(broadcast ? 1 : h->batch) * z_in * 8;
-    double* dout = isA ? h->dAval : h->dHval;
-    long long total = (long long)h->batch * z_out;
-    if (csc_order && !broadcast) {
+    size_t bytes = (size_t)(broadcast ? 1 : h->batch) * zin * 8;
+    long long total = (long long)h->batch * M.z;
+    if (!map && !broadcast) {
         // one DMA copy straight into place (no staging, no SM-side copy: it must not queue behind resident solve CTAs)
-        CK(cudaMemcpyAsync(dout, vals, bytes, loc == SQPB200_LOC_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, h->stream));
+        CK(cudaMemcpyAsync(M.dval, vals, bytes, loc == SQPB200_LOC_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, h->stream));
         if (h->first_solved) { if (isA) h->upd_A = true; else h->upd_H = true; }
         return 0;
     }
     if (loc == SQPB200_LOC_HOST && ensure_stage(h, bytes)) return SQPB200_ERR_CUDA;
     const void* din;
     if (to_device(h, vals, bytes, loc, 0, &din)) return SQPB200_ERR_CUDA;
-    if (csc_order) {
-        broadcast_rows_kernel<<<grid_for(total, 256), 256, 0, h->stream>>>(total, z_out, 0, z_out, (const double*)din, dout);
-        h->launches++;
-    } else {
-        scatter_values_kernel<<<grid_for(total, 256), 256, 0, h->stream>>>(total, z_in, z_out, isA ? h->dAsrc : h->dHsrc,
-                                                                           (const double*)din, broadcast, dout);
-        h->launches++;
-    }
+    if (!map) broadcast_rows_kernel<<<grid_for(total, 256), 256, 0, h->stream>>>(total, M.z, 0, M.z, (const double*)din, M.dval);
+    else scatter_values_kernel<<<grid_for(total, 256), 256, 0, h->stream>>>(total, zin, M.z, map, (const double*)din, broadcast, M.dval);
+    h->launches++;
     CK(cudaGetLastError());
     // change flags: src/qpOASESInterface.cpp:407-409, 427-429
     if (h->first_solved) { if (isA) h->upd_A = true; else h->upd_H = true; }
     return 0;
 }
 
-int sqpb200_set_values_A(sqpb200_handle h, const double* vals, int loc, int broadcast) { return set_values(h, SQPB200_MAT_A, vals, loc, broadcast, false); }
-int sqpb200_set_values_H(sqpb200_handle h, const double* vals, int loc, int broadcast) { return set_values(h, SQPB200_MAT_H, vals, loc, broadcast, false); }
-int sqpb200_set_values_csc(sqpb200_handle h, int which, const double* vals, int loc, int broadcast) { return set_values(h, which, vals, loc, broadcast, true); }
+int sqpb200_set_values_A(sqpb200_handle h, const double* vals, int loc, int broadcast) {
+    return h ? set_values(h, SQPB200_MAT_A, vals, loc, broadcast, h->A.dsrc, h->A.zin) : SQPB200_ERR_INVALID;
+}
+int sqpb200_set_values_H(sqpb200_handle h, const double* vals, int loc, int broadcast) {
+    return h ? set_values(h, SQPB200_MAT_H, vals, loc, broadcast, h->H.dsrc, h->H.zin) : SQPB200_ERR_INVALID;
+}
+int sqpb200_set_values_csc(sqpb200_handle h, int which, const double* vals, int loc, int broadcast) {
+    return h ? set_values(h, which, vals, loc, broadcast, nullptr, mat(h, which).z) : SQPB200_ERR_INVALID;
+}
 
-int sqpb200_get_values_csc(sqpb200_handle h, int which, double* vals, int loc) {
-    if (!h || !vals) return SQPB200_ERR_INVALID;
+// vals[batch][z] of A or H in compressed-column storage order (map: none) or in another order, vals[b][e] = value[b][map[e]]
+static int get_values(sqpb200_handle h, int which, double* vals, int loc, const int* map) {
     CK(cudaSetDevice(h->device));
-    bool isA = which == SQPB200_MAT_A;
-    size_t bytes = (size_t)h->batch * (isA ? h->zA : h->zH) * 8;
-    CK(cudaMemcpyAsync(vals, isA ? h->dAval : h->dHval, bytes, loc == SQPB200_LOC_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, h->stream));
+    const SparseMat& M = mat(h, which);
+    if (M.z == 0) return 0;
+    const size_t bytes = (size_t)h->batch * M.z * 8;
+    if (!map) {
+        CK(cudaMemcpyAsync(vals, M.dval, bytes, loc == SQPB200_LOC_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, h->stream));
+    } else {
+        double* dout = vals;
+        if (loc == SQPB200_LOC_HOST) { if (ensure_stage(h, bytes)) return SQPB200_ERR_CUDA; dout = (double*)h->stage; }
+        const long long total = (long long)h->batch * M.z;
+        scatter_values_kernel<<<grid_for(total, 256), 256, 0, h->stream>>>(total, M.z, M.z, map, M.dval, 0, dout);
+        h->launches++;
+        CK(cudaGetLastError());
+        if (loc == SQPB200_LOC_HOST) CK(cudaMemcpyAsync(vals, dout, bytes, cudaMemcpyDeviceToHost, h->stream));
+    }
     CK(cudaStreamSynchronize(h->stream));
     return 0;
+}
+
+int sqpb200_get_values_csc(sqpb200_handle h, int which, double* vals, int loc) {
+    return h && vals ? get_values(h, which, vals, loc, nullptr) : SQPB200_ERR_INVALID;
 }
 
 // ------------------------------------------------------------------------------ vectors
@@ -672,7 +757,6 @@ int sqpb200_qphandler_bounds(sqpb200_handle h, int mode, int n, int m, const dou
         (const double*)dcu, (const double*)dck, h->dlb, h->dub, h->dlbA, h->dubA);
     h->launches++;
     CK(cudaGetLastError());
-    if (mode == 0 && m == 0) { /* nothing else */ }
     if (h->first_solved) h->upd_bounds = true;
     return 0;
 }
@@ -698,7 +782,7 @@ static void fill_dims(sqpb200_handle h, QPKernelArgs& a, int cap) {
     memset(&a, 0, sizeof a);
     a.batch = h->batch; a.nV = h->nV; a.nC = h->nC; a.cap = cap; a.large = h->large ? 1 : 0;
     a.is_lp = (h->qptype == SQPB200_LP); a.has_H = !a.is_lp;
-    a.zA = h->zA; a.zH = a.is_lp ? 0 : h->zH;  // an LP handle never holds H (src/qpOASESInterface.cpp:122-124)
+    a.zA = h->A.z; a.zH = a.is_lp ? 0 : h->H.z;  // an LP handle never holds H (src/qpOASESInterface.cpp:122-124)
     qp_fill_layout(a);
 }
 
@@ -759,7 +843,7 @@ static int choose_config(sqpb200_handle h) {
     if (cap < 0 || cap > nV) cap = nV;
     if (cap == h->cfg_cap_key && h->team != 0) return 0;  // configuration already chosen for this capacity
     h->cfg_cap_key = cap;
-    const bool fits16 = h->zA < 32768 && h->zH < 32768;
+    const bool fits16 = h->A.z < 32768 && h->H.z < 32768;
     h->large = (h->opt.team_size == 1024);
     if (!h->large) {
         h->have_rescue = fits16 && config_for_cap(h, nV, h->cfg_rescue);
@@ -803,20 +887,14 @@ static int prepare_large(sqpb200_handle h, const QPKernelArgs& a) {
     }
     if (!h->dgpat) {
         std::vector<int> pat((size_t)a.pat_shorts + 4, 0);
-        std::vector<int> Arp(h->nC + 1, 0), Aci(h->zA), Aperm(h->zA);
-        for (int e = 0; e < h->zA; e++) Arp[h->Ai[e] + 1]++;
-        for (int r = 0; r < h->nC; r++) Arp[r + 1] += Arp[r];
-        std::vector<int> fill(Arp.begin(), Arp.end() - 1);
-        for (int c = 0; c < h->nV; c++)
-            for (int e = h->Ap[c]; e < h->Ap[c + 1]; e++) { int r = h->Ai[e]; Aci[fill[r]] = c; Aperm[fill[r]] = e; fill[r]++; }
-        std::copy(h->Ap.begin(), h->Ap.end(), pat.begin() + a.pAp);
-        std::copy(h->Ai.begin(), h->Ai.end(), pat.begin() + a.pAi);
-        std::copy(Arp.begin(), Arp.end(), pat.begin() + a.pArp);
-        std::copy(Aci.begin(), Aci.end(), pat.begin() + a.pAci);
-        std::copy(Aperm.begin(), Aperm.end(), pat.begin() + a.pAperm);
+        std::copy(h->A.p.begin(), h->A.p.end(), pat.begin() + a.pAp);
+        std::copy(h->A.i.begin(), h->A.i.end(), pat.begin() + a.pAi);
+        std::copy(h->Arp.begin(), h->Arp.end(), pat.begin() + a.pArp);
+        std::copy(h->Aci.begin(), h->Aci.end(), pat.begin() + a.pAci);
+        std::copy(h->Aperm.begin(), h->Aperm.end(), pat.begin() + a.pAperm);
         if (a.zH > 0) {
-            std::copy(h->Hp.begin(), h->Hp.end(), pat.begin() + a.pHp);
-            std::copy(h->Hi.begin(), h->Hi.end(), pat.begin() + a.pHi);
+            std::copy(h->H.p.begin(), h->H.p.end(), pat.begin() + a.pHp);
+            std::copy(h->H.i.begin(), h->H.i.end(), pat.begin() + a.pHi);
         }
         if (upload_vec(h, &h->dgpat, pat)) return SQPB200_ERR_CUDA;
     }
@@ -855,8 +933,8 @@ int sqpb200_device_buffers(sqpb200_handle h, void** out) {
 int sqpb200_solve_prepare(sqpb200_handle h) {
     if (!h) return SQPB200_ERR_INVALID;
     CK(cudaSetDevice(h->device));
-    if (!h->A_set) { h->err = "set_structure_A has not been called"; return SQPB200_ERR_STATE; }
-    if (h->qptype == SQPB200_QP && !h->H_set) { h->err = "set_structure_H has not been called"; return SQPB200_ERR_STATE; }
+    if (!h->A.set) { h->err = "set_structure_A has not been called"; return SQPB200_ERR_STATE; }
+    if (h->qptype == SQPB200_QP && !h->H.set) { h->err = "set_structure_H has not been called"; return SQPB200_ERR_STATE; }
     int rc = choose_config(h);
     if (rc) return rc;
     if (!h->large && h->opt.keep_state && !h->dstate) {
@@ -903,9 +981,9 @@ static int solve_impl(sqpb200_handle h, int mode_qp, int maxiter, const unsigned
               (h->opt.enable_drift ? FLAG_DRIFT : 0) | (h->opt.keep_state ? FLAG_KEEP_STATE : 0) |
               (h->opt.debug_force_error_branch ? FLAG_FORCE_GUESS : 0) | (h->opt.refactorise_every == 1 ? FLAG_NO_CARRY : 0);
     a.mode = mode;
-    a.Ap = h->dAp; a.Ai = h->dAi; a.Arp = h->dArp; a.Aci = h->dAci; a.Aperm = h->dAperm;
-    a.Hp = h->dHp; a.Hi = h->dHi;
-    a.Aval = h->dAval; a.Hval = h->dHval;
+    a.Ap = h->A.dp; a.Ai = h->A.di; a.Arp = h->dArp; a.Aci = h->dAci; a.Aperm = h->dAperm;
+    a.Hp = h->H.dp; a.Hi = h->H.di;
+    a.Aval = h->A.dval; a.Hval = h->H.dval;
     a.gN = h->dg; a.lbN = h->dlb; a.ubN = h->dub; a.lbAN = h->dlbA; a.ubAN = h->dubA;
     if (active_mask && mask_on_device) a.mask = active_mask;
     else if (active_mask) {
@@ -977,13 +1055,13 @@ int sqpb200_solve_host(sqpb200_handle h, int mode, int maxiter, const void* in_b
         if (h->first_solved) { h->upd_g = true; h->upd_bounds = true; }
     }
     if (Aval_csc) {
-        if (!h->A_set) { h->err = "structure not set"; return SQPB200_ERR_STATE; }
-        if (h->zA > 0) CK(cudaMemcpyAsync(h->dAval, Aval_csc, (size_t)h->batch * h->zA * 8, cudaMemcpyHostToDevice, h->stream));
+        if (!h->A.set) { h->err = "structure not set"; return SQPB200_ERR_STATE; }
+        if (h->A.z > 0) CK(cudaMemcpyAsync(h->A.dval, Aval_csc, (size_t)h->batch * h->A.z * 8, cudaMemcpyHostToDevice, h->stream));
         if (h->first_solved) h->upd_A = true;
     }
     if (Hval_csc) {
-        if (!h->H_set) { h->err = "structure not set"; return SQPB200_ERR_STATE; }
-        if (h->zH > 0) CK(cudaMemcpyAsync(h->dHval, Hval_csc, (size_t)h->batch * h->zH * 8, cudaMemcpyHostToDevice, h->stream));
+        if (!h->H.set) { h->err = "structure not set"; return SQPB200_ERR_STATE; }
+        if (h->H.z > 0) CK(cudaMemcpyAsync(h->H.dval, Hval_csc, (size_t)h->batch * h->H.z * 8, cudaMemcpyHostToDevice, h->stream));
         if (h->first_solved) h->upd_H = true;
     }
     int rc = solve_impl(h, mode, maxiter, nullptr, false, nullptr);
@@ -1072,13 +1150,13 @@ int sqpb200_kkt_residuals(sqpb200_handle h, double* out, int loc) {
 int sqpb200_kkt_residuals_recompute(sqpb200_handle h, double* out, int loc) {
     if (!h || !out) return SQPB200_ERR_INVALID;
     CK(cudaSetDevice(h->device));
-    if (!h->A_set) return SQPB200_ERR_STATE;
+    if (!h->A.set) return SQPB200_ERR_STATE;
     KKTArgs a;
     memset(&a, 0, sizeof a);
-    a.batch = h->batch; a.nV = h->nV; a.nC = h->nC; a.zA = h->zA; a.zH = h->zH;
-    a.has_H = (h->qptype == SQPB200_QP && h->H_set) ? 1 : 0;
-    a.Ap = h->dAp; a.Ai = h->dAi; a.Arp = h->dArp; a.Aci = h->dAci; a.Aperm = h->dAperm; a.Hp = h->dHp; a.Hi = h->dHi;
-    a.Aval = h->dAval; a.Hval = h->dHval; a.g = h->dg; a.lb = h->dlb; a.ub = h->dub; a.lbA = h->dlbA; a.ubA = h->dubA;
+    a.batch = h->batch; a.nV = h->nV; a.nC = h->nC; a.zA = h->A.z; a.zH = h->H.z;
+    a.has_H = (h->qptype == SQPB200_QP && h->H.set) ? 1 : 0;
+    a.Ap = h->A.dp; a.Ai = h->A.di; a.Arp = h->dArp; a.Aci = h->dAci; a.Aperm = h->dAperm; a.Hp = h->H.dp; a.Hi = h->H.di;
+    a.Aval = h->A.dval; a.Hval = h->H.dval; a.g = h->dg; a.lb = h->dlb; a.ub = h->dub; a.lbA = h->dlbA; a.ubA = h->dubA;
     a.x = h->dx; a.y = h->dy; a.wsB = h->dwsB; a.wsC = h->dwsC; a.WB = h->dWB; a.WC = h->dWC;
     if (ensure_stage(h, (size_t)h->batch * 5 * 8)) return SQPB200_ERR_CUDA;
     a.out = (loc == SQPB200_LOC_DEVICE) ? out : (double*)h->stage;
@@ -1088,12 +1166,12 @@ int sqpb200_kkt_residuals_recompute(sqpb200_handle h, double* out, int loc) {
         const bool aligned = (((uintptr_t)a.Aval | (uintptr_t)a.Hval | (uintptr_t)a.x | (uintptr_t)a.y | (uintptr_t)a.g | (uintptr_t)a.lb |
                                (uintptr_t)a.ub | (uintptr_t)a.lbA | (uintptr_t)a.ubA) & 15) == 0;
         // (G warps per CTA, stages) that keeps the most warps resident per SM; ties go to two stages
-        const int zHk = a.has_H ? h->zH : 0;
+        const int zHk = a.has_H ? h->H.z : 0;
         int G = 0, stages = 0, best_warps = 0;
         size_t smem_t = 0;
         for (int st = 2; st >= 1 && aligned; st--)
             for (int g = 8; g >= 2; g >>= 1) {
-                KKTLayout Lg = kkt_layout(g, st, h->nV, h->nC, h->zA, zHk);
+                KKTLayout Lg = kkt_layout(g, st, h->nV, h->nC, h->A.z, zHk);
                 size_t sm = kkt_smem_bytes(Lg);
                 if (sm > 227 * 1024) continue;
                 int ctas = (int)((228 * 1024) / (sm + 1024));
@@ -1104,7 +1182,7 @@ int sqpb200_kkt_residuals_recompute(sqpb200_handle h, double* out, int loc) {
         if (G) {
             KKTArgs at = a;
             if (!at.has_H) at.zH = 0;
-            KKTLayout Lg = kkt_layout(G, stages, h->nV, h->nC, h->zA, at.zH);
+            KKTLayout Lg = kkt_layout(G, stages, h->nV, h->nC, h->A.z, at.zH);
             if (smem_t > 48 * 1024) CK(cudaFuncSetAttribute(kkt_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_t));
             long long ngroups = ((long long)h->batch + G - 1) / G;
             int per_sm = (int)((228 * 1024) / (smem_t + 1024));
@@ -1119,7 +1197,7 @@ int sqpb200_kkt_residuals_recompute(sqpb200_handle h, double* out, int loc) {
             return 0;
         }
     }
-    const size_t per_warp = kkt_warp_doubles(h->nV, h->nC, h->zA, h->zH) * 8;
+    const size_t per_warp = kkt_warp_doubles(h->nV, h->nC, h->A.z, h->H.z) * 8;
     int warps = 4;
     while (warps > 1 && (size_t)warps * per_warp > 24 * 1024) warps >>= 1;
     size_t smem = (size_t)warps * per_warp;
@@ -1137,13 +1215,13 @@ int sqpb200_spmv(sqpb200_handle h, int which, int transpose, const double* x, do
     if (!h || !x || !y) return SQPB200_ERR_INVALID;
     CK(cudaSetDevice(h->device));
     bool isA = which == SQPB200_MAT_A;
-    if (isA ? !h->A_set : !h->H_set) return SQPB200_ERR_STATE;
+    if (isA ? !h->A.set : !h->H.set) return SQPB200_ERR_STATE;
     int nin, nout, nnz;
     const int *ptr, *idx, *perm;
     const double* val;
-    if (isA && !transpose) { nin = h->nV; nout = h->nC; nnz = h->zA; ptr = h->dArp; idx = h->dAci; perm = h->dAperm; val = h->dAval; }
-    else if (isA) { nin = h->nC; nout = h->nV; nnz = h->zA; ptr = h->dAp; idx = h->dAi; perm = nullptr; val = h->dAval; }
-    else { nin = h->nV; nout = h->nV; nnz = h->zH; ptr = h->dHp; idx = h->dHi; perm = nullptr; val = h->dHval; }
+    if (isA && !transpose) { nin = h->nV; nout = h->nC; nnz = h->A.z; ptr = h->dArp; idx = h->dAci; perm = h->dAperm; val = h->A.dval; }
+    else if (isA) { nin = h->nC; nout = h->nV; nnz = h->A.z; ptr = h->A.dp; idx = h->A.di; perm = nullptr; val = h->A.dval; }
+    else { nin = h->nV; nout = h->nV; nnz = h->H.z; ptr = h->H.dp; idx = h->H.di; perm = nullptr; val = h->H.dval; }
     size_t B = h->batch, bin = B * nin * 8, bout = B * nout * 8;
     if (nout == 0) return 0;
     const void* dxv = x;
@@ -1202,138 +1280,24 @@ __global__ void qore_workingset_kernel(long long total, int nV, int nC, const si
     }
 }
 
-// compressed-row (rp, ci) -> compressed-column (cp, ri) plus the position map q2c; entries with equal keys keep their order
-static void csr_to_csc(int nrow, int ncol, const std::vector<int>& rp, const std::vector<int>& ci, std::vector<int>& cp,
-                       std::vector<int>& ri, std::vector<int>& q2c) {
-    const int z = (int)ci.size();
-    cp.assign(ncol + 1, 0); ri.assign(z, 0); q2c.assign(z, 0);
-    for (int e = 0; e < z; e++) cp[ci[e] + 1]++;
-    for (int c = 0; c < ncol; c++) cp[c + 1] += cp[c];
-    std::vector<int> fill(cp.begin(), cp.end() - 1);
-    for (int r = 0; r < nrow; r++)
-        for (int e = rp[r]; e < rp[r + 1]; e++) { const int pos = fill[ci[e]]++; ri[pos] = r; q2c[e] = pos; }
-}
-
-static int finish_csr_view(sqpb200_handle h, sqpb200_handle_s::CsrView& q) {
-    const int z = (int)q.ci.size();
-    q.c2q.assign(z, 0);
-    for (int e = 0; e < z; e++) q.c2q[q.q2c[e]] = e;
-    if (upload_vec(h, &q.dq2c, q.q2c) || upload_vec(h, &q.dc2q, q.c2q)) return SQPB200_ERR_CUDA;
-    q.set = true;
-    return 0;
-}
-
-static int finish_structure_H(sqpb200_handle h) {
-    int rc = 0;
-    rc |= upload_vec(h, &h->dHp, h->Hp); rc |= upload_vec(h, &h->dHi, h->Hi); rc |= upload_vec(h, &h->dHsrc, h->Hsrc);
-    if (rc) return SQPB200_ERR_CUDA;
-    if (h->dHval) { CK(cudaFree(h->dHval)); h->dHval = nullptr; }
-    if (dev_alloc(h, &h->dHval, (size_t)h->batch * h->zH)) return SQPB200_ERR_CUDA;
-    h->H_set = true;
-    h->cfg_cap_key = -1;
-    return 0;
-}
-
 int sqpb200_set_structure_A_csr(sqpb200_handle h, int zJ, const int* row1, const int* col1, int I_len, const int* I_irow,
                                 const int* I_jcol, const int* I_size, const double* I_value) {
     if (!h || zJ < 0) return SQPB200_ERR_INVALID;
-    CK(cudaSetDevice(h->device));
-    // entry list of SpHbMat::setStructure(rhs, I_info), src/SpHbMat.cpp:203-227
-    std::vector<int> er, ec;
-    std::vector<double> ev;
-    for (int i = 0; i < zJ; i++) { er.push_back(row1[i]); ec.push_back(col1[i]); ev.push_back(0.0); }
-    for (int b = 0; b < I_len; b++)
-        for (int j = 0; j < I_size[b]; j++) { er.push_back(I_irow[b] + j); ec.push_back(I_jcol[b] + j); ev.push_back(I_value[b]); }
-    const int z = (int)er.size();
-    for (int i = 0; i < z; i++)
-        if (er[i] < 1 || er[i] > h->nC || ec[i] < 1 || ec[i] > h->nV) { h->err = "triplet index out of range"; return SQPB200_ERR_INVALID; }
-    if (h->nV >= (1 << 21)) { h->err = "matrix too large for packed keys"; return SQPB200_ERR_TOO_LARGE; }
-    // compressed-row branch (:238-250): the device sort with the roles of row and column exchanged, key (row, column, counter)
-    auto& q = h->qA;
-    q.rp.assign(h->nC + 1, 0); q.ci.assign(z, 0); q.order.assign(z, 0);
-    int seg[2] = {0, z}, nrow[1] = {h->nC};
-    if (z > 0) {
-        int rc = run_assembly(h, h->stream, 1, seg, nrow, ec.data(), er.data(), q.rp.data(), q.ci.data(), q.order.data(), nullptr, &h->err);
-        h->launches++;
-        if (rc) return rc;
-    }
-    h->zA = z; h->zJ = zJ;
-    csr_to_csc(h->nC, h->nV, q.rp, q.ci, h->Ap, h->Ai, q.q2c);
-    h->Aorder.assign(z, 0); h->Asrc.assign(z, -1); h->A_init.assign(z, 0.0);
-    for (int i = 0; i < z; i++) {
-        h->Aorder[i] = q.q2c[q.order[i]];
-        if (i < zJ) h->Asrc[h->Aorder[i]] = i;
-        else h->A_init[h->Aorder[i]] = ev[i];
-    }
-    int rc = finish_structure_A(h);
-    if (!rc) rc = finish_csr_view(h, q);
-    return rc ? rc : z;
+    return set_triplets(h, SQPB200_MAT_A, entries_A(zJ, row1, col1, I_len, I_irow, I_jcol, I_size, I_value), zJ, true);
 }
 
 int sqpb200_set_structure_H_csr(sqpb200_handle h, int zH, const int* row1, const int* col1, int is_symmetric) {
     if (!h || zH < 0) return SQPB200_ERR_INVALID;
-    CK(cudaSetDevice(h->device));
-    // entry list of SpHbMat::setStructure(rhs), src/SpHbMat.cpp:296-309
-    std::vector<int> er, ec, srct;
-    for (int i = 0; i < zH; i++) {
-        er.push_back(row1[i]); ec.push_back(col1[i]); srct.push_back(i);
-        if (is_symmetric && row1[i] != col1[i]) { er.push_back(col1[i]); ec.push_back(row1[i]); srct.push_back(i); }
-    }
-    const int z = (int)er.size();
-    for (int i = 0; i < z; i++)
-        if (er[i] < 1 || er[i] > h->nV || ec[i] < 1 || ec[i] > h->nV) { h->err = "triplet index out of range"; return SQPB200_ERR_INVALID; }
-    if (h->nV >= (1 << 21)) { h->err = "matrix too large for packed keys"; return SQPB200_ERR_TOO_LARGE; }
-    auto& q = h->qH;
-    q.rp.assign(h->nV + 1, 0); q.ci.assign(z, 0); q.order.assign(z, 0);
-    int seg[2] = {0, z}, nrow[1] = {h->nV};
-    if (z > 0) {  // compressed-row branch (:324-337)
-        int rc = run_assembly(h, h->stream, 1, seg, nrow, ec.data(), er.data(), q.rp.data(), q.ci.data(), q.order.data(), nullptr, &h->err);
-        h->launches++;
-        if (rc) return rc;
-    }
-    h->zH = z; h->zHt = zH;
-    csr_to_csc(h->nV, h->nV, q.rp, q.ci, h->Hp, h->Hi, q.q2c);
-    h->Horder.assign(z, 0); h->Hsrc.assign(z, -1);
-    for (int i = 0; i < z; i++) { h->Horder[i] = q.q2c[q.order[i]]; h->Hsrc[h->Horder[i]] = srct[i]; }
-    int rc = finish_structure_H(h);
-    if (!rc) rc = finish_csr_view(h, q);
-    return rc ? rc : z;
+    return set_triplets(h, SQPB200_MAT_H, entries_H(zH, row1, col1, is_symmetric), zH, true);
 }
 
 int sqpb200_set_structure_csr(sqpb200_handle h, int which, int nnz, const int* rowptr, const int* colidx) {
-    if (!h || nnz < 0 || !rowptr || (nnz > 0 && !colidx) || (which != SQPB200_MAT_A && which != SQPB200_MAT_H)) return SQPB200_ERR_INVALID;
-    CK(cudaSetDevice(h->device));
-    const bool isA = which == SQPB200_MAT_A;
-    const int nrow = isA ? h->nC : h->nV;
-    if (rowptr[0] != 0 || rowptr[nrow] != nnz) { h->err = "rowptr[0] != 0 or rowptr[nrow] != nnz"; return SQPB200_ERR_INVALID; }
-    for (int r = 0; r < nrow; r++)
-        if (rowptr[r + 1] < rowptr[r]) { h->err = "rowptr not monotone"; return SQPB200_ERR_INVALID; }
-    for (int e = 0; e < nnz; e++)
-        if (colidx[e] < 0 || colidx[e] >= h->nV) { h->err = "column index out of range"; return SQPB200_ERR_INVALID; }
-    auto& q = isA ? h->qA : h->qH;
-    q.rp.assign(rowptr, rowptr + nrow + 1); q.ci.assign(colidx, colidx + nnz); q.order.resize(nnz);
-    for (int e = 0; e < nnz; e++) q.order[e] = e;
-    int rc;
-    if (isA) {
-        h->zA = nnz; h->zJ = nnz;
-        csr_to_csc(nrow, h->nV, q.rp, q.ci, h->Ap, h->Ai, q.q2c);
-        h->Aorder = q.q2c; h->Asrc.assign(nnz, 0); h->A_init.clear();
-        for (int e = 0; e < nnz; e++) h->Asrc[q.q2c[e]] = e;
-        rc = finish_structure_A(h);
-    } else {
-        h->zH = nnz; h->zHt = nnz;
-        csr_to_csc(nrow, h->nV, q.rp, q.ci, h->Hp, h->Hi, q.q2c);
-        h->Horder = q.q2c; h->Hsrc.assign(nnz, 0);
-        for (int e = 0; e < nnz; e++) h->Hsrc[q.q2c[e]] = e;
-        rc = finish_structure_H(h);
-    }
-    if (!rc) rc = finish_csr_view(h, q);
-    return rc ? rc : nnz;
+    return set_direct(h, which, nnz, rowptr, colidx, true);
 }
 
 int sqpb200_get_structure_csr(sqpb200_handle h, int which, int* rowptr, int* colidx, int* order) {
     if (!h) return SQPB200_ERR_INVALID;
-    const auto& q = which == SQPB200_MAT_A ? h->qA : h->qH;
+    const CsrView& q = mat(h, which).q;
     if (!q.set) { h->err = "structure was not given in compressed-row form"; return SQPB200_ERR_STATE; }
     if (rowptr) std::copy(q.rp.begin(), q.rp.end(), rowptr);
     if (colidx) std::copy(q.ci.begin(), q.ci.end(), colidx);
@@ -1343,45 +1307,16 @@ int sqpb200_get_structure_csr(sqpb200_handle h, int which, int* rowptr, int* col
 
 int sqpb200_set_values_csr(sqpb200_handle h, int which, const double* vals, int loc, int broadcast) {
     if (!h || !vals) return SQPB200_ERR_INVALID;
-    CK(cudaSetDevice(h->device));
-    const bool isA = which == SQPB200_MAT_A;
-    const auto& q = isA ? h->qA : h->qH;
-    if (!q.set || (isA ? !h->A_set : !h->H_set)) { h->err = "structure was not given in compressed-row form"; return SQPB200_ERR_STATE; }
-    const int z = isA ? h->zA : h->zH;
-    if (z > 0) {
-        const size_t bytes = (size_t)(broadcast ? 1 : h->batch) * z * 8;
-        if (loc == SQPB200_LOC_HOST && ensure_stage(h, bytes)) return SQPB200_ERR_CUDA;
-        const void* din;
-        if (to_device(h, vals, bytes, loc, 0, &din)) return SQPB200_ERR_CUDA;
-        const long long total = (long long)h->batch * z;
-        // out[b][compressed-column position] = in[b][c2q[position]]
-        scatter_values_kernel<<<grid_for(total, 256), 256, 0, h->stream>>>(total, z, z, q.dc2q, (const double*)din, broadcast,
-                                                                           isA ? h->dAval : h->dHval);
-        h->launches++;
-        CK(cudaGetLastError());
-    }
-    if (h->first_solved) { if (isA) h->upd_A = true; else h->upd_H = true; }
-    return 0;
+    const SparseMat& M = mat(h, which);
+    if (!M.q.set) { h->err = "structure was not given in compressed-row form"; return SQPB200_ERR_STATE; }
+    return set_values(h, which, vals, loc, broadcast, M.dc2q, M.z);
 }
 
 int sqpb200_get_values_csr(sqpb200_handle h, int which, double* vals, int loc) {
     if (!h || !vals) return SQPB200_ERR_INVALID;
-    CK(cudaSetDevice(h->device));
-    const bool isA = which == SQPB200_MAT_A;
-    const auto& q = isA ? h->qA : h->qH;
-    if (!q.set) { h->err = "structure was not given in compressed-row form"; return SQPB200_ERR_STATE; }
-    const int z = isA ? h->zA : h->zH;
-    if (z == 0) return 0;
-    const size_t bytes = (size_t)h->batch * z * 8;
-    double* dout = vals;
-    if (loc == SQPB200_LOC_HOST) { if (ensure_stage(h, bytes)) return SQPB200_ERR_CUDA; dout = (double*)h->stage; }
-    const long long total = (long long)h->batch * z;
-    scatter_values_kernel<<<grid_for(total, 256), 256, 0, h->stream>>>(total, z, z, q.dq2c, isA ? h->dAval : h->dHval, 0, dout);
-    h->launches++;
-    CK(cudaGetLastError());
-    if (loc == SQPB200_LOC_HOST) CK(cudaMemcpyAsync(vals, dout, bytes, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    return 0;
+    const SparseMat& M = mat(h, which);
+    if (!M.q.set) { h->err = "structure was not given in compressed-row form"; return SQPB200_ERR_STATE; }
+    return get_values(h, which, vals, loc, M.dq2c);
 }
 
 int sqpb200_set_bounds_stacked(sqpb200_handle h, const double* lb, const double* ub, int loc, int broadcast) {
@@ -1444,7 +1379,7 @@ int sqpb200_get_solution_stacked(sqpb200_handle h, double* primal, double* dual,
     if (primal) {  // "primalsol" = [x ; A x] (src/QOREInterface.cpp:120; its test_optimality reads x_qp_(nV + i) as the activity)
         CK(cudaMemcpy2DAsync(primal, ld * 8, h->dx, (size_t)nV * 8, (size_t)nV * 8, B, kind, h->stream));
         if (nC > 0) {
-            if (!h->A_set) { h->err = "structure of A not set"; return SQPB200_ERR_STATE; }
+            if (!h->A.set) { h->err = "structure of A not set"; return SQPB200_ERR_STATE; }
             int rc = sqpb200_spmv(h, SQPB200_MAT_A, 0, h->dx, dAx, SQPB200_LOC_DEVICE);
             if (rc) return rc;
             CK(cudaMemcpy2DAsync(primal + nV, ld * 8, dAx, (size_t)nC * 8, (size_t)nC * 8, B, kind, h->stream));
