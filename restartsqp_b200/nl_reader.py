@@ -11,13 +11,12 @@ layer delivers to Algorithm.cpp for the text ("g") .nl format of the Hock-Schitt
 
 All instances of a batch share the model and differ in x, so every evaluation is a straight-line program over
 [batch]-long vectors.  The expression DAG is differentiated symbolically once (first and second order, with constant
-folding so that structural zeros vanish) and emitted as numpy source; `cuda_source()` emits the same straight-line
-program as a CUDA kernel body (one thread per instance) for a device-resident outer loop.
+folding so that structural zeros vanish) and emitted three times from one table of outputs: as numpy source for the host
+mirror, by `cuda_source()` as CUDA kernels (one thread per instance) for a device-resident outer loop, and by `c_source()`
+as C for one instance, the evaluator of the CPU oracle.
 """
 import math
 import os
-
-import re
 
 import numpy as np
 
@@ -462,20 +461,24 @@ class NLModel:
                 raise NotImplementedError("nl segment %r" % ln)
 
 
-_NP_FUN = {"sqrt": "np.sqrt", "sin": "np.sin", "cos": "np.cos", "log": "np.log", "exp": "np.exp", "abs": "np.abs", "tan": "np.tan",
-           "atan": "np.arctan", "tanh": "np.tanh", "sinh": "np.sinh", "cosh": "np.cosh", "log10": "np.log10", "acos": "np.arccos",
-           "asin": "np.arcsin", "ncdf": "_ncdf"}
-_C_FUN = {"abs": "fabs"}
 _INFIX = {"add": "+", "sub": "-", "mul": "*", "div": "/"}
 _CMP_C = {"le": "<=", "lt": "<", "eq": "=="}
 _MATH_NAMES = ("pow", "sqrt", "sin", "cos", "log", "exp", "tan", "atan", "tanh", "sinh", "cosh", "log10", "acos", "asin")
-_MATH_CALL = re.compile(r"(?<![A-Za-z0-9_])(%s)\(" % "|".join(_MATH_NAMES))
+# the functions each dialect of _emit calls (a name missing from a table is called as is); "nl" is C whose transcendental
+# functions go through __noinline__ wrappers (emitted once by cuda_source for the chunked form): inlined, every pow() is a few
+# hundred instructions and the kernels of hs025 / hs105 reach 5 MB of SASS
+_FUN = {"py": {"pow": "np.power", "sqrt": "np.sqrt", "sin": "np.sin", "cos": "np.cos", "log": "np.log", "exp": "np.exp", "abs": "np.abs",
+               "tan": "np.tan", "atan": "np.arctan", "tanh": "np.tanh", "sinh": "np.sinh", "cosh": "np.cosh", "log10": "np.log10",
+               "acos": "np.arccos", "asin": "np.arcsin", "ncdf": "_ncdf"},
+        "c": {"abs": "fabs"}}
+_FUN["nl"] = dict(_FUN["c"], **{f: "nl_" + f for f in _MATH_NAMES})
 _MATH_WRAPPERS = (["static __device__ __noinline__ double nl_pow(double a, double b) { return pow(a, b); }"] +
                   ["static __device__ __noinline__ double nl_%s(double a) { return %s(a); }" % (f, f) for f in _MATH_NAMES if f != "pow"])
 
 
 def _emit(G, roots, lang):
-    """Straight-line code computing the nodes `roots`; returns (lines, name_of(node))."""
+    """Straight-line code computing the nodes `roots` in dialect `lang` ("py", "c" or "nl", see _FUN); returns (lines,
+    name_of(node), the compute nodes in the order of `lines`, the sorted indices of the variables the program reads)."""
     order, seen = [], set()
 
     def visit(a):
@@ -497,17 +500,16 @@ def _emit(G, roots, lang):
 
     for r in roots:
         visit(r)
-    name = {}
-    lines = []
+    py, fun = lang == "py", _FUN[lang]
+    name, lines, compute, xs = {}, [], [], []
     for a in order:
         t = G.nodes[a]
         if t[0] == "const":
-            name[a] = repr(t[1]) if lang == "py" else ("%r" % t[1])
-            if t[1] < 0:
-                name[a] = "(" + name[a] + ")"
+            name[a] = repr(t[1]) if t[1] >= 0 else "(%r)" % t[1]
             continue
         if t[0] == "var":
             name[a] = "x%d" % t[1]
+            xs.append(t[1])
             continue
         nm = "t%d" % a
         if t[0] in _INFIX:
@@ -517,18 +519,19 @@ def _emit(G, roots, lang):
             if ce == 2.0:
                 rhs = "%s * %s" % (name[t[1]], name[t[1]])
             else:
-                rhs = ("np.power(%s, %s)" if lang == "py" else "pow(%s, %s)") % (name[t[1]], name[t[2]])
+                rhs = "%s(%s, %s)" % (fun.get("pow", "pow"), name[t[1]], name[t[2]])
         elif t[0] == "neg":
             rhs = "-%s" % name[t[1]]
         elif t[0] in _CMP_C:
-            rhs = ("(%s %s %s) * 1.0" if lang == "py" else "(%s %s %s ? 1.0 : 0.0)") % (name[t[1]], _CMP_C[t[0]], name[t[2]])
+            rhs = ("(%s %s %s) * 1.0" if py else "(%s %s %s ? 1.0 : 0.0)") % (name[t[1]], _CMP_C[t[0]], name[t[2]])
         elif t[0] == "if":
-            rhs = ("np.where(%s != 0.0, %s, %s)" if lang == "py" else "(%s != 0.0 ? %s : %s)") % (name[t[1]], name[t[2]], name[t[3]])
+            rhs = ("np.where(%s != 0.0, %s, %s)" if py else "(%s != 0.0 ? %s : %s)") % (name[t[1]], name[t[2]], name[t[3]])
         else:
-            rhs = "%s(%s)" % ((_NP_FUN[t[0]] if lang == "py" else _C_FUN.get(t[0], t[0])), name[t[1]])
-        lines.append(("%s = %s" if lang == "py" else "const double %s = %s;") % (nm, rhs))
+            rhs = "%s(%s)" % (fun.get(t[0], t[0]), name[t[1]])
+        lines.append(("%s = %s" if py else "const double %s = %s;") % (nm, rhs))
         name[a] = nm
-    return lines, name
+        compute.append(a)
+    return lines, name, compute, sorted(xs)
 
 
 def _emit_chunked_cuda(G, roots, tag, chunk, n):
@@ -537,13 +540,7 @@ def _emit_chunked_cuda(G, roots, tag, chunk, n):
     kernel: 47 s), while the sum over pieces of a few thousand statements stays linear.  Values that cross a piece boundary go
     through a per-thread scratch array T (local memory); evaluation order and arithmetic are exactly those of the one-piece
     program.  Returns (source lines of the device functions, body lines of the kernel after `b` / bounds check, name_of(root))."""
-    lines, name = _emit(G, roots, "c")
-    # transcendental functions through __noinline__ wrappers (emitted once by cuda_source): inlined, every pow() is a few hundred
-    # instructions and the kernels of hs025 / hs105 reach 5 MB of SASS
-    lines = [_MATH_CALL.sub(lambda mo: "nl_" + mo.group(1) + "(", ln) for ln in lines]
-    order = []  # compute nodes in emission order: _emit names them t<node id>
-    for ln in lines:
-        order.append(int(ln.split()[2][1:]))
+    lines, name, order, _ = _emit(G, roots, "nl")
     pos = {a: i // chunk for i, a in enumerate(order)}
     npieces = (len(order) + chunk - 1) // chunk
     last_use = {}  # node -> last piece that reads it (npieces = the kernel epilogue)
@@ -629,49 +626,37 @@ class AmplNLP:
         self.H_col1 = np.array([j + 1 for j, i in hk], np.int32)
         self.H_row1 = np.array([i + 1 for j, i in hk], np.int32)
         self._hess_terms = [hess[k] for k in hk]
+        # what every evaluator stores, in store order, keyed by the name of the output array (and of the numpy function, eval_<key>):
+        # an entry is a sum of terms (k, node), the node times lam[k-1] when k > 0
+        self._outputs = {"f": [[(0, self.f_node)]], "c": [[(0, a)] for a in self.c_nodes], "grad": [[(0, a)] for a in self.grad_nodes],
+                         "jac": [[(0, a)] for a in self.jac_nodes], "hess": self._hess_terms}
         self._compile()
 
     # ---- code generation
+    def _roots(self, outs):
+        """The nodes the outputs `outs` store, in store order."""
+        return [a for o in outs for terms in self._outputs[o] for _, a in terms]
+
+    def _stores(self, outs, nm, store, lam):
+        """Statements writing the outputs `outs` from the program's values nm: store(output, entry, value) is one statement of
+        the dialect, lam(k) the multiplier of constraint k."""
+        return ["    " + store(o, e, " + ".join(nm[a] if k == 0 else "%s * %s" % (lam(k - 1), nm[a]) for k, a in terms))
+                for o in outs for e, terms in enumerate(self._outputs[o])]
+
     def _compile(self):
-        G, n, m = self.model.G, self.n, self.m
         src = ["import numpy as np", "from scipy.special import ndtr as _ncdf", ""]
-
-        def fun(name, roots, extra_args, body_tail):
-            lines, nm = _emit(G, roots, "py")
-            src.append("def %s(x%s):" % (name, extra_args))
-            src.append("    B = x.shape[0]")
-            for j in range(n):
-                src.append("    x%d = x[:, %d]" % (j, j))
-            for ln in lines:
-                src.append("    " + ln)
-            for ln in body_tail(nm):
-                src.append("    " + ln)
+        store = lambda o, e, v: "return np.zeros(B) + %s" % v if o == "f" else "out[:, %d] = %s" % (e, v)
+        for o, entries in self._outputs.items():
+            lines, nm, _, _ = _emit(self.model.G, self._roots([o]), "py")
+            src += ["def eval_%s(x%s):" % (o, ", lam" if o == "hess" else ""), "    B = x.shape[0]"]
+            src += ["    x%d = x[:, %d]" % (j, j) for j in range(self.n)] + ["    " + ln for ln in lines]
+            stores = self._stores([o], nm, store, lambda k: "lam[:, %d]" % k)
+            src += stores if o == "f" else ["    out = np.empty((B, %d))" % len(entries)] + stores + ["    return out"]
             src.append("")
-
-        full = lambda e: "np.zeros(B) + %s" % e
-        fun("eval_f", [self.f_node], "", lambda nm: ["return %s" % full(nm[self.f_node])])
-        fun("eval_c", self.c_nodes, "", lambda nm: ["out = np.empty((B, %d))" % m] +
-            ["out[:, %d] = %s" % (i, nm[a]) for i, a in enumerate(self.c_nodes)] + ["return out"])
-        fun("eval_grad", self.grad_nodes, "", lambda nm: ["out = np.empty((B, %d))" % n] +
-            ["out[:, %d] = %s" % (i, nm[a]) for i, a in enumerate(self.grad_nodes)] + ["return out"])
-        fun("eval_jac", self.jac_nodes, "", lambda nm: ["out = np.empty((B, %d))" % len(self.jac_nodes)] +
-            ["out[:, %d] = %s" % (i, nm[a]) for i, a in enumerate(self.jac_nodes)] + ["return out"])
-        hroots = [d2 for terms in self._hess_terms for _, d2 in terms]
-
-        def htail(nm):
-            out = ["out = np.empty((B, %d))" % len(self._hess_terms)]
-            for e, terms in enumerate(self._hess_terms):
-                parts = []
-                for k, d2 in terms:
-                    parts.append(nm[d2] if k == 0 else "lam[:, %d] * %s" % (k - 1, nm[d2]))
-                out.append("out[:, %d] = %s" % (e, " + ".join(parts)))
-            return out + ["return out"]
-
-        fun("eval_hess", hroots, ", lam", htail)
         self.source = "\n".join(src)
         ns = {}
         exec(compile(self.source, "<nl:%s>" % self.name, "exec"), ns)
-        self._f, self._c, self._g, self._j, self._h = ns["eval_f"], ns["eval_c"], ns["eval_grad"], ns["eval_jac"], ns["eval_hess"]
+        self._f, self._c, self._g, self._j, self._h = (ns["eval_" + o] for o in self._outputs)
 
     CUDA_PIECE = 1500  # statements per device function of the chunked form (large DAGs)
 
@@ -680,109 +665,48 @@ class AmplNLP:
         nlp_eval_fc (f, c at trial points) and nlp_eval_all (f, c, grad f, Jacobian and Lagrangian-Hessian triplet
         values).  Compiled at run time by sqpb200_nlp_compile (NVRTC, sm_100a, --fmad=false).  Programs longer than `piece`
         statements are cut into __noinline__ device functions of that length (_emit_chunked_cuda)."""
-        G, n, m = self.model.G, self.n, self.m
-        zJ, zH = len(self.jac_nodes), len(self._hess_terms)
-        hroots = [d2 for terms in self._hess_terms for _, d2 in terms]
+        G, n = self.model.G, self.n
         piece = self.CUDA_PIECE if piece is None else piece
-        ncompute = sum(1 for t in G.nodes if t[0] not in ("const", "var"))
-        if ncompute > piece:
-            head = ["    const int b = blockIdx.x * blockDim.x + threadIdx.x;", "    if (b >= B) return;"]
-            f1, b1, n1 = _emit_chunked_cuda(G, [self.f_node] + self.c_nodes, "fc", piece, n)
-            f2, b2, n2 = _emit_chunked_cuda(G, [self.f_node] + self.c_nodes + self.grad_nodes + self.jac_nodes + hroots, "all", piece, n)
-            src = ["// generated by restartsqp_b200/nl_reader.py from %s.nl (chunked: %d statements per device function)" % (self.name, piece)]
-            src += ["static __device__ __forceinline__ double ncdf(double u) { return 0.5 * erfc(-u * 0.7071067811865476); }"]
-            src += _MATH_WRAPPERS + [""] + f1 + f2
-            src += ['extern "C" __global__ void nlp_eval_fc(int B, const double* __restrict__ x, double* __restrict__ f, double* __restrict__ c) {']
-            src += head + b1 + ["    f[b] = %s;" % n1[self.f_node]]
-            src += ["    c[(size_t)b * %d + %d] = %s;" % (m, i, n1[a]) for i, a in enumerate(self.c_nodes)] + ["}", ""]
-            src += ['extern "C" __global__ void nlp_eval_all(int B, const double* __restrict__ x, const double* __restrict__ lam,',
-                    "                                        double* __restrict__ f, double* __restrict__ c, double* __restrict__ grad,",
-                    "                                        double* __restrict__ jac, double* __restrict__ hess) {"]
-            src += head + b2 + ["    f[b] = %s;" % n2[self.f_node]]
-            src += ["    c[(size_t)b * %d + %d] = %s;" % (m, i, n2[a]) for i, a in enumerate(self.c_nodes)]
-            src += ["    grad[(size_t)b * %d + %d] = %s;" % (n, i, n2[a]) for i, a in enumerate(self.grad_nodes)]
-            src += ["    jac[(size_t)b * %d + %d] = %s;" % (zJ, i, n2[a]) for i, a in enumerate(self.jac_nodes)]
-            for e, terms in enumerate(self._hess_terms):
-                parts = [n2[d2] if k == 0 else "lam[(size_t)b * %d + %d] * %s" % (m, k - 1, n2[d2]) for k, d2 in terms]
-                src.append("    hess[(size_t)b * %d + %d] = %s;" % (zH, e, " + ".join(parts)))
-            src.append("}")
-            return "\n".join(src)
-
-        def body(roots):
-            lines, nm = _emit(G, roots, "c")
-            used = set()
-            for r_ in roots:
-                stack = [r_]
-                while stack:
-                    a = stack.pop()
-                    if a in used:
-                        continue
-                    used.add(a)
-                    t = G.nodes[a]
-                    if t[0] not in ("const", "var"):
-                        stack.extend(t[1:])
-            xs = sorted(G.nodes[a][1] for a in used if G.nodes[a][0] == "var")
-            out = ["    const int b = blockIdx.x * blockDim.x + threadIdx.x;", "    if (b >= B) return;"]
-            out += ["    const double x%d = x[(size_t)b * %d + %d];" % (j, n, j) for j in xs]
-            out += ["    " + ln for ln in lines]
-            return out, nm
-
-        src = ["// generated by restartsqp_b200/nl_reader.py from %s.nl" % self.name,
-               "static __device__ __forceinline__ double ncdf(double u) { return 0.5 * erfc(-u * 0.7071067811865476); }",
-               'extern "C" __global__ void nlp_eval_fc(int B, const double* __restrict__ x, double* __restrict__ f, double* __restrict__ c) {']
-        out, nm = body([self.f_node] + self.c_nodes)
-        src += out + ["    f[b] = %s;" % nm[self.f_node]]
-        src += ["    c[(size_t)b * %d + %d] = %s;" % (m, i, nm[a]) for i, a in enumerate(self.c_nodes)] + ["}", ""]
-        src += ['extern "C" __global__ void nlp_eval_all(int B, const double* __restrict__ x, const double* __restrict__ lam,',
-                "                                        double* __restrict__ f, double* __restrict__ c, double* __restrict__ grad,",
-                "                                        double* __restrict__ jac, double* __restrict__ hess) {"]
-        out, nm = body([self.f_node] + self.c_nodes + self.grad_nodes + self.jac_nodes + hroots)
-        src += out + ["    f[b] = %s;" % nm[self.f_node]]
-        src += ["    c[(size_t)b * %d + %d] = %s;" % (m, i, nm[a]) for i, a in enumerate(self.c_nodes)]
-        src += ["    grad[(size_t)b * %d + %d] = %s;" % (n, i, nm[a]) for i, a in enumerate(self.grad_nodes)]
-        src += ["    jac[(size_t)b * %d + %d] = %s;" % (zJ, i, nm[a]) for i, a in enumerate(self.jac_nodes)]
-        for e, terms in enumerate(self._hess_terms):
-            parts = [nm[d2] if k == 0 else "lam[(size_t)b * %d + %d] * %s" % (m, k - 1, nm[d2]) for k, d2 in terms]
-            src.append("    hess[(size_t)b * %d + %d] = %s;" % (zH, e, " + ".join(parts)))
-        src.append("}")
-        return "\n".join(src)
+        chunked = sum(1 for t in G.nodes if t[0] not in ("const", "var")) > piece
+        src = ["// generated by restartsqp_b200/nl_reader.py from %s.nl" % self.name +
+               (" (chunked: %d statements per device function)" % piece if chunked else ""),
+               "static __device__ __forceinline__ double ncdf(double u) { return 0.5 * erfc(-u * 0.7071067811865476); }"]
+        if chunked:
+            src += _MATH_WRAPPERS + [""]
+        store = lambda o, e, v: ("f[b] = %s;" % v if o == "f" else
+                                 "%s[(size_t)b * %d + %d] = %s;" % (o, len(self._outputs[o]), e, v))
+        lam = lambda k: "lam[(size_t)b * %d + %d]" % (self.m, k)
+        kernels = []
+        for tag, outs, sig in (
+                ("fc", ("f", "c"),
+                 ['extern "C" __global__ void nlp_eval_fc(int B, const double* __restrict__ x, double* __restrict__ f, double* __restrict__ c) {']),
+                ("all", tuple(self._outputs),
+                 ['extern "C" __global__ void nlp_eval_all(int B, const double* __restrict__ x, const double* __restrict__ lam,',
+                  "                                        double* __restrict__ f, double* __restrict__ c, double* __restrict__ grad,",
+                  "                                        double* __restrict__ jac, double* __restrict__ hess) {"])):
+            if chunked:  # the device functions go ahead of both kernels
+                funcs, body, nm = _emit_chunked_cuda(G, self._roots(outs), tag, piece, n)
+                src += funcs
+            else:
+                lines, nm, _, xs = _emit(G, self._roots(outs), "c")
+                body = ["    const double x%d = x[(size_t)b * %d + %d];" % (j, n, j) for j in xs] + ["    " + ln for ln in lines]
+            kernels += sig + ["    const int b = blockIdx.x * blockDim.x + threadIdx.x;", "    if (b >= B) return;"] + body
+            kernels += self._stores(outs, nm, store, lam) + ["}", ""]
+        return "\n".join(src + kernels[:-1])  # no blank line after the last kernel
 
     def c_source(self):
         """The straight-line programs as plain C for ONE instance (nlp_fc, nlp_all): used by the CPU oracle's SQP loop
         (oracle/oracle_sqp.c), i.e. by tests and by bench.py's CPU figure, never by the product path."""
-        G, n, m = self.model.G, self.n, self.m
-        hroots = [d2 for terms in self._hess_terms for _, d2 in terms]
-
-        def body(roots):
-            lines, nm = _emit(G, roots, "c")
-            used, stack = set(), list(roots)
-            while stack:
-                a = stack.pop()
-                if a in used:
-                    continue
-                used.add(a)
-                t = G.nodes[a]
-                if t[0] not in ("const", "var"):
-                    stack.extend(t[1:])
-            xs = sorted(G.nodes[a][1] for a in used if G.nodes[a][0] == "var")
-            return ["    const double x%d = x[%d];" % (j, j) for j in xs] + ["    " + ln for ln in lines], nm
-
         src = ["#include <math.h>", "/* generated by restartsqp_b200/nl_reader.py from %s.nl */" % self.name,
-               "static double ncdf(double u) { return 0.5 * erfc(-u * 0.7071067811865476); }",
-               "void nlp_fc(const double* x, double* f, double* c) {"]
-        out, nm = body([self.f_node] + self.c_nodes)
-        src += out + ["    *f = %s;" % nm[self.f_node]] + ["    c[%d] = %s;" % (i, nm[a]) for i, a in enumerate(self.c_nodes)] + ["}", ""]
-        src.append("void nlp_all(const double* x, const double* lam, double* f, double* c, double* grad, double* jac, double* hess) {")
-        out, nm = body([self.f_node] + self.c_nodes + self.grad_nodes + self.jac_nodes + hroots)
-        src += out + ["    *f = %s;" % nm[self.f_node]]
-        src += ["    c[%d] = %s;" % (i, nm[a]) for i, a in enumerate(self.c_nodes)]
-        src += ["    grad[%d] = %s;" % (i, nm[a]) for i, a in enumerate(self.grad_nodes)]
-        src += ["    jac[%d] = %s;" % (i, nm[a]) for i, a in enumerate(self.jac_nodes)]
-        for e, terms in enumerate(self._hess_terms):
-            parts = [nm[d2] if k == 0 else "lam[%d] * %s" % (k - 1, nm[d2]) for k, d2 in terms]
-            src.append("    hess[%d] = %s;" % (e, " + ".join(parts)))
-        src.append("}")
-        return "\n".join(src)
+               "static double ncdf(double u) { return 0.5 * erfc(-u * 0.7071067811865476); }"]
+        store = lambda o, e, v: "*f = %s;" % v if o == "f" else "%s[%d] = %s;" % (o, e, v)
+        for sig, outs in (("void nlp_fc(const double* x, double* f, double* c) {", ("f", "c")),
+                          ("void nlp_all(const double* x, const double* lam, double* f, double* c, double* grad, double* jac, double* hess) {",
+                           tuple(self._outputs))):
+            lines, nm, _, xs = _emit(self.model.G, self._roots(outs), "c")
+            src += [sig] + ["    const double x%d = x[%d];" % (j, j) for j in xs] + ["    " + ln for ln in lines]
+            src += self._stores(outs, nm, store, lambda k: "lam[%d]" % k) + ["}", ""]
+        return "\n".join(src[:-1])  # no blank line after the last function
 
     # ---- SQPTNLP interface (src/SQPTNLP.cpp)
     def Get_nlp_info(self):
